@@ -5,6 +5,7 @@ rays/s of a training step (march + encode + decode + composite + backward) of
   camera, 16 384 rays / step / GPU, occupancy-octree 'ray' march with 128 steps on a pruned level-7 octree.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4|5] [--march ray|voxel]
+                  [--dump-outputs DIR]
 Prints ONE JSON line (rank 0).  The other BASELINE configs (1-based, BASELINE.md section 3):
   1  PanopticDeltaNeF + hash_grid_torch (L=16, T=2^19), 4 096 rays x 64 samples (the reference's CPU-runnable case)
   3  PanopticNeF + tcnn-style hash grid (L=14, T=2^19, base 16), 65 536 rays x 128 samples dense
@@ -275,6 +276,9 @@ class Workload:
         # NB: keeping `rb` alive keeps its autograd graph -- and the parameters' AccumulateGrad nodes, which remember the
         # stream they were created on -- alive; CUDA-graph capture needs them re-created on the capture stream.
         self.last_rb = rb if self.keep_rb else None
+        # detached views of the rendered channels (no autograd graph): under CUDA-graph replay these are the graph's static
+        # output buffers, refreshed by every replay; --dump-outputs reads them
+        self.last_out = {c: getattr(rb, c).detach() for c in self.channels + ['alpha'] if getattr(rb, c, None) is not None}
         return loss
 
     def batch(self, from_host=False):
@@ -436,6 +440,29 @@ def peaks():
     return 6650.0, 1590.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_MAX_ELEMENTS = 1 << 20      # per array: 4 MB as float32
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: write {name: tensor} as path/<name>.npy, float64 kept, everything else as float32.  An array of more than
+    DUMP_MAX_ELEMENTS elements is stored as a 1-D sample of its flattened elements at sorted indices drawn with a fixed seed: the
+    same positions for the same shape in every run, so that the dumps of two builds can be compared element for element."""
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[name] = t.cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def _leave(world, dist=None):
     """Multi-rank exit: barrier (every rank still alive), then tear the NCCL communicator down properly.  A watchdog turns a
     teardown that hangs (captured graphs still holding NCCL kernels have done that) into a loud message instead of a stuck job."""
@@ -519,7 +546,13 @@ def main():
                          "tensor cores (fp16 operands); fp32 is the reported value, tc is reported beside it")
     ap.add_argument("--dd", action="store_true", help="PanopticDDensity field + tracer (own panoptic density stream) instead of the "
                                                       "BASELINE config-2 delta field; informational, not the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0's): training: the "
+                         "loss, the rendered channels and every parameter gradient; config 5: the frame's rgb, depth and label maps "
+                         "(git ignores bench_outputs/)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     cfg = CONFIGS[args.config]
     infer = cfg['mode'] == 'infer'
     if args.steps is None:
@@ -638,11 +671,14 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        run(False)
+        loss = run(False)
     e1.record()
     sync()
     ms = e0.elapsed_time(e1) / args.steps
     trace(f"timed region done: {ms:.3f} ms/step")
+    if args.dump_outputs and rank == 0:      # before the phases below run more steps over the same buffers
+        named = list(wl.nef.named_parameters()) + ([("camera_extrinsics", wl.pipe.camera_extrinsics)] if wl.pipe is not None else [])
+        dump_outputs(args.dump_outputs, {"loss": loss, **wl.last_out, **{"grad." + n: p.grad for n, p in named if p.grad is not None}})
     t_host0 = time.perf_counter()           # CPU time to enqueue a step into an empty stream (GPU-bound when << ms_per_step)
     for _ in range(3):
         run(False)
@@ -833,6 +869,8 @@ def bench_inference(args, cfg, config, metric, unit, rank, world, device, dist):
             out.append(full)
         return out
 
+    last_maps = {}
+
     def time_frames(precision, steps, warmup, e2e):
         for _ in range(max(warmup, 1)):
             gather(render_frame(dev_o, dev_d, precision))
@@ -847,7 +885,7 @@ def bench_inference(args, cfg, config, metric, unit, rank, world, device, dist):
                     dst.copy_(src, non_blocking=True)
                 torch.cuda.current_stream().synchronize()      # the frame is on the host
             else:
-                gather(render_frame(dev_o, dev_d, precision))
+                last_maps[precision] = gather(render_frame(dev_o, dev_d, precision))
         e1.record()
         sync()
         t = torch.tensor([e0.elapsed_time(e1) / steps], device=device, dtype=torch.float64)
@@ -858,6 +896,8 @@ def bench_inference(args, cfg, config, metric, unit, rank, world, device, dist):
     prec = args.infer_precision
     clocks = ClockSampler(device.index or 0) if rank == 0 else None
     ms = time_frames(prec, args.steps, max(args.warmup, 3), False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("rgb", "depth", "semantic_labels", "instance_labels"), last_maps[prec])))
     ms_e2e = time_frames(prec, args.steps, 1, True)
     other = 'tc' if prec == 'fp32' else 'fp32'
     ms_other = time_frames(other, max(2, args.steps // 3), 2, False)

@@ -346,6 +346,24 @@ def test_fused_adam_refuses_cpu_and_amsgrad():
         opt.step()
 
 
+def test_bench_dump_outputs_format(tmp_path):
+    """bench.py --dump-outputs writer: float32 (float64 kept), small arrays whole, large ones as the same seeded sample every time."""
+    import bench
+    big = torch.arange(3 * bench.DUMP_MAX_ELEMENTS, dtype=torch.float64).reshape(3, -1)
+    arrays = {"loss": torch.tensor(2.5), "hit": torch.tensor([True, False]), "grad.a": torch.ones(4, 5, dtype=torch.float16), "big": big}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    a = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in arrays}
+    assert a["loss"].dtype == np.float32 and a["loss"] == 2.5
+    assert a["hit"].tolist() == [1.0, 0.0] and a["grad.a"].dtype == np.float32 and a["grad.a"].shape == (4, 5)
+    assert a["big"].dtype == np.float64 and a["big"].shape == (bench.DUMP_MAX_ELEMENTS,)
+    assert np.all(np.diff(a["big"]) > 0), "distinct elements in index order"
+    assert np.array_equal(a["big"], np.load(tmp_path / "b" / "big.npy")), "same sample positions in every run"
+    with pytest.raises(RuntimeError, match="limit"):
+        bench.dump_outputs(str(tmp_path / "c"), {f"x{i}": torch.zeros(bench.DUMP_MAX_ELEMENTS) for i in range(17)})
+    assert not (tmp_path / "c").exists()
+
+
 def test_bench_configs_build_and_reference_arm_line():
     """bench.py plumbing on the CPU: every BASELINE config's field constructs with the documented shapes, the confined rays of the
     dense configs stay inside the cube, and `--impl reference` prints one JSON line with the same `config` object our arm prints."""
