@@ -365,6 +365,21 @@ int pag_panoptic_loss_bwd(const float* rgb, const float* sem, const float* inst,
                           int64_t N, int Cs, int Ci, float w_rgb, float w_sem, float w_inst, float eps, const float* g_loss, float* g_rgb,
                           float* g_sem, float* g_inst, void* stream);
 
+/* ---- panoptic quality update on the device (validation metric) ----
+ * Replaces the update of the vendored torchmetrics PanopticQuality (utils/metrics/panoptic_quality.py; called from evaluate_metrics,
+ * pc_nerf/trainer.py:651-941: torch.unique per image, a device-to-host copy per segment colour, Python loops over segment pairs).
+ * preds / target i64[B, P, 2] (category, instance), 16-byte aligned.  cat_ids i32[K] sorted ascending, cat_code i32[K] = continuous id
+ * (| 0x100 for a thing) of each; K <= 256.  Accumulates iou_sum f64[K] and counts i64[3][K] (tp | fp | fn), and into errors i64[2] the
+ * number of prediction pixels of an unknown category (unless allow_unknown_preds) and of thing pixels whose instance id lies outside
+ * [0, 2^31).  Three launches (histogram, match, unmatched), no host synchronisation, geometry from (B, P) only; B <= 65535,
+ * P <= 2^30.  workspace: pag_pq_workspace(B, P, &bytes) bytes = 44 * B * C with C the smallest power of two >= 2P (hash tables of
+ * 2+ slots per pixel: never full, whatever the data), zero-filled by the caller ONCE -- every update leaves it zeroed again.
+ * Layout in csrc/metrics.cu. */
+int pag_pq_workspace(int64_t B, int64_t P, int64_t* bytes /* host */);
+int pag_pq_update(const int64_t* preds, const int64_t* target, int64_t B, int64_t P, const int32_t* cat_ids, const int32_t* cat_code,
+                  int K, int allow_unknown_preds, void* workspace, int64_t workspace_bytes, double* iou_sum, int64_t* counts,
+                  int64_t* errors, void* stream);
+
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;
  * configs/bup20/best.yaml:114 optimizer_type adam): n_tensors <= 48 fp32 tensors in one launch, host arrays of device pointers,

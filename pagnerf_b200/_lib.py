@@ -21,6 +21,7 @@ _protos = None
 # kernels launched per entry point (for bench.py's gpu_launches accounting)
 KERNELS_PER_CALL = {
     "pag_march_ray_count": 2, "pag_march_ray_bits_count": 2, "pag_compact_count": 2, "pag_raytrace_count": 2, "pag_voxel_filter_count": 2, "pag_voxel_filter_count_staged": 2, "pag_raytrace_stage": 4, "pag_octree_from_mask": 12, "pag_adam_step": 2, "pag_pan_composite_bwd_tc": 2, "pag_decode_dc_bwd_tc_dyn": 2,
+    "pag_pq_update": 3,
 }
 launch_count = 0
 

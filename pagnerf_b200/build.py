@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libpagnerf_b200.so")
-SOURCES = ["octree.cu", "permuto.cu", "hashgrid.cu", "composite.cu", "pose.cu", "adam.cu", "allreduce.cu", "loss.cu", "decoder.cu", "decoder_tiled.cu", "decoder_tc.cu", "decoder_tc_fused.cu", "tc_test.cu"]
+SOURCES = ["octree.cu", "permuto.cu", "hashgrid.cu", "composite.cu", "pose.cu", "adam.cu", "allreduce.cu", "loss.cu", "metrics.cu", "decoder.cu", "decoder_tiled.cu", "decoder_tc.cu", "decoder_tc_fused.cu", "tc_test.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 
