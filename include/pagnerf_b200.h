@@ -263,6 +263,14 @@ int pag_pan_composite_fwd_f32(const float* feats, const float* dfeats, const flo
                               const float* const* weights, int hidden, int Cs, int Ci, int sem_softmax, int inst_softmax,
                               float inst_temperature, const float* w, const float* alpha, const int64_t* ridx,
                               float* out_sem, float* out_inst, void* stream);
+/* labels of the semantic / instance heads for the point-map export (utils/render_map.py, which calls the nef on every map point and
+ * takes the argmax on the host): same inputs, checks and error codes as pag_pan_composite_fwd_f32, but per sample the argmax class of
+ * the head's logits (lowest index on ties) -> *_label i64[M], and that class's value of the channel the nef returns -> *_score f32[M]
+ * (softmax ? 1 / sum_c exp((z_c - z_max) * s) : z_max * s, s = 1 / inst_temperature for the instance head when > 0, else 1).
+ * No per-class output; nullable pairs skip their head (Cs / Ci = 0). */
+int pag_pan_labels_fwd_f32(const float* feats, const float* dfeats, const float* lodw, int64_t M, int IN, const float* const* weights,
+                           int hidden, int Cs, int Ci, int sem_softmax, int inst_softmax, float inst_temperature, int64_t* sem_label,
+                           float* sem_score, int64_t* inst_label, float* inst_score, void* stream);
 
 /* panoptic heads fused with their compositing (training mode): out[ray] = alpha_ray * sum_s w_s * head(panop_s) with
  * alpha, w detached (tracers/panoptic_packed_rf_tracer.py:148-155,178-205); the [M,C] probabilities never reach HBM.
@@ -379,6 +387,18 @@ int pag_pq_workspace(int64_t B, int64_t P, int64_t* bytes /* host */);
 int pag_pq_update(const int64_t* preds, const int64_t* target, int64_t B, int64_t P, const int32_t* cat_ids, const int32_t* cat_code,
                   int K, int allow_unknown_preds, void* workspace, int64_t workspace_bytes, double* iou_sum, int64_t* counts,
                   int64_t* errors, void* stream);
+
+/* ---- panoptic point-map export (utils/render_map.py: the nef evaluated on the occupied octree cells, labelled, exported) ----
+ * pag_map_cell_points: cells i16[C,3] (leaf cells of `level`, e.g. the octree's level points) -> xyz f32[C*k^3, 3], k in [1, 8]:
+ * sub-point s = (ix*k + iy)*k + iz of cell c at row c*k^3 + s, coordinate (2*(p*k + i) + 1) / (k << level) - 1 in fp32 (IEEE division).
+ * pag_map_instance_stats: per-instance statistics of labelled points (xyz f32[P,3], rgb f32[P,3], semantic / instance i64[P]); a point
+ * counts toward its instance only when bit `semantic` of thing_mask is set (Cs <= 32).  Accumulates count i64[Ci], sum_xyz / sum_rgb
+ * f64[Ci,3] and votes i64[Ci,Cs] (zeroed by the caller) and bbox_min / bbox_max f32[Ci,3] (set to +inf / -inf by the caller); points
+ * with a label outside [0, Cs) / [0, Ci) are skipped and counted in errors i64[1]. */
+int pag_map_cell_points(const int16_t* cells, int64_t C, int level, int k, float* xyz, void* stream);
+int pag_map_instance_stats(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* instance, int64_t P, int Cs, int Ci,
+                           uint32_t thing_mask, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
+                           float* bbox_max, int64_t* errors, void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

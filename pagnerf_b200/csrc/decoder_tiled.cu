@@ -313,6 +313,151 @@ pan_comp_fwd_tiled_kernel(const float* __restrict__ feats, const float* __restri
     }
 }
 
+// Output head reduced to its label: the logits of tl_head (same registers, same arithmetic order), then per sample the winning
+// class and its value of the channel the nef returns -- the [M,C] probabilities are never formed.  (z_max, argmax) and the softmax
+// denominator are reduced over the 16 lanes of the sample group with shuffles; ties go to the lowest class index (torch.argmax).
+// score = softmax ? 1 / sum_c exp((z_c - z_max) * scale) : z_max * scale.  Lane j < 8 of the group writes sample j of its 8.
+template <int NC, int ROWS>
+__device__ __forceinline__ void tl_head_label(const float* __restrict__ A, const float* __restrict__ WT, const float* __restrict__ b, int C,
+                                              bool softmax, float scale, int64_t row0, int64_t M, int64_t* __restrict__ label,
+                                              float* __restrict__ score, int tid) {
+    constexpr int NP = NC / 2;
+    const int cg = tid & 15, sg = tid >> 4;
+    float2 acc[4][NC];
+#pragma unroll
+    for (int i = 0; i < NC; ++i) {
+        const float bv = b[tl_class<NC>(i, cg)];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[j][i] = make_float2(bv, bv);
+    }
+    {
+        const float* a = A + sg * 8;
+        const float* wt = WT + 2 * cg;
+        const float* wl = WT + NP * 32 + cg;
+#pragma unroll 2
+        for (int k = 0; k < H; ++k) {
+            const float4 a0 = *reinterpret_cast<const float4*>(a + k * TL_LDA(ROWS));
+            const float4 a1 = *reinterpret_cast<const float4*>(a + k * TL_LDA(ROWS) + 4);
+            const float2 av[4] = {make_float2(a0.x, a0.y), make_float2(a0.z, a0.w), make_float2(a1.x, a1.y), make_float2(a1.z, a1.w)};
+#pragma unroll
+            for (int ip = 0; ip < NP; ++ip) {
+                const float2 wv = *reinterpret_cast<const float2*>(wt + k * (16 * NC) + ip * 32);
+#pragma unroll
+                for (int j = 0; j < 4; ++j) { ffma2(acc[j][2 * ip], av[j], wv.x); ffma2(acc[j][2 * ip + 1], av[j], wv.y); }
+            }
+            if (NC & 1) {
+                const float wv = wl[k * (16 * NC)];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) ffma2(acc[j][NC - 1], av[j], wv);
+            }
+        }
+    }
+    // per lane: classes tl_class<NC>(i, cg) ascend with i, so a strict > keeps the lowest index among equal logits
+    float mx[8];
+    int am[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { mx[j] = -INFINITY; am[j] = 0x7fffffff; }
+#pragma unroll
+    for (int i = 0; i < NC; ++i) {
+        const int c = tl_class<NC>(i, cg);
+        if (c < C) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                if (acc[j][i].x > mx[2 * j] || am[2 * j] == 0x7fffffff) { mx[2 * j] = acc[j][i].x; am[2 * j] = c; }
+                if (acc[j][i].y > mx[2 * j + 1] || am[2 * j + 1] == 0x7fffffff) { mx[2 * j + 1] = acc[j][i].y; am[2 * j + 1] = c; }
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+#pragma unroll
+        for (int o = 1; o < 16; o <<= 1) {
+            const float v = __shfl_xor_sync(0xffffffffu, mx[j], o);
+            const int c = __shfl_xor_sync(0xffffffffu, am[j], o);
+            if (v > mx[j] || (v == mx[j] && c < am[j]) || am[j] == 0x7fffffff) { mx[j] = v; am[j] = c; }
+        }
+    }
+    float sc[8];
+    if (softmax) {
+        const float sc2 = scale * 1.4426950408889634f;      // exp((z - mx) * scale) = 2^((z - mx) * scale * log2 e)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) sc[j] = 0.f;
+#pragma unroll
+        for (int i = 0; i < NC; ++i)
+            if (tl_class<NC>(i, cg) < C) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    sc[2 * j] += ex2_approx((acc[j][i].x - mx[2 * j]) * sc2);
+                    sc[2 * j + 1] += ex2_approx((acc[j][i].y - mx[2 * j + 1]) * sc2);
+                }
+            }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+#pragma unroll
+            for (int o = 1; o < 16; o <<= 1) sc[j] += __shfl_xor_sync(0xffffffffu, sc[j], o);
+            sc[j] = 1.f / sc[j];
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) sc[j] = mx[j] * scale;
+    }
+    // lane cg < 8 writes sample sg * 8 + cg (a select chain keeps the arrays in registers)
+    int lab = am[0];
+    float s = sc[0];
+#pragma unroll
+    for (int j = 1; j < 8; ++j)
+        if (cg == j) { lab = am[j]; s = sc[j]; }
+    const int64_t m = row0 + sg * 8 + cg;
+    if (cg < 8 && m < M) { label[m] = lab; score[m] = s; }
+}
+
+// Labels of the semantic / instance heads (csrc map export): the staging, tiling and layers of pan_comp_fwd_tiled_kernel with the
+// label epilogue instead of the compositing one.
+__global__ void __launch_bounds__(PAN_MAXG * (2 * PAN_ROWS), 1)
+pan_labels_fwd_tiled_kernel(const float* __restrict__ feats, const float* __restrict__ dfeats, const float* __restrict__ lodw,
+                            int64_t M, int IN, PanParams p, int Cs, int Ci, int sem_softmax, int inst_softmax, float inv_temp,
+                            int64_t* __restrict__ sem_label, float* __restrict__ sem_score, int64_t* __restrict__ inst_label,
+                            float* __restrict__ inst_score) {
+    extern __shared__ __align__(16) float smem[];
+    const int NG = blockDim.x / (2 * PAN_ROWS), grp = threadIdx.x / (2 * PAN_ROWS), gt = threadIdx.x - grp * (2 * PAN_ROWS);
+    const TlPanLayout l = tl_pan_layout(IN, NG);
+    float* P = smem + l.groups + grp * l.gstride;
+    float *Q = P + TL_BUF(PAN_ROWS), *R = Q + TL_BUF(PAN_ROWS);
+    const int64_t ntiles = (M + PAN_ROWS - 1) / PAN_ROWS;
+    const int64_t tile0 = (int64_t)blockIdx.x * NG + grp, tstride = (int64_t)gridDim.x * NG;
+    auto fetch = [&](int64_t tile) {
+        tl_fetch_rows<PAN_ROWS>(P, feats, IN, tile * PAN_ROWS, M, gt);
+        if (dfeats) tl_fetch_rows<PAN_ROWS>(Q, dfeats, IN, tile * PAN_ROWS, M, gt);
+        cp_async_commit();
+    };
+    if (tile0 < ntiles) fetch(tile0);
+    if (Cs > 0) {
+        tl_stage_wt(smem + l.Ws1T, p.Ws1, H, H, IN, IN); tl_stage_b(smem + l.bs1, p.bs1, H, H);
+        tl_stage_wt(smem + l.Ws2T, p.Ws2, Cs, 16, H, H); tl_stage_b(smem + l.bs2, p.bs2, Cs, 16);
+    }
+    if (Ci > 0) {
+        tl_stage_wt(smem + l.Wi1T, p.Wi1, H, H, IN, IN); tl_stage_b(smem + l.bi1, p.bi1, H, H);
+        tl_stage_wt(smem + l.Wi2T, p.Wi2, H, H, H, H); tl_stage_b(smem + l.bi2, p.bi2, H, H);
+        tl_stage_wt(smem + l.Wi3T, p.Wi3, Ci, TL_CIP, H, H); tl_stage_b(smem + l.bi3, p.bi3, Ci, TL_CIP);
+    }
+    __syncthreads();                       // weights staged (the only block-wide barrier)
+    for (int64_t tile = tile0; tile < ntiles; tile += tstride) {
+        const int64_t row0 = tile * PAN_ROWS;
+        cp_async_wait_all();
+        group_sync<PAN_ROWS>(grp);                   // raw rows landed; the previous tile's instance head is done with R
+        tl_transpose_x<PAN_ROWS>(R, P, dfeats ? Q : nullptr, lodw, IN, row0, M, gt);
+        group_sync<PAN_ROWS>(grp);
+        if (Cs > 0) tl_layer64<PAN_ROWS>(R, IN, smem + l.Ws1T, smem + l.bs1, P, gt);
+        if (Ci > 0) tl_layer64<PAN_ROWS>(R, IN, smem + l.Wi1T, smem + l.bi1, Q, gt);
+        group_sync<PAN_ROWS>(grp);
+        if (Cs > 0) tl_head_label<1, PAN_ROWS>(P, smem + l.Ws2T, smem + l.bs2, Cs, sem_softmax != 0, 1.f, row0, M, sem_label, sem_score, gt);
+        if (Ci > 0) tl_layer64<PAN_ROWS>(Q, H, smem + l.Wi2T, smem + l.bi2, R, gt);
+        group_sync<PAN_ROWS>(grp);
+        if (tile + tstride < ntiles) fetch(tile + tstride);
+        if (Ci > 0) tl_head_label<13, PAN_ROWS>(R, smem + l.Wi3T, smem + l.bi3, Ci, inst_softmax != 0, inv_temp, row0, M, inst_label, inst_score, gt);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // density + colour
 // ---------------------------------------------------------------------------------------------
@@ -475,6 +620,32 @@ int pag_pan_composite_fwd_f32(const float* feats, const float* dfeats, const flo
     const float it = inst_temperature > 0.f ? 1.f / inst_temperature : 1.f;
     pan_comp_fwd_tiled_kernel<<<grid, NG * (2 * PAN_ROWS), bytes, (cudaStream_t)stream>>>(feats, dfeats, lodw, M, IN, p, Cs, Ci, sem_softmax,
                                                                             inst_softmax, it, w, alpha, ridx, out_sem, out_inst);
+    PAG_LAUNCH_CHECK();
+    return PAG_OK;
+}
+
+// Semantic + instance labels of (feats + dfeats) * lodw, exact FP32, forward only: argmax class (lowest on ties) and its value of
+// the head's output channel per sample, no per-class output.
+int pag_pan_labels_fwd_f32(const float* feats, const float* dfeats, const float* lodw, int64_t M, int IN, const float* const* weights,
+                           int hidden, int Cs, int Ci, int sem_softmax, int inst_softmax, float inst_temperature, int64_t* sem_label,
+                           float* sem_score, int64_t* inst_label, float* inst_score, void* stream) {
+    if (hidden != H || IN < 4 || IN > 64 || (IN & 3) || Cs < 0 || Cs > 16 || Ci < 0 || Ci > TL_CIP) return PAG_ERR_UNSUPPORTED;
+    if (M == 0 || (Cs == 0 && Ci == 0)) return PAG_OK;
+    if (!feats || (Cs && (!sem_label || !sem_score)) || (Ci && (!inst_label || !inst_score))) return PAG_ERR_ARG;
+    PanParams p{};
+    p.Ws1 = weights[0]; p.bs1 = weights[1]; p.Ws2 = weights[2]; p.bs2 = weights[3]; p.Wi1 = weights[4]; p.bi1 = weights[5];
+    p.Wi2 = weights[6]; p.bi2 = weights[7]; p.Wi3 = weights[8]; p.bi3 = weights[9];
+    int NG = PAN_MAXG;
+    while (NG > 1 && (size_t)tl_pan_layout(IN, NG).total * sizeof(float) > 227 * 1024) --NG;
+    const size_t bytes = (size_t)tl_pan_layout(IN, NG).total * sizeof(float);
+    if (bytes > 227 * 1024) return PAG_ERR_UNSUPPORTED;
+    cudaError_t e = cudaFuncSetAttribute(pan_labels_fwd_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) return (int)e;
+    const int64_t tiles = ((M + PAN_ROWS - 1) / PAN_ROWS + NG - 1) / NG;
+    const int grid = (int)(tiles < tl_num_sms() ? tiles : tl_num_sms());
+    const float it = inst_temperature > 0.f ? 1.f / inst_temperature : 1.f;
+    pan_labels_fwd_tiled_kernel<<<grid, NG * (2 * PAN_ROWS), bytes, (cudaStream_t)stream>>>(feats, dfeats, lodw, M, IN, p, Cs, Ci, sem_softmax,
+                                                                              inst_softmax, it, sem_label, sem_score, inst_label, inst_score);
     PAG_LAUNCH_CHECK();
     return PAG_OK;
 }

@@ -1,0 +1,195 @@
+"""Labelled 3-D panoptic point map of a trained field, on the device: what the reference's utils/render_map.py exports by calling the
+nef on the octree, without the [P, C] probability tensors, the per-thread decoder kernels or the host-side argmax.
+
+    pts = extract_panoptic_map(nef, samples_per_axis=2)        # PanopticPoints of CUDA tensors, P kept points
+    summ = instance_summary(pts, num_instances=nef.num_instances, num_classes=nef.num_classes, things={0})
+    write_ply("map.ply", pts)
+
+Definitions (the CPU oracle, oracle/mapping.py, and the tests follow them exactly):
+  * Points.  Every occupied leaf cell of nef.grid.blas at nef.grid.blas_level (spc.unbatched_get_level_points, Morton order) gets
+    k^3 sub-cell centres, k = samples_per_axis in [1, 8].  Sub-point s = (ix*k + iy)*k + iz (the axis order of
+    pag_octree_level_bits); per axis, in fp32 with IEEE division, x = (float)(2*(p*k + i) + 1) / (float)(k << L) - 1.0f for the
+    cell's integer coordinate p at level L.  Numerator and denominator are exact integers, there is no jitter: the map is
+    deterministic.  Output order is cell order, then sub-point order, filtered by the density test; it does not depend on
+    chunk_points.
+  * Density and colour come from the colour branch: the density head after its ReLU, and the colour seen along the single
+    direction view_dir (normalised here).  The default (0, 0, -1) is the look direction of the synthetic robot pass of bench.py
+    and the tests; with real data pass the mean viewing direction.  All LODs are used (lod_idx = num_lods - 1), exact fp32, no
+    autocast, like validation.  PanopticDDensityNeF's panoptic density is not used: the map's geometry is the colour density for
+    every field.
+  * A point is kept iff density > min_density.  The default is prune()'s cell threshold 0.01 * 512 / sqrt(3): "in the map" means
+    what "kept by prune" means.
+  * Labels are the argmax over the channel the nef's forward returns (logits times 1/T when inst_soft_temperature T > 0), taken on
+    the logits, lowest class index on ties.  The score is the winning class's value of that channel: 1 / sum_c exp((z_c - z_max) * s)
+    with a softmax head, z_max * s without one.
+  * The heads read _panoptic_inputs(feats, coords, lod_idx, rows), the (a + b) * lod_weights the fused render uses; the delta grid
+    is looked up for the kept rows only.
+  * Supported fields: those whose heads the fused kernels serve (PanopticNeF._fused_heads_unsupported): plain heads, detached,
+    'cat', feature width <= 48 and a multiple of 4, <= 16 classes, <= 208 instances.  Anything else raises NotImplementedError
+    with the reason; a field on the CPU raises RuntimeError (no CPU fallback).
+  * Host reads: one per chunk, the kept count (the size of that chunk's output, torch.nonzero).
+
+instance_summary counts a point toward instance `inst` only when its semantic class is in `things` (every class when None), and
+returns centroid = sum_xyz / count in float64 (NaN where count == 0; bbox_min / bbox_max stay +inf / -inf there).
+"""
+import math
+from typing import NamedTuple
+
+import numpy as np
+import torch
+
+from .. import ops, spc
+from ..pc_nerf import PanopticNeF
+from ..pc_nerf.panoptic_nef import _decoder_tensors
+
+MAX_SAMPLES_PER_AXIS = 8
+PRUNE_MIN_DENSITY = (0.01 * 512) / math.sqrt(3)      # PanopticNeF.prune()'s cell threshold
+MAX_SUMMARY_CLASSES = 32                             # thing mask: one bit per class
+
+
+class PanopticPoints(NamedTuple):
+    xyz: torch.Tensor              # f32 [P, 3]
+    rgb: torch.Tensor              # f32 [P, 3]
+    density: torch.Tensor          # f32 [P]
+    semantic: torch.Tensor         # i64 [P]
+    semantic_score: torch.Tensor   # f32 [P]
+    instance: torch.Tensor         # i64 [P]
+    instance_score: torch.Tensor   # f32 [P]
+
+
+class InstanceSummary(NamedTuple):
+    count: torch.Tensor            # i64 [Ci]
+    centroid: torch.Tensor         # f64 [Ci, 3]
+    bbox_min: torch.Tensor         # f32 [Ci, 3]
+    bbox_max: torch.Tensor         # f32 [Ci, 3]
+    mean_rgb: torch.Tensor         # f64 [Ci, 3]
+    votes: torch.Tensor            # i64 [Ci, Cs]
+    category: torch.Tensor         # i64 [Ci]: argmax of votes (lowest class on ties), -1 where count == 0
+
+
+def _empty_points(device):
+    f = lambda *s: torch.empty(*s, dtype=torch.float32, device=device)
+    i = lambda *s: torch.empty(*s, dtype=torch.int64, device=device)
+    return PanopticPoints(f(0, 3), f(0, 3), f(0), i(0), f(0), i(0), f(0))
+
+
+def _check_field(nef):
+    if not isinstance(nef, PanopticNeF):
+        raise NotImplementedError(f"map export serves PanopticNeF and its subclasses, not {type(nef).__name__}")
+    if nef.position_input:
+        raise NotImplementedError("map export: position_input fields are not served by the fused decoders")
+    reason = nef._fused_heads_unsupported()
+    if reason is not None:
+        raise NotImplementedError(f"map export: the label kernel does not serve {reason}")
+    if not nef.decoder_density.lout.weight.is_cuda:
+        raise RuntimeError("pagnerf_b200 map export runs on CUDA fields only (no CPU fallback)")
+
+
+def extract_panoptic_map(nef, samples_per_axis=2, min_density=None, view_dir=(0.0, 0.0, -1.0), chunk_points=1 << 21):
+    """-> PanopticPoints of the k^3 sub-cell centres of every occupied leaf cell whose density exceeds min_density (see the module
+    docstring for the exact definitions).  Works in chunks of at most max(chunk_points, k^3) points; one host read per chunk."""
+    k = samples_per_axis
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= MAX_SAMPLES_PER_AXIS:
+        raise ValueError(f"samples_per_axis must be an integer in [1, {MAX_SAMPLES_PER_AXIS}], got {k!r}")
+    k = int(k)
+    if int(chunk_points) < 1:
+        raise ValueError(f"chunk_points must be positive, got {chunk_points}")
+    _check_field(nef)
+    dev = nef.decoder_density.lout.weight.device
+    vd = torch.as_tensor(view_dir, dtype=torch.float32).reshape(3)
+    if not torch.isfinite(vd).all() or float(vd.norm()) == 0.0:
+        raise ValueError(f"view_dir must be a finite non-zero 3-vector, got {view_dir}")
+    vd = (vd / vd.norm()).reshape(1, 3).to(dev)
+    thr = PRUNE_MIN_DENSITY if min_density is None else float(min_density)
+    grid = nef.grid
+    level = int(grid.blas_level)
+    blas = grid.blas.to(dev)
+    cells = spc.unbatched_get_level_points(blas.points, blas.pyramid, level)
+    C = cells.shape[0]
+    if C == 0:
+        return _empty_points(dev)
+    kk = k ** 3
+    cells_per_chunk = max(1, int(chunk_points) // kk)
+    lod_idx = nef.num_lods - 1
+    w_dc = _decoder_tensors(nef.decoder_density, 1) + _decoder_tensors(nef.decoder_color, 2)
+    w_pan = _decoder_tensors(nef.decoder_semantics, 1) + _decoder_tensors(nef.decoder_inst, 2)
+    Cs, Ci = int(nef.num_classes), int(nef.num_instances)
+    temp = float(getattr(nef, 'inst_soft_temperature', 0.0))
+    parts = []
+    with torch.no_grad(), torch.autocast('cuda', enabled=False):
+        lodw = nef._lodw(dev)
+        for c0 in range(0, C, cells_per_chunk):
+            xyz = ops.map_cell_points(cells[c0:c0 + cells_per_chunk], level, k)
+            coords = xyz[:, None]
+            feats = nef._encode(grid, coords, lod_idx)
+            n = xyz.shape[0]
+            # one ray carrying the chunk's points: every point is seen along view_dir
+            sigma, rgb = ops.DecodeDCFn.apply(feats, lodw, vd, n, True, 'tiled', *w_dc)
+            rows = torch.nonzero(sigma > thr).reshape(-1)          # the chunk's one host read: its output size
+            if rows.numel() == 0:
+                continue
+            a, b = nef._panoptic_inputs(feats, coords, lod_idx, rows)
+            del feats
+            sl, ss, il, is_ = ops.pan_labels_f32(a, b, lodw, Cs, Ci, bool(nef.sem_softmax), bool(nef.inst_softmax), temp, *w_pan)
+            del a, b
+            parts.append((xyz.index_select(0, rows), rgb.index_select(0, rows), sigma.index_select(0, rows), sl, ss, il, is_))
+    if not parts:
+        return _empty_points(dev)
+    if len(parts) == 1:
+        return PanopticPoints(*parts[0])
+    return PanopticPoints(*(torch.cat(col) for col in zip(*parts)))
+
+
+def instance_summary(pts, num_instances, num_classes, things=None):
+    """Per-instance statistics of a labelled map (csrc/mapping.cu, one launch + one host read for the error count) -> InstanceSummary.
+    A point counts toward its instance only when its semantic class is in `things` (every class when None).  Raises ValueError if a
+    point carries a semantic label outside [0, num_classes) or an instance label outside [0, num_instances)."""
+    Ci, Cs = int(num_instances), int(num_classes)
+    if Ci < 1 or not 1 <= Cs <= MAX_SUMMARY_CLASSES:
+        raise ValueError(f"num_instances must be >= 1 and num_classes in [1, {MAX_SUMMARY_CLASSES}], got {Ci}, {Cs}")
+    if things is None:
+        mask = (1 << Cs) - 1
+    else:
+        things = set(int(c) for c in things)
+        if not all(0 <= c < Cs for c in things):
+            raise ValueError(f"things must be classes in [0, {Cs}), got {sorted(things)}")
+        mask = sum(1 << c for c in things)
+    if not pts.xyz.is_cuda:
+        raise RuntimeError("pagnerf_b200 map export runs on CUDA tensors only (no CPU fallback)")
+    count, sum_xyz, sum_rgb, votes, bmin, bmax, errors = ops.map_instance_stats(pts.xyz, pts.rgb, pts.semantic, pts.instance, Cs, Ci, mask)
+    bad = int(errors.item())
+    if bad:
+        raise ValueError(f"{bad} points carry a semantic label outside [0, {Cs}) or an instance label outside [0, {Ci})")
+    n = count.to(torch.float64)[:, None]
+    category = torch.where(count > 0, votes.argmax(dim=1), torch.full_like(count, -1))
+    return InstanceSummary(count, sum_xyz / n, bmin, bmax, sum_rgb / n, votes, category)
+
+
+PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),
+                  ("red", "uchar", "u1"), ("green", "uchar", "u1"), ("blue", "uchar", "u1"),
+                  ("density", "float", "<f4"), ("semantic", "int", "<i4"), ("semantic_score", "float", "<f4"),
+                  ("instance", "int", "<i4"), ("instance_score", "float", "<f4")]
+
+
+def write_ply(path, pts):
+    """Binary little-endian PLY of a map, one vertex per point: x y z (float), red green blue (uchar, round(255 * clamp(rgb, 0, 1))),
+    density, semantic (int), semantic_score, instance (int), instance_score."""
+    P = int(pts.xyz.shape[0])
+    rec = np.empty(P, dtype=[(n, t) for n, _, t in PLY_PROPERTIES])
+    xyz = pts.xyz.detach().cpu().numpy().astype(np.float32)
+    rgb = np.rint(np.clip(pts.rgb.detach().cpu().numpy().astype(np.float64), 0.0, 1.0) * 255.0).astype(np.uint8)
+    for i, n in enumerate("xyz"):
+        rec[n] = xyz[:, i]
+    for i, n in enumerate(("red", "green", "blue")):
+        rec[n] = rgb[:, i]
+    rec["density"] = pts.density.detach().cpu().numpy()
+    rec["semantic"] = pts.semantic.detach().cpu().numpy()
+    rec["semantic_score"] = pts.semantic_score.detach().cpu().numpy()
+    rec["instance"] = pts.instance.detach().cpu().numpy()
+    rec["instance_score"] = pts.instance_score.detach().cpu().numpy()
+    header = ["ply", "format binary_little_endian 1.0", f"element vertex {P}"]
+    header += [f"property {t} {n}" for n, t, _ in PLY_PROPERTIES]
+    header += ["end_header"]
+    with open(path, "wb") as f:
+        f.write(("\n".join(header) + "\n").encode("ascii"))
+        f.write(rec.tobytes())

@@ -588,6 +588,55 @@ def pan_composite_f32(feats, dfeats, lodw, w, alpha, ridx, N, Cs, Ci, sem_softma
     return sem, inst
 
 
+def pan_labels_f32(feats, dfeats, lodw, Cs, Ci, sem_softmax, inst_softmax, inst_temperature, *weights):
+    """Exact-FP32 semantic + instance heads reduced to labels, forward only (map export; csrc/decoder_tiled.cu):
+    -> (sem_label i64[M], sem_score f32[M], inst_label i64[M], inst_score f32[M]), None for a head with C = 0.  label = argmax of
+    the logits (lowest class on ties), score = that class's value of the head's output channel -- the [M,C] tensors never exist."""
+    _chk(feats, dfeats, *weights)
+    with torch.no_grad():
+        f, df = _f32(feats), _f32(dfeats)
+        M, IN = f.shape
+        wt = [_f32(x) for x in weights]
+        lw = _f32(lodw)
+        dev = f.device
+        sl = torch.empty(M, dtype=torch.int64, device=dev) if Cs else None
+        ss = torch.empty(M, dtype=torch.float32, device=dev) if Cs else None
+        il = torch.empty(M, dtype=torch.int64, device=dev) if Ci else None
+        is_ = torch.empty(M, dtype=torch.float32, device=dev) if Ci else None
+        call("pag_pan_labels_fwd_f32", ptr(f), ptr(df), ptr(lw), M, IN, ptr_array(wt), HIDDEN, int(Cs), int(Ci),
+             int(bool(sem_softmax)), int(bool(inst_softmax)), float(inst_temperature), ptr(sl), ptr(ss), ptr(il), ptr(is_))
+    return sl, ss, il, is_
+
+
+def map_cell_points(cells, level, k):
+    """Sub-cell centres of the leaf cells i16[C,3] of `level`: -> f32[C*k^3, 3] (csrc/mapping.cu pag_map_cell_points)."""
+    _chk(cells)
+    c = cells.to(torch.int16).contiguous()
+    xyz = torch.empty(c.shape[0] * k ** 3, 3, dtype=torch.float32, device=c.device)
+    call("pag_map_cell_points", ptr(c), c.shape[0], int(level), int(k), ptr(xyz))
+    return xyz
+
+
+def map_instance_stats(xyz, rgb, semantic, instance, Cs, Ci, thing_mask):
+    """-> count i64[Ci], sum_xyz f64[Ci,3], sum_rgb f64[Ci,3], votes i64[Ci,Cs], bbox_min / bbox_max f32[Ci,3], errors i64[1]
+    (points with an out-of-range label, counted on the device; csrc/mapping.cu pag_map_instance_stats)."""
+    _chk(xyz, rgb, semantic, instance)
+    dev = xyz.device
+    x, r = _f32(xyz).reshape(-1, 3), _f32(rgb).reshape(-1, 3)
+    s, q = semantic.to(torch.int64).contiguous(), instance.to(torch.int64).contiguous()
+    P = x.shape[0]
+    count = torch.zeros(Ci, dtype=torch.int64, device=dev)
+    sum_xyz = torch.zeros(Ci, 3, dtype=torch.float64, device=dev)
+    sum_rgb = torch.zeros(Ci, 3, dtype=torch.float64, device=dev)
+    votes = torch.zeros(Ci, Cs, dtype=torch.int64, device=dev)
+    bmin = torch.full((Ci, 3), float('inf'), dtype=torch.float32, device=dev)
+    bmax = torch.full((Ci, 3), float('-inf'), dtype=torch.float32, device=dev)
+    errors = torch.zeros(1, dtype=torch.int64, device=dev)
+    call("pag_map_instance_stats", ptr(x), ptr(r), ptr(s), ptr(q), P, int(Cs), int(Ci), int(thing_mask) & 0xFFFFFFFF, ptr(count),
+         ptr(sum_xyz), ptr(sum_rgb), ptr(votes), ptr(bmin), ptr(bmax), ptr(errors))
+    return count, sum_xyz, sum_rgb, votes, bmin, bmax, errors
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""

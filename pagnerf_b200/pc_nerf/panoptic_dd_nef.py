@@ -77,6 +77,16 @@ class PanopticDDensityNeF(PanopticNeF):
     def _pan_src(self):
         return 'delta'
 
+    def _panoptic_inputs(self, feats, coords, lod_idx, rows=None):
+        """(a, b) of rgb_semantics (:229): (feats.detach(), delta), or (delta, None) with separate_sem_grid.  rows (int64 [K],
+        inference only): evaluate packed samples `rows` only -- the delta grid is looked up for those only."""
+        a = feats.detach()
+        if rows is not None:
+            a = a.index_select(0, rows)
+            coords = coords.reshape(-1, 1, 3).index_select(0, rows)
+        dfe = self._encode(self.delta_grid, coords.detach(), lod_idx)
+        return (a, dfe) if not self.separate_sem_grid else (dfe, None)
+
     def fused_trace_tensors(self):
         table, dtable, wts = super().fused_trace_tensors()
         dec = self.decoder_delta_density          # Linear(+Identity) layers collapsed into one map (autograd reaches both layers)

@@ -243,11 +243,24 @@ class PanopticNeF(BaseNeuralField):
             return False
         if not self._use_tc() and (torch.is_grad_enabled() or not ops.TILED_F32):
             return False
-        plain = not (self.sem_sigmoid or self.sem_normalize or self.inst_sigmoid or self.inst_normalize or self.inst_direct_pos)
-        det = self.sem_detach and self.inst_detach
-        shapes = (self.effective_feature_dim <= 48 and self.effective_feature_dim % 4 == 0 and self.num_classes <= 16
-                  and self.num_instances <= 208 and self.multiscale_type == 'cat')
-        return plain and det and shapes and self.panoptic_features_type in (None, 'delta', 'separate', 'appearance')
+        return self._fused_heads_unsupported() is None
+
+    def _fused_heads_unsupported(self):
+        """None when the fused-head kernels (csrc/decoder_tc_fused.cu, csrc/decoder_tiled.cu) serve this field's semantic /
+        instance heads, else the reason they do not."""
+        if self.sem_sigmoid or self.sem_normalize or self.inst_sigmoid or self.inst_normalize or self.inst_direct_pos:
+            return "sigmoid / normalize / inst_direct_pos head options"
+        if not (self.sem_detach and self.inst_detach):
+            return "non-detached panoptic heads (sem_detach / inst_detach False)"
+        if self.multiscale_type != 'cat':
+            return f"multiscale_type '{self.multiscale_type}'"
+        if self.effective_feature_dim > 48 or self.effective_feature_dim % 4:
+            return f"feature width {self.effective_feature_dim} (needs <= 48 and a multiple of 4)"
+        if self.num_classes > 16 or self.num_instances > 208:
+            return f"{self.num_classes} classes / {self.num_instances} instances (at most 16 / 208)"
+        if self.panoptic_features_type not in (None, 'delta', 'separate', 'appearance'):
+            return f"panoptic_features_type '{self.panoptic_features_type}'"
+        return None
 
     def _pan_src(self):
         """Which features feed the panoptic heads in the fused kernels."""
