@@ -394,11 +394,32 @@ int pag_pq_update(const int64_t* preds, const int64_t* target, int64_t B, int64_
  * pag_map_instance_stats: per-instance statistics of labelled points (xyz f32[P,3], rgb f32[P,3], semantic / instance i64[P]); a point
  * counts toward its instance only when bit `semantic` of thing_mask is set (Cs <= 32).  Accumulates count i64[Ci], sum_xyz / sum_rgb
  * f64[Ci,3] and votes i64[Ci,Cs] (zeroed by the caller) and bbox_min / bbox_max f32[Ci,3] (set to +inf / -inf by the caller); points
- * with a label outside [0, Cs) / [0, Ci) are skipped and counted in errors i64[1]. */
+ * with a label outside [0, Cs) / [0, Ci) are skipped and counted in errors i64[1].  Label counts whose per-CTA slots fit in shared
+ * memory accumulate there; larger ones accumulate in global memory, runs of equal labels reduced per warp first. */
 int pag_map_cell_points(const int16_t* cells, int64_t C, int level, int k, float* xyz, void* stream);
 int pag_map_instance_stats(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* instance, int64_t P, int Cs, int Ci,
                            uint32_t thing_mask, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
                            float* bbox_max, int64_t* errors, void* stream);
+/* ---- connected components of a labelled map (no reference counterpart: objects of the exported map) ----
+ * pag_map_components: xyz f32[P,3] on the lattice of (k, level), D = k << level (a coordinate is bit for bit
+ * fl(fl((2j+1)/D) - 1), j in [0, D)), semantic / instance i64[P].  A point is active iff its labels are in [0, Cs) / [0, Ci) and bit
+ * `semantic` of thing_mask is set; two active points are adjacent iff their lattice indices differ by a vector of {-1,0,1}^3 \ {0}
+ * (connectivity 26) or by one unit step (connectivity 6) and their instance labels are equal.  Writes component i64[P]: the object
+ * of each point, numbered 0..K-1 in the order of each object's smallest point index, -1 for inactive points and for objects of
+ * fewer than min_points points.  info i64[4] (set by the call) = K | points off the lattice | points repeating the lattice index of
+ * another point | points with a label out of range; component is meaningful only when the three counts are 0.  Seven launches,
+ * no host synchronisation; P <= 2^30, Cs <= 32.  workspace: pag_map_components_workspace(P, &bytes) bytes = 12 C + 16 P +
+ * 12 ceil(P / 1024) + 8, C = the smallest power of two >= 2P (hash table key u64 | point u32, never full), 8-byte aligned, no
+ * initialisation needed.  Layout in csrc/mapping.cu.
+ * pag_map_component_stats: pag_map_instance_stats per object (K labels, points with component -1 skipped, no thing mask, no error
+ * count) plus object_instance i64[K], the instance label of each object. */
+int pag_map_components_workspace(int64_t P, int64_t* bytes /* host */);
+int pag_map_components(const float* xyz, const int64_t* semantic, const int64_t* instance, int64_t P, int level, int k, int Cs, int Ci,
+                       uint32_t thing_mask, int connectivity, int64_t min_points, void* workspace, int64_t workspace_bytes,
+                       int64_t* component, int64_t* info, void* stream);
+int pag_map_component_stats(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* instance, const int64_t* component,
+                            int64_t P, int Cs, int K, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
+                            float* bbox_max, int64_t* object_instance, void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

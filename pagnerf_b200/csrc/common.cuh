@@ -30,6 +30,33 @@ __device__ __forceinline__ float pag_jitter(uint32_t seed, uint64_t idx) {
     return (float)(pag_lowbias32(x) >> 8) * (1.0f / 16777216.0f);
 }
 
+// open-addressing hash tables of 64-bit keys (key 0 = empty slot), linear probing, C a power of two.  pag_hash_slots(n): the
+// smallest power of two >= 2n, so that n distinct keys fill at most half of a table: it never overflows, whatever the data.
+static inline int64_t pag_hash_slots(int64_t n) {
+    int64_t c = 2;
+    while (c < 2 * n) c <<= 1;
+    return c;
+}
+
+__device__ __forceinline__ uint32_t pag_hash64(unsigned long long k) {      // murmur3 fmix64
+    k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
+    return (uint32_t)k;
+}
+
+// slot of `key` in table[C], inserted if absent; *inserted says whether this call put it there.  A slot's key goes from 0 to its
+// final value once, so a plain load that sees the key (or another key) is final; a stale 0 only sends us to the CAS, which
+// returns the truth.
+__device__ __forceinline__ uint32_t pag_hash_insert(unsigned long long* __restrict__ table, uint32_t C, unsigned long long key,
+                                                    bool* inserted) {
+    uint32_t s = pag_hash64(key) & (C - 1);
+    while (true) {
+        unsigned long long cur = __ldcg(table + s);
+        if (cur == 0ull) cur = atomicCAS(table + s, 0ull, key);
+        if (cur == 0ull || cur == key) { *inserted = cur == 0ull; return s; }
+        s = (s + 1) & (C - 1);
+    }
+}
+
 __device__ __forceinline__ float2 ldg2(const float* p) { return __ldg(reinterpret_cast<const float2*>(p)); }
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 

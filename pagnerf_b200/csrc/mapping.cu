@@ -9,6 +9,7 @@
 #include "common.cuh"
 
 #define MAP_STATS_BLOCK 256
+#define MAP_CC_MAX_POINTS (1ll << 30)
 
 __global__ void __launch_bounds__(256) map_cell_points_kernel(const int16_t* __restrict__ cells, int64_t n, int level, int k,
                                                               float* __restrict__ xyz) {
@@ -46,11 +47,14 @@ __host__ __device__ inline MapStatsLayout map_stats_layout(int Cs, int Ci) {
     return l;
 }
 
+// Both statistics kernels read a label lab[m] per point (an instance, or an object of pag_map_components).  With unlabelled_ok a
+// label of -1 means "no object" and is skipped silently; any other label outside [0, Ci), or a class outside [0, Cs), is skipped and
+// counted in errors (nullable).  inst_out (nullable) receives, per label, inst_src of one of its points.
 __global__ void __launch_bounds__(MAP_STATS_BLOCK) map_instance_stats_kernel(
-        const float* __restrict__ xyz, const float* __restrict__ rgb, const int64_t* __restrict__ sem, const int64_t* __restrict__ inst,
-        int64_t P, int Cs, int Ci, uint32_t thing_mask, long long* __restrict__ count, double* __restrict__ sum_xyz,
-        double* __restrict__ sum_rgb, int64_t* __restrict__ votes, float* __restrict__ bbox_min, float* __restrict__ bbox_max,
-        long long* __restrict__ errors) {
+        const float* __restrict__ xyz, const float* __restrict__ rgb, const int64_t* __restrict__ sem, const int64_t* __restrict__ lab,
+        int64_t P, int Cs, int Ci, uint32_t thing_mask, int unlabelled_ok, const int64_t* __restrict__ inst_src,
+        int64_t* __restrict__ inst_out, long long* __restrict__ count, double* __restrict__ sum_xyz, double* __restrict__ sum_rgb,
+        int64_t* __restrict__ votes, float* __restrict__ bbox_min, float* __restrict__ bbox_max, long long* __restrict__ errors) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const MapStatsLayout l = map_stats_layout(Cs, Ci);
     double* s_xyz = reinterpret_cast<double*>(smem_raw + l.sum_xyz);
@@ -65,10 +69,12 @@ __global__ void __launch_bounds__(MAP_STATS_BLOCK) map_instance_stats_kernel(
     __syncthreads();
     unsigned n_bad = 0;
     for (int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; m < P; m += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t c = sem[m], q = inst[m];
+        const int64_t c = sem[m], q = lab[m];
+        if (q == -1 && unlabelled_ok) continue;
         if (c < 0 || c >= Cs || q < 0 || q >= Ci) { ++n_bad; continue; }
         if (!((thing_mask >> c) & 1u)) continue;
         const int i = (int)q;
+        if (inst_out && (m == 0 || lab[m - 1] != q)) inst_out[i] = inst_src[m];
         atomicAdd(s_cnt + i, 1u);
         atomicAdd(s_votes + i * Cs + (int)c, 1u);
 #pragma unroll
@@ -81,7 +87,7 @@ __global__ void __launch_bounds__(MAP_STATS_BLOCK) map_instance_stats_kernel(
         }
     }
     for (int o = 16; o > 0; o >>= 1) n_bad += __shfl_xor_sync(0xffffffffu, n_bad, o);
-    if ((threadIdx.x & 31) == 0 && n_bad) atomicAdd(reinterpret_cast<unsigned long long*>(errors), (unsigned long long)n_bad);
+    if ((threadIdx.x & 31) == 0 && n_bad && errors) atomicAdd(reinterpret_cast<unsigned long long*>(errors), (unsigned long long)n_bad);
     __syncthreads();
     for (int i = threadIdx.x; i < Ci; i += blockDim.x) {
         const unsigned int n = s_cnt[i];
@@ -101,6 +107,77 @@ __global__ void __launch_bounds__(MAP_STATS_BLOCK) map_instance_stats_kernel(
     }
 }
 
+// The same statistics accumulated straight into global memory, for label counts whose slots do not fit in shared memory.  Each
+// warp takes 32 consecutive points and reduces every run of equal labels (a segmented shuffle scan) before one set of atomics per
+// run: map points arrive in Morton cell order, so neighbouring lanes mostly share a label.
+__global__ void __launch_bounds__(MAP_STATS_BLOCK) map_instance_stats_global_kernel(
+        const float* __restrict__ xyz, const float* __restrict__ rgb, const int64_t* __restrict__ sem, const int64_t* __restrict__ lab,
+        int64_t P, int Cs, int Ci, uint32_t thing_mask, int unlabelled_ok, const int64_t* __restrict__ inst_src,
+        int64_t* __restrict__ inst_out, long long* __restrict__ count, double* __restrict__ sum_xyz, double* __restrict__ sum_rgb,
+        int64_t* __restrict__ votes, float* __restrict__ bbox_min, float* __restrict__ bbox_max, long long* __restrict__ errors) {
+    const unsigned FULL = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    const unsigned lanes_le = FULL >> (31 - lane);
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    unsigned n_bad = 0;
+    for (int64_t base = ((int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31)); base < P; base += nwarps * 32) {
+        const int64_t m = base + lane;
+        long long q = -1;      // -1: this lane adds nothing
+        int c = 0;
+        if (m < P) {
+            const int64_t c64 = sem[m], q64 = lab[m];
+            const bool unlabelled = q64 == -1 && unlabelled_ok;
+            const bool bad = !unlabelled && (c64 < 0 || c64 >= Cs || q64 < 0 || q64 >= Ci);
+            n_bad += bad;
+            if (!unlabelled && !bad && ((thing_mask >> c64) & 1u)) {
+                q = q64;
+                c = (int)c64;
+            }
+        }
+        double sx[3] = {0.0, 0.0, 0.0}, sr[3] = {0.0, 0.0, 0.0};
+        float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+        if (q >= 0) {
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                lo[a] = hi[a] = xyz[3 * m + a];
+                sx[a] = (double)lo[a];
+                sr[a] = (double)rgb[3 * m + a];
+            }
+        }
+        const long long qp = __shfl_up_sync(FULL, q, 1), qn = __shfl_down_sync(FULL, q, 1);
+        const bool head = lane == 0 || qp != q, tail = lane == 31 || qn != q;
+        const int h = 31 - __clz(__ballot_sync(FULL, head) & lanes_le);          // first lane of this lane's run
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const bool take = lane - o >= h;
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const double ux = __shfl_up_sync(FULL, sx[a], o), ur = __shfl_up_sync(FULL, sr[a], o);
+                const float ul = __shfl_up_sync(FULL, lo[a], o), uh = __shfl_up_sync(FULL, hi[a], o);
+                if (take) { sx[a] += ux; sr[a] += ur; lo[a] = fminf(lo[a], ul); hi[a] = fmaxf(hi[a], uh); }
+            }
+        }
+        if (tail && q >= 0) {      // the run's last lane holds its totals
+            atomicAdd(reinterpret_cast<unsigned long long*>(count + q), (unsigned long long)(lane - h + 1));
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                atomicAdd(sum_xyz + 3 * q + a, sx[a]);
+                atomicAdd(sum_rgb + 3 * q + a, sr[a]);
+                pag_atomic_min_f32(bbox_min + 3 * q + a, lo[a]);
+                pag_atomic_max_f32(bbox_max + 3 * q + a, hi[a]);
+            }
+            if (inst_out) inst_out[q] = inst_src[m];
+        }
+        // votes: runs of equal (label, class) inside the label's run; their lengths are the counts
+        const int cp = __shfl_up_sync(FULL, c, 1), cn = __shfl_down_sync(FULL, c, 1);
+        const bool head2 = head || cp != c, tail2 = tail || cn != c;
+        const int h2 = 31 - __clz(__ballot_sync(FULL, head2) & lanes_le);
+        if (tail2 && q >= 0) atomicAdd(reinterpret_cast<unsigned long long*>(votes + q * Cs + c), (unsigned long long)(lane - h2 + 1));
+    }
+    for (int o = 16; o > 0; o >>= 1) n_bad += __shfl_xor_sync(FULL, n_bad, o);
+    if (lane == 0 && n_bad && errors) atomicAdd(reinterpret_cast<unsigned long long*>(errors), (unsigned long long)n_bad);
+}
+
 static int map_num_sms() {
     static int n = 0;
     if (!n) {
@@ -111,6 +188,253 @@ static int map_num_sms() {
     }
     return n;
 }
+
+// ---- connected components of the map (pag_map_components) ----
+// Lattice index j per axis in [0, D), D = k << level, packed 21 bits per axis (D <= 2^18); hash key = packed + 1 (0 = empty slot).
+#define MAP_CC_BLOCK 256
+#define MAP_CC_SCAN_BLOCK 1024
+#define MAP_CC_AXIS_BITS 21
+
+struct CcWorkspace {      // layout in pag_map_components_workspace's comment (include/pagnerf_b200.h)
+    unsigned long long* table_key;
+    long long* key;       // per point: its hash key (0 = off the lattice); after the union step, the rank of each root
+    int64_t* boff;        // exclusive scan of bsum, nb + 1 entries
+    uint32_t* table_val;
+    int* parent;          // -1 for inactive points
+    int* count;
+    int* bsum;
+};
+
+static int64_t cc_blocks(int64_t P) { return (P + MAP_CC_SCAN_BLOCK - 1) / MAP_CC_SCAN_BLOCK; }
+
+static int64_t cc_workspace_bytes(int64_t P) {
+    const int64_t C = pag_hash_slots(P), nb = cc_blocks(P);
+    return 12 * C + 16 * P + 8 * (nb + 1) + 4 * nb;
+}
+
+static CcWorkspace cc_workspace(void* ws, int64_t P) {
+    const int64_t C = pag_hash_slots(P), nb = cc_blocks(P);
+    CcWorkspace w;
+    w.table_key = reinterpret_cast<unsigned long long*>(ws);
+    w.key = reinterpret_cast<long long*>(w.table_key + C);
+    w.boff = reinterpret_cast<int64_t*>(w.key + P);
+    w.table_val = reinterpret_cast<uint32_t*>(w.boff + nb + 1);
+    w.parent = reinterpret_cast<int*>(w.table_val + C);
+    w.count = w.parent + P;
+    w.bsum = w.count + P;
+    return w;
+}
+
+// lattice index of coordinate x, or -1 when x is not bit for bit fl(fl((2j+1)/D) - 1) for any j in [0, D).  For a lattice point
+// |x - ((2j+1)/D - 1)| <= 2^-23 + 2^-25 (one rounding of a value below 2, one of the subtraction), so (x+1) D / 2 - 1/2 lies
+// within D * 2^-24 * 1.25 <= 0.02 of j and rounding recovers it; the exact formula then decides.
+__device__ __forceinline__ int cc_lattice_index(float x, int D) {
+    const double t = ((double)x + 1.0) * (double)D * 0.5 - 0.5;
+    if (!(t > -0.5 && t < (double)D - 0.5)) return -1;
+    const int j = __double2int_rn(t);
+    const float y = __fsub_rn(__fdiv_rn((float)(2 * j + 1), (float)D), 1.0f);
+    return __float_as_uint(y) == __float_as_uint(x) ? j : -1;
+}
+
+__device__ __forceinline__ unsigned long long cc_key(int jx, int jy, int jz) {
+    return (((unsigned long long)jx << (2 * MAP_CC_AXIS_BITS)) | ((unsigned long long)jy << MAP_CC_AXIS_BITS) | (unsigned long long)jz) + 1ull;
+}
+
+// keys and insert: lattice recovery, label checks, active test, every on-lattice point into the table (key -> point index).
+// info[1] += points off the lattice, info[2] += points whose lattice index an earlier insert already holds, info[3] += points with
+// a label out of range.
+__global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_keys_kernel(const float* __restrict__ xyz, const int64_t* __restrict__ sem,
+                                                                   const int64_t* __restrict__ inst, int64_t P, int D, int Cs, int Ci,
+                                                                   uint32_t thing_mask, uint32_t C, CcWorkspace w,
+                                                                   long long* __restrict__ info) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool off = false, dup = false, bad = false;
+    if (i < P) {
+        int j[3];
+#pragma unroll
+        for (int a = 0; a < 3; ++a) j[a] = cc_lattice_index(xyz[3 * i + a], D);
+        off = j[0] < 0 || j[1] < 0 || j[2] < 0;
+        const int64_t c = sem[i], q = inst[i];
+        bad = c < 0 || c >= Cs || q < 0 || q >= Ci;
+        const bool active = !off && !bad && ((thing_mask >> c) & 1u);
+        unsigned long long key = 0ull;
+        if (!off) {
+            key = cc_key(j[0], j[1], j[2]);
+            bool inserted;
+            const uint32_t s = pag_hash_insert(w.table_key, C, key, &inserted);
+            if (inserted) w.table_val[s] = (uint32_t)i;
+            dup = !inserted;
+        }
+        w.key[i] = (long long)key;
+        w.parent[i] = active ? (int)i : -1;
+    }
+    const int lane = threadIdx.x & 31;
+    const unsigned n_off = __popc(__ballot_sync(0xffffffffu, off)), n_dup = __popc(__ballot_sync(0xffffffffu, dup)),
+                   n_bad = __popc(__ballot_sync(0xffffffffu, bad));
+    if (lane == 0) {
+        if (n_off) atomicAdd(reinterpret_cast<unsigned long long*>(info + 1), (unsigned long long)n_off);
+        if (n_dup) atomicAdd(reinterpret_cast<unsigned long long*>(info + 2), (unsigned long long)n_dup);
+        if (n_bad) atomicAdd(reinterpret_cast<unsigned long long*>(info + 3), (unsigned long long)n_bad);
+    }
+}
+
+// root of x with path halving.  parent[x] <= x always (links go from the larger root to the smaller index), so the walk ends at
+// the smallest point index of the tree.  volatile: the loads must see other threads' CAS results.
+__device__ __forceinline__ int cc_find(volatile int* parent, int x) {
+    int cur = parent[x];
+    if (cur != x) {
+        int next, prev = x;
+        while (cur > (next = parent[cur])) {
+            parent[prev] = next;
+            prev = cur;
+            cur = next;
+        }
+    }
+    return cur;
+}
+
+// root of x without writes: flatten stores each point's root while other threads walk through it, and a path-halving write
+// there could replace a stored root by an intermediate ancestor
+__device__ __forceinline__ int cc_root(volatile int* parent, int x) {
+    int p;
+    while ((p = parent[x]) != x) x = p;
+    return x;
+}
+
+// lock-free union (ECL-CC, Jaiganesh & Burtscher 2018): hook the larger root under the smaller with atomicCAS.  A failed CAS means
+// that root was hooked meanwhile: continue from the node it now points to.  a is the caller's representative of its own point,
+// kept across its neighbours; on return it is a node of the merged tree.
+__device__ __forceinline__ void cc_hook(int* parent, int& a, int b) {
+    while (a != b) {
+        if (a < b) {
+            const int r = atomicCAS(parent + b, b, a);
+            if (r == b) return;
+            b = r;
+        } else {
+            const int r = atomicCAS(parent + a, a, b);
+            a = r == a ? b : r;
+        }
+    }
+}
+
+// forward neighbour offsets (dx, dy, dz) > 0 lexicographically: each adjacent pair is visited once, from its smaller lattice index
+__constant__ signed char c_cc_fwd[13][3] = {{0, 0, 1},  {0, 1, -1}, {0, 1, 0},  {0, 1, 1},  {1, -1, -1}, {1, -1, 0}, {1, -1, 1},
+                                            {1, 0, -1}, {1, 0, 0},  {1, 0, 1},  {1, 1, -1}, {1, 1, 0},   {1, 1, 1}};
+
+__global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_union_kernel(const int64_t* __restrict__ inst, int64_t P, int D, int conn6,
+                                                                    uint32_t C, CcWorkspace w) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    volatile int* parent = w.parent;
+    if (parent[i] < 0) return;      // inactive
+    const unsigned long long k = (unsigned long long)w.key[i] - 1ull;
+    const unsigned mask = (1u << MAP_CC_AXIS_BITS) - 1u;
+    const int jx = (int)(k >> (2 * MAP_CC_AXIS_BITS)), jy = (int)((k >> MAP_CC_AXIS_BITS) & mask), jz = (int)(k & mask);
+    const int64_t q = inst[i];
+    int rep = cc_find(parent, (int)i);
+#pragma unroll
+    for (int o = 0; o < 13; ++o) {
+        const int dx = c_cc_fwd[o][0], dy = c_cc_fwd[o][1], dz = c_cc_fwd[o][2];
+        if (conn6 && abs(dx) + abs(dy) + abs(dz) != 1) continue;
+        const int nx = jx + dx, ny = jy + dy, nz = jz + dz;
+        if (nx >= D || ny < 0 || ny >= D || nz < 0 || nz >= D) continue;      // nx >= jx >= 0
+        const unsigned long long nk = cc_key(nx, ny, nz);
+        uint32_t s = pag_hash64(nk) & (C - 1);
+        int n = -1;
+        while (true) {
+            const unsigned long long cur = w.table_key[s];
+            if (cur == nk) { n = (int)w.table_val[s]; break; }
+            if (cur == 0ull) break;
+            s = (s + 1) & (C - 1);
+        }
+        if (n >= 0 && parent[n] >= 0 && inst[n] == q) cc_hook(w.parent, rep, cc_find(parent, n));
+    }
+}
+
+// parent[i] = root(i) and count[root] += 1 (lanes with the same root add once)
+__global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_flatten_kernel(int64_t P, CcWorkspace w) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int r = -1;
+    if (i < P && w.parent[i] >= 0) {
+        r = cc_root(w.parent, (int)i);
+        w.parent[i] = r;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, r);
+    if (r >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(w.count + r, __popc(peers));
+}
+
+__device__ __forceinline__ bool cc_kept_root(const CcWorkspace& w, int64_t i, int64_t min_points) {
+    return w.parent[i] == i && w.count[i] >= min_points;
+}
+
+// bsum[b] = number of kept roots among points [b * 1024, (b + 1) * 1024)
+__global__ void __launch_bounds__(MAP_CC_SCAN_BLOCK) map_cc_flags_kernel(int64_t P, int64_t min_points, CcWorkspace w) {
+    const int64_t i = (int64_t)blockIdx.x * MAP_CC_SCAN_BLOCK + threadIdx.x;
+    const int n = __syncthreads_count(i < P && cc_kept_root(w, i, min_points));
+    if (threadIdx.x == 0) w.bsum[blockIdx.x] = n;
+}
+
+// rank of each kept root = number of kept roots before it (block-local scan + boff); info[0] = K
+__global__ void __launch_bounds__(MAP_CC_SCAN_BLOCK) map_cc_rank_kernel(int64_t P, int64_t min_points, int64_t nb, CcWorkspace w,
+                                                                        long long* __restrict__ info) {
+    __shared__ int warp_tot[MAP_CC_SCAN_BLOCK / 32];
+    const int64_t i = (int64_t)blockIdx.x * MAP_CC_SCAN_BLOCK + threadIdx.x;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const bool flag = i < P && cc_kept_root(w, i, min_points);
+    const unsigned b = __ballot_sync(0xffffffffu, flag);
+    if (lane == 0) warp_tot[wid] = __popc(b);
+    __syncthreads();
+    if (wid == 0) {
+        const int v = warp_tot[lane];
+        int incl = v;
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += t;
+        }
+        warp_tot[lane] = incl - v;
+    }
+    __syncthreads();
+    if (flag) w.key[i] = w.boff[blockIdx.x] + warp_tot[wid] + __popc(b & ((1u << lane) - 1u));
+    if (i == 0) info[0] = w.boff[nb];
+}
+
+__global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_label_kernel(int64_t P, int64_t min_points, CcWorkspace w,
+                                                                    int64_t* __restrict__ component) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    const int r = w.parent[i];
+    component[i] = (r >= 0 && w.count[r] >= min_points) ? w.key[r] : -1;
+}
+
+static int map_stats_launch(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* lab, int64_t P, int Cs, int Ci,
+                            uint32_t thing_mask, int unlabelled_ok, const int64_t* inst_src, int64_t* inst_out, int64_t* count,
+                            double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min, float* bbox_max, int64_t* errors,
+                            cudaStream_t stream) {
+    // a few CTAs per SM: every CTA of the shared-memory kernel flushes its non-empty slots once, so fewer, longer-lived CTAs mean
+    // fewer global atomics
+    const int64_t want = pag_grid(P, MAP_STATS_BLOCK);
+    const int64_t cap = 4 * (int64_t)map_num_sms();
+    const int grid = (int)(want < cap ? want : cap);
+    const int64_t slot_bytes = 76 + 4 * (int64_t)Cs;      // map_stats_layout per label
+    if ((int64_t)Ci * slot_bytes <= 227 * 1024) {
+        const size_t bytes = (size_t)map_stats_layout(Cs, Ci).total;
+        if (bytes > 48 * 1024) {
+            cudaError_t e = cudaFuncSetAttribute(map_instance_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+            if (e != cudaSuccess) return (int)e;
+        }
+        map_instance_stats_kernel<<<grid, MAP_STATS_BLOCK, bytes, stream>>>(
+            xyz, rgb, semantic, lab, P, Cs, Ci, thing_mask, unlabelled_ok, inst_src, inst_out, reinterpret_cast<long long*>(count),
+            sum_xyz, sum_rgb, votes, bbox_min, bbox_max, reinterpret_cast<long long*>(errors));
+    } else {
+        map_instance_stats_global_kernel<<<(int)want, MAP_STATS_BLOCK, 0, stream>>>(
+            xyz, rgb, semantic, lab, P, Cs, Ci, thing_mask, unlabelled_ok, inst_src, inst_out, reinterpret_cast<long long*>(count),
+            sum_xyz, sum_rgb, votes, bbox_min, bbox_max, reinterpret_cast<long long*>(errors));
+    }
+    PAG_LAUNCH_CHECK();
+    return PAG_OK;
+}
+
+extern "C" int pag_exclusive_scan_i32(const int32_t* in, int64_t N, int64_t* out, void* stream);      // csrc/octree.cu
 
 extern "C" {
 
@@ -128,24 +452,64 @@ int pag_map_instance_stats(const float* xyz, const float* rgb, const int64_t* se
                            uint32_t thing_mask, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
                            float* bbox_max, int64_t* errors, void* stream) {
     if (P < 0 || Cs < 1 || Cs > 32 || Ci < 1) return PAG_ERR_ARG;
-    const size_t bytes = (size_t)map_stats_layout(Cs, Ci).total;
-    if (bytes > 227 * 1024) return PAG_ERR_UNSUPPORTED;
     if (P == 0) return PAG_OK;
     if (!xyz || !rgb || !semantic || !instance || !count || !sum_xyz || !sum_rgb || !votes || !bbox_min || !bbox_max || !errors)
         return PAG_ERR_ARG;
-    if (bytes > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(map_instance_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-        if (e != cudaSuccess) return (int)e;
-    }
-    // a few CTAs per SM: every CTA flushes its non-empty slots once, so fewer, longer-lived CTAs mean fewer global atomics
-    const int64_t want = pag_grid(P, MAP_STATS_BLOCK);
-    const int64_t cap = 4 * (int64_t)map_num_sms();
-    const int grid = (int)(want < cap ? want : cap);
-    map_instance_stats_kernel<<<grid, MAP_STATS_BLOCK, bytes, (cudaStream_t)stream>>>(
-        xyz, rgb, semantic, instance, P, Cs, Ci, thing_mask, reinterpret_cast<long long*>(count), sum_xyz, sum_rgb, votes, bbox_min,
-        bbox_max, reinterpret_cast<long long*>(errors));
+    return map_stats_launch(xyz, rgb, semantic, instance, P, Cs, Ci, thing_mask, 0, nullptr, nullptr, count, sum_xyz, sum_rgb, votes,
+                            bbox_min, bbox_max, errors, (cudaStream_t)stream);
+}
+
+int pag_map_components_workspace(int64_t P, int64_t* bytes) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || bytes == nullptr) return PAG_ERR_ARG;
+    *bytes = cc_workspace_bytes(P);
+    return PAG_OK;
+}
+
+int pag_map_components(const float* xyz, const int64_t* semantic, const int64_t* instance, int64_t P, int level, int k, int Cs, int Ci,
+                       uint32_t thing_mask, int connectivity, int64_t min_points, void* workspace, int64_t workspace_bytes,
+                       int64_t* component, int64_t* info, void* stream) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || level < 0 || level > 15 || k < 1 || k > 8 || Cs < 1 || Cs > 32 || Ci < 1) return PAG_ERR_ARG;
+    if ((connectivity != 6 && connectivity != 26) || min_points < 1 || !info) return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(info, 0, 4 * sizeof(int64_t), s);
+    if (e != cudaSuccess) return (int)e;
+    if (P == 0) return PAG_OK;
+    if (!xyz || !semantic || !instance || !component || !workspace || workspace_bytes < cc_workspace_bytes(P)) return PAG_ERR_ARG;
+    if (reinterpret_cast<uintptr_t>(workspace) & 7) return PAG_ERR_ARG;
+    const int64_t C = pag_hash_slots(P), nb = cc_blocks(P);
+    const CcWorkspace w = cc_workspace(workspace, P);
+    const int D = k << level;
+    long long* inf = reinterpret_cast<long long*>(info);
+    if ((e = cudaMemsetAsync(w.table_key, 0, C * sizeof(unsigned long long), s)) != cudaSuccess) return (int)e;
+    if ((e = cudaMemsetAsync(w.count, 0, P * sizeof(int), s)) != cudaSuccess) return (int)e;
+    const int g = pag_grid(P, MAP_CC_BLOCK);
+    map_cc_keys_kernel<<<g, MAP_CC_BLOCK, 0, s>>>(xyz, semantic, instance, P, D, Cs, Ci, thing_mask, (uint32_t)C, w, inf);
+    PAG_LAUNCH_CHECK();
+    map_cc_union_kernel<<<g, MAP_CC_BLOCK, 0, s>>>(instance, P, D, connectivity == 6, (uint32_t)C, w);
+    PAG_LAUNCH_CHECK();
+    map_cc_flatten_kernel<<<g, MAP_CC_BLOCK, 0, s>>>(P, w);
+    PAG_LAUNCH_CHECK();
+    map_cc_flags_kernel<<<(int)nb, MAP_CC_SCAN_BLOCK, 0, s>>>(P, min_points, w);
+    PAG_LAUNCH_CHECK();
+    const int rc = pag_exclusive_scan_i32(w.bsum, nb, w.boff, stream);
+    if (rc != PAG_OK) return rc;
+    map_cc_rank_kernel<<<(int)nb, MAP_CC_SCAN_BLOCK, 0, s>>>(P, min_points, nb, w, inf);
+    PAG_LAUNCH_CHECK();
+    map_cc_label_kernel<<<g, MAP_CC_BLOCK, 0, s>>>(P, min_points, w, component);
     PAG_LAUNCH_CHECK();
     return PAG_OK;
+}
+
+int pag_map_component_stats(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* instance, const int64_t* component,
+                            int64_t P, int Cs, int K, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
+                            float* bbox_max, int64_t* object_instance, void* stream) {
+    if (P < 0 || Cs < 1 || Cs > 32 || K < 0) return PAG_ERR_ARG;
+    if (P == 0 || K == 0) return PAG_OK;
+    if (!xyz || !rgb || !semantic || !instance || !component || !count || !sum_xyz || !sum_rgb || !votes || !bbox_min || !bbox_max ||
+        !object_instance)
+        return PAG_ERR_ARG;
+    return map_stats_launch(xyz, rgb, semantic, component, P, Cs, K, 0xffffffffu, 1, instance, object_instance, count, sum_xyz, sum_rgb,
+                            votes, bbox_min, bbox_max, nullptr, (cudaStream_t)stream);
 }
 
 }  // extern "C"

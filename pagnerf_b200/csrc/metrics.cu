@@ -16,7 +16,7 @@
 //              of its area counts as FP (prediction) or FN (target).  Clears the segment slot.
 // The workspace therefore starts and ends zeroed: the caller zero-fills it once and every update leaves it clean.
 //
-// Workspace of B images of P pixels, C = pag_pq_table_slots(P) = smallest power of two >= 2P slots per table (so that P distinct
+// Workspace of B images of P pixels, C = pag_hash_slots(P) = smallest power of two >= 2P slots per table (so that P distinct
 // segments -- every pixel its own segment -- fill at most half of a table: nothing overflows, whatever the data):
 //   u64 pred_key[B][C] | u64 tgt_key[B][C] | u64 pair_key[B][C] | u32 pred_area[B][C] | u32 pred_void[B][C] | u32 tgt_area[B][C]
 //   | u32 tgt_void[B][C] | u32 pair_cnt[B][C]                                           = 44 * B * C bytes (key 0 = empty slot)
@@ -27,12 +27,6 @@
 #define PQ_MAX_CATEGORIES 256
 #define PQ_HIST_BLOCK 256
 #define PQ_HIST_PIXELS_PER_THREAD 4
-
-static inline int64_t pq_table_slots(int64_t P) {
-    int64_t c = 2;
-    while (c < 2 * P) c <<= 1;
-    return c;
-}
 
 struct PqTables {
     unsigned long long *pred_key, *tgt_key, *pair_key;
@@ -52,23 +46,6 @@ static PqTables pq_tables(void* ws, int64_t n) {      // n = B * C slots per tab
     t.tgt_void = u + 3 * n;
     t.pair_cnt = u + 4 * n;
     return t;
-}
-
-__device__ __forceinline__ uint32_t pq_hash(unsigned long long k) {      // murmur3 fmix64
-    k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
-    return (uint32_t)k;
-}
-
-// slot of `key` in table[C] (C a power of two), inserted if absent.  A slot's key goes from 0 to its final value once, so a plain
-// load that sees the key (or another key) is final; a stale 0 only sends us to the CAS, which returns the truth.
-__device__ __forceinline__ uint32_t pq_insert(unsigned long long* __restrict__ table, uint32_t C, unsigned long long key) {
-    uint32_t s = pq_hash(key) & (C - 1);
-    while (true) {
-        unsigned long long cur = __ldcg(table + s);
-        if (cur == 0ull) cur = atomicCAS(table + s, 0ull, key);
-        if (cur == 0ull || cur == key) return s;
-        s = (s + 1) & (C - 1);
-    }
 }
 
 // -> continuous id | 0x100 if thing, or -1 if the category is unknown (sorted ids in shared memory, binary search)
@@ -107,7 +84,8 @@ __device__ __forceinline__ uint32_t pq_count(unsigned long long* __restrict__ ke
     const int leader = __ffs(peers) - 1;
     uint32_t slot = 0;
     if (key != 0ull && lane == leader) {
-        slot = pq_insert(keys, C, key);
+        bool inserted;
+        slot = pag_hash_insert(keys, C, key, &inserted);
         atomicAdd(area + slot, (unsigned)__popc(peers));
         if (voida != nullptr) {
             const unsigned nv = (unsigned)__popc(peers & void_mask);
@@ -214,7 +192,7 @@ __global__ void __launch_bounds__(256) pq_unmatched_kernel(PqTables t, int64_t n
 
 extern "C" int pag_pq_workspace(int64_t B, int64_t P, int64_t* bytes) {
     if (B < 1 || P < 1 || P > 0x40000000ll || bytes == nullptr) return PAG_ERR_ARG;
-    *bytes = 44 * B * pq_table_slots(P);
+    *bytes = 44 * B * pag_hash_slots(P);
     return PAG_OK;
 }
 
@@ -224,7 +202,7 @@ extern "C" int pag_pq_update(const int64_t* preds, const int64_t* target, int64_
     if (B < 1 || B > 65535 || P < 1 || P > 0x40000000ll || K < 1 || K > PQ_MAX_CATEGORIES) return PAG_ERR_ARG;
     if (!preds || !target || !cat_ids || !cat_code || !workspace || !iou_sum || !counts || !errors) return PAG_ERR_ARG;
     if ((reinterpret_cast<uintptr_t>(preds) | reinterpret_cast<uintptr_t>(target)) & 15) return PAG_ERR_ARG;
-    const int64_t C = pq_table_slots(P);
+    const int64_t C = pag_hash_slots(P);
     if (workspace_bytes < 44 * B * C || (reinterpret_cast<uintptr_t>(workspace) & 15)) return PAG_ERR_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t n = B * C;

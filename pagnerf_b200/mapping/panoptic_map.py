@@ -31,6 +31,29 @@ Definitions (the CPU oracle, oracle/mapping.py, and the tests follow them exactl
 
 instance_summary counts a point toward instance `inst` only when its semantic class is in `things` (every class when None), and
 returns centroid = sum_xyz / count in float64 (NaN where count == 0; bbox_min / bbox_max stay +inf / -inf there).
+
+instance_components splits the map into objects:
+
+    comps = instance_components(pts, samples_per_axis=2, level=nef.grid.blas_level, num_instances=nef.num_instances,
+                                num_classes=nef.num_classes, things={0}, connectivity=26, min_points=20)
+    comps.count.numel()             # number of objects; comps.component[i] = object of point i or -1
+
+  * Lattice.  D = k << level.  A point has lattice index j in [0, D)^3 iff each coordinate equals, bit for bit,
+    fl(fl((2j+1)/D) - 1) (the point formula above), so every map of extract_panoptic_map(nef, k) is on the lattice of
+    (k, nef.grid.blas_level).  Points off the lattice, and points whose lattice index another point has, raise ValueError with
+    their number.  xyz must be float32.
+  * Active points: semantic class in `things` (every class when None).  Labels outside [0, num_classes) / [0, num_instances) raise
+    ValueError with their number, as in instance_summary.
+  * Adjacency: two active points are adjacent iff their lattice indices differ by a vector of {-1,0,1}^3 \\ {0} (connectivity=26)
+    or by one unit step along one axis (connectivity=6), and their instance labels are equal.  Objects are the transitive closure.
+  * Numbering: objects of fewer than min_points points are dropped; their points and inactive points get component -1.  The others
+    are numbered 0..K-1 in the order of their smallest point index.  The result does not depend on thread scheduling, and the
+    partition does not depend on point order.
+  * Statistics per object: count, centroid = float64 sum / count, bbox_min / bbox_max in float32, mean_rgb (float64), votes
+    [K, num_classes], category = argmax of votes (lowest class on ties) and instance, the label the object's points share.
+  * Host reads: one per call (the error counts and K).  Device memory: at most 12 C + 24 P + 12 ceil(P / 1024) + 8 bytes for the
+    labelling (C = the smallest power of two >= 2P: a hash table of 12-byte slots, 16 bytes of workspace per point and the i64
+    component, so at most 72 bytes per point) plus (160 + 8 num_classes) bytes per object; 11.2 M points take 0.65 GB.
 """
 import math
 from typing import NamedTuple
@@ -45,6 +68,8 @@ from ..pc_nerf.panoptic_nef import _decoder_tensors
 MAX_SAMPLES_PER_AXIS = 8
 PRUNE_MIN_DENSITY = (0.01 * 512) / math.sqrt(3)      # PanopticNeF.prune()'s cell threshold
 MAX_SUMMARY_CLASSES = 32                             # thing mask: one bit per class
+MAX_LEVEL = 15                                       # pag_map_cell_points' octree levels
+MAX_COMPONENT_POINTS = 1 << 30                       # i32 union-find parents, u32 table values
 
 
 class PanopticPoints(NamedTuple):
@@ -55,6 +80,18 @@ class PanopticPoints(NamedTuple):
     semantic_score: torch.Tensor   # f32 [P]
     instance: torch.Tensor         # i64 [P]
     instance_score: torch.Tensor   # f32 [P]
+
+
+class InstanceComponents(NamedTuple):
+    component: torch.Tensor        # i64 [P]: object of each point, -1 if the point is in no object
+    count: torch.Tensor            # i64 [K]
+    instance: torch.Tensor         # i64 [K]: the instance label all points of the object share
+    category: torch.Tensor         # i64 [K]: argmax of votes (lowest class on ties)
+    centroid: torch.Tensor         # f64 [K, 3]
+    mean_rgb: torch.Tensor         # f64 [K, 3]
+    bbox_min: torch.Tensor         # f32 [K, 3]
+    bbox_max: torch.Tensor         # f32 [K, 3]
+    votes: torch.Tensor            # i64 [K, Cs]
 
 
 class InstanceSummary(NamedTuple):
@@ -140,20 +177,24 @@ def extract_panoptic_map(nef, samples_per_axis=2, min_density=None, view_dir=(0.
     return PanopticPoints(*(torch.cat(col) for col in zip(*parts)))
 
 
-def instance_summary(pts, num_instances, num_classes, things=None):
-    """Per-instance statistics of a labelled map (csrc/mapping.cu, one launch + one host read for the error count) -> InstanceSummary.
-    A point counts toward its instance only when its semantic class is in `things` (every class when None).  Raises ValueError if a
-    point carries a semantic label outside [0, num_classes) or an instance label outside [0, num_instances)."""
+def _thing_mask(num_instances, num_classes, things):
+    """-> (Ci, Cs, thing mask with one bit per class in `things`, every class when None)."""
     Ci, Cs = int(num_instances), int(num_classes)
     if Ci < 1 or not 1 <= Cs <= MAX_SUMMARY_CLASSES:
         raise ValueError(f"num_instances must be >= 1 and num_classes in [1, {MAX_SUMMARY_CLASSES}], got {Ci}, {Cs}")
     if things is None:
-        mask = (1 << Cs) - 1
-    else:
-        things = set(int(c) for c in things)
-        if not all(0 <= c < Cs for c in things):
-            raise ValueError(f"things must be classes in [0, {Cs}), got {sorted(things)}")
-        mask = sum(1 << c for c in things)
+        return Ci, Cs, (1 << Cs) - 1
+    things = set(int(c) for c in things)
+    if not all(0 <= c < Cs for c in things):
+        raise ValueError(f"things must be classes in [0, {Cs}), got {sorted(things)}")
+    return Ci, Cs, sum(1 << c for c in things)
+
+
+def instance_summary(pts, num_instances, num_classes, things=None):
+    """Per-instance statistics of a labelled map (csrc/mapping.cu, one launch + one host read for the error count) -> InstanceSummary.
+    A point counts toward its instance only when its semantic class is in `things` (every class when None).  Raises ValueError if a
+    point carries a semantic label outside [0, num_classes) or an instance label outside [0, num_instances)."""
+    Ci, Cs, mask = _thing_mask(num_instances, num_classes, things)
     if not pts.xyz.is_cuda:
         raise RuntimeError("pagnerf_b200 map export runs on CUDA tensors only (no CPU fallback)")
     count, sum_xyz, sum_rgb, votes, bmin, bmax, errors = ops.map_instance_stats(pts.xyz, pts.rgb, pts.semantic, pts.instance, Cs, Ci, mask)
@@ -165,17 +206,61 @@ def instance_summary(pts, num_instances, num_classes, things=None):
     return InstanceSummary(count, sum_xyz / n, bmin, bmax, sum_rgb / n, votes, category)
 
 
+def _is_int(v):
+    return not isinstance(v, bool) and isinstance(v, (int, np.integer))
+
+
+def instance_components(pts, samples_per_axis, level, num_instances, num_classes, things=None, connectivity=26, min_points=1):
+    """Objects of a labelled lattice map: connected components of equal instance labels (csrc/mapping.cu, one host read) ->
+    InstanceComponents.  See the module docstring for the exact definitions and the memory bound.  Raises ValueError for points off
+    the lattice of (samples_per_axis, level), for two points with the same lattice index and for out-of-range labels, with the
+    number of points affected."""
+    k = samples_per_axis
+    if not _is_int(k) or not 1 <= k <= MAX_SAMPLES_PER_AXIS:
+        raise ValueError(f"samples_per_axis must be an integer in [1, {MAX_SAMPLES_PER_AXIS}], got {k!r}")
+    if not _is_int(level) or not 0 <= level <= MAX_LEVEL:
+        raise ValueError(f"level must be an integer in [0, {MAX_LEVEL}], got {level!r}")
+    Ci, Cs, mask = _thing_mask(num_instances, num_classes, things)
+    if connectivity not in (6, 26) or isinstance(connectivity, bool):
+        raise ValueError(f"connectivity must be 6 or 26, got {connectivity!r}")
+    if not _is_int(min_points) or min_points < 1:
+        raise ValueError(f"min_points must be an integer >= 1, got {min_points!r}")
+    if not pts.xyz.is_cuda:
+        raise RuntimeError("pagnerf_b200 map export runs on CUDA tensors only (no CPU fallback)")
+    if pts.xyz.shape[0] > MAX_COMPONENT_POINTS:
+        raise ValueError(f"instance_components serves up to {MAX_COMPONENT_POINTS} points, got {pts.xyz.shape[0]}")
+    k, level = int(k), int(level)
+    component, info = ops.map_components(pts.xyz, pts.semantic, pts.instance, level, k, Cs, Ci, mask, int(connectivity),
+                                         int(min_points))
+    K, off, dup, bad = info.tolist()                # the call's one host read: the error counts and the output size
+    errors = []
+    if off:
+        errors.append(f"{off} points are not on the lattice of samples_per_axis={k}, level={level}")
+    if dup:
+        errors.append(f"{dup} points repeat the lattice index of another point")
+    if bad:
+        errors.append(f"{bad} points carry a semantic label outside [0, {Cs}) or an instance label outside [0, {Ci})")
+    if errors:
+        raise ValueError("; ".join(errors))
+    count, sum_xyz, sum_rgb, votes, bmin, bmax, inst = ops.map_component_stats(pts.xyz, pts.rgb, pts.semantic, pts.instance, component,
+                                                                              Cs, K)
+    n = count.to(torch.float64)[:, None]
+    return InstanceComponents(component, count, inst, votes.argmax(dim=1), sum_xyz / n, sum_rgb / n, bmin, bmax, votes)
+
+
 PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),
                   ("red", "uchar", "u1"), ("green", "uchar", "u1"), ("blue", "uchar", "u1"),
                   ("density", "float", "<f4"), ("semantic", "int", "<i4"), ("semantic_score", "float", "<f4"),
                   ("instance", "int", "<i4"), ("instance_score", "float", "<f4")]
 
 
-def write_ply(path, pts):
+def write_ply(path, pts, component=None):
     """Binary little-endian PLY of a map, one vertex per point: x y z (float), red green blue (uchar, round(255 * clamp(rgb, 0, 1))),
-    density, semantic (int), semantic_score, instance (int), instance_score."""
+    density, semantic (int), semantic_score, instance (int), instance_score, and with `component` (i64 [P], e.g.
+    InstanceComponents.component) a last int property `component`."""
     P = int(pts.xyz.shape[0])
-    rec = np.empty(P, dtype=[(n, t) for n, _, t in PLY_PROPERTIES])
+    props = PLY_PROPERTIES + ([("component", "int", "<i4")] if component is not None else [])
+    rec = np.empty(P, dtype=[(n, t) for n, _, t in props])
     xyz = pts.xyz.detach().cpu().numpy().astype(np.float32)
     rgb = np.rint(np.clip(pts.rgb.detach().cpu().numpy().astype(np.float64), 0.0, 1.0) * 255.0).astype(np.uint8)
     for i, n in enumerate("xyz"):
@@ -187,8 +272,12 @@ def write_ply(path, pts):
     rec["semantic_score"] = pts.semantic_score.detach().cpu().numpy()
     rec["instance"] = pts.instance.detach().cpu().numpy()
     rec["instance_score"] = pts.instance_score.detach().cpu().numpy()
+    if component is not None:
+        if tuple(component.shape) != (P,):
+            raise ValueError(f"component must have shape ({P},), got {tuple(component.shape)}")
+        rec["component"] = component.detach().cpu().numpy()
     header = ["ply", "format binary_little_endian 1.0", f"element vertex {P}"]
-    header += [f"property {t} {n}" for n, t, _ in PLY_PROPERTIES]
+    header += [f"property {t} {n}" for n, t, _ in props]
     header += ["end_header"]
     with open(path, "wb") as f:
         f.write(("\n".join(header) + "\n").encode("ascii"))

@@ -637,6 +637,43 @@ def map_instance_stats(xyz, rgb, semantic, instance, Cs, Ci, thing_mask):
     return count, sum_xyz, sum_rgb, votes, bmin, bmax, errors
 
 
+def map_components(xyz, semantic, instance, level, k, Cs, Ci, thing_mask, connectivity, min_points):
+    """Connected components of a labelled lattice map (xyz f32[P,3]; csrc/mapping.cu pag_map_components) -> component i64[P],
+    info i64[4] = (K, points off the lattice, duplicate points, points with an out-of-range label), both on the device."""
+    _chk(xyz, semantic, instance)
+    if xyz.dtype != torch.float32:
+        raise TypeError(f"map_components: xyz must be float32 (the lattice is defined bit for bit in fp32), got {xyz.dtype}")
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    s, q = semantic.to(torch.int64).contiguous(), instance.to(torch.int64).contiguous()
+    P = x.shape[0]
+    component = torch.empty(P, dtype=torch.int64, device=x.device)
+    info = torch.empty(4, dtype=torch.int64, device=x.device)
+    ws = _ws("pag_map_components_workspace", x.device, P)
+    call("pag_map_components", ptr(x), ptr(s), ptr(q), P, int(level), int(k), int(Cs), int(Ci), int(thing_mask) & 0xFFFFFFFF,
+         int(connectivity), int(min_points), *ws.args, ptr(component), ptr(info))
+    return component, info
+
+
+def map_component_stats(xyz, rgb, semantic, instance, component, Cs, K):
+    """Per-object statistics of map_components' labelling -> count i64[K], sum_xyz f64[K,3], sum_rgb f64[K,3], votes i64[K,Cs],
+    bbox_min / bbox_max f32[K,3], instance i64[K] (csrc/mapping.cu pag_map_component_stats)."""
+    _chk(xyz, rgb, semantic, instance, component)
+    dev = xyz.device
+    x, r = _f32(xyz).reshape(-1, 3), _f32(rgb).reshape(-1, 3)
+    s, q = semantic.to(torch.int64).contiguous(), instance.to(torch.int64).contiguous()
+    comp = component.to(torch.int64).contiguous()
+    count = torch.zeros(K, dtype=torch.int64, device=dev)
+    sum_xyz = torch.zeros(K, 3, dtype=torch.float64, device=dev)
+    sum_rgb = torch.zeros(K, 3, dtype=torch.float64, device=dev)
+    votes = torch.zeros(K, Cs, dtype=torch.int64, device=dev)
+    bmin = torch.full((K, 3), float('inf'), dtype=torch.float32, device=dev)
+    bmax = torch.full((K, 3), float('-inf'), dtype=torch.float32, device=dev)
+    inst = torch.empty(K, dtype=torch.int64, device=dev)
+    call("pag_map_component_stats", ptr(x), ptr(r), ptr(s), ptr(q), ptr(comp), x.shape[0], int(Cs), int(K), ptr(count), ptr(sum_xyz),
+         ptr(sum_rgb), ptr(votes), ptr(bmin), ptr(bmax), ptr(inst))
+    return count, sum_xyz, sum_rgb, votes, bmin, bmax, inst
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""
