@@ -420,6 +420,30 @@ int pag_map_components(const float* xyz, const int64_t* semantic, const int64_t*
 int pag_map_component_stats(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* instance, const int64_t* component,
                             int64_t P, int Cs, int K, int64_t* count, double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min,
                             float* bbox_max, int64_t* object_instance, void* stream);
+/* ---- lattice index of a map, and which map point / object a 3-D point or a rendered pixel lies on ----
+ * pag_map_index: every point of xyz f32[P,3] (on the lattice of (k, level), D = k << level, as for pag_map_components; labels are not
+ * read) into an open-addressing table: keys i64[C] (packed lattice index (jx << 42 | jy << 21 | jz) + 1, 0 = empty slot, linear
+ * probing from fmix64(key) & (C-1)) and points i32[C] (the point of each filled slot).  C = pag_map_index_bytes(P, &bytes) / 12 = the
+ * smallest power of two >= 2P; the call zero-fills keys itself.  info i64[4] (set by the call) = points inserted | points off the
+ * lattice | points repeating the lattice index of another point | 0; the index is meaningful only when the two counts are 0.  One
+ * launch, no host synchronisation; P <= 2^30.
+ * pag_map_lookup_points: per query xyz f32[Q,3], per axis in float64 with explicitly rounded operations: t = ((x + 1) D) 0.5 - 0.5,
+ * j0 = floor(t + 0.5).  point i64[Q] = the map point with lattice index j in [0, D)^3, |j - j0| <= radius per axis (radius in [0, 4])
+ * and the smallest ((tx-jx)^2 + (ty-jy)^2) + (tz-jz)^2, then the smallest point index; -1 with no candidate, for a non-finite
+ * coordinate and for t outside [-radius - 0.5, D - 0.5 + radius].  object i64[Q] (with component i64[P], nullable) = component[point],
+ * -1 where point is -1.
+ * pag_map_lookup_rays: the same for the surface point of each rendered ray: s = depth[i] / alpha[i] (fp32 IEEE), x = o + d s per axis
+ * (fp32, separately rounded mul and add); origins / dirs f32[Q,3], depth / alpha f32[Q].  Rays with alpha < min_alpha (min_alpha in
+ * (0, 1]) or a non-finite s get -1.
+ * Lookups: one launch each, geometry from (Q, radius) only, no host synchronisation (graph capturable), results independent of
+ * query order. */
+int pag_map_index_bytes(int64_t P, int64_t* bytes /* host */);
+int pag_map_index(const float* xyz, int64_t P, int level, int k, int64_t* keys, int32_t* points, int64_t C, int64_t* info, void* stream);
+int pag_map_lookup_points(const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* xyz, int64_t Q,
+                          int radius, const int64_t* component, int64_t* point, int64_t* object, void* stream);
+int pag_map_lookup_rays(const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* origins,
+                        const float* dirs, const float* depth, const float* alpha, float min_alpha, int64_t Q, int radius,
+                        const int64_t* component, int64_t* point, int64_t* object, void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

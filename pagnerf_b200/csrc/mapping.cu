@@ -240,6 +240,25 @@ __device__ __forceinline__ unsigned long long cc_key(int jx, int jy, int jz) {
     return (((unsigned long long)jx << (2 * MAP_CC_AXIS_BITS)) | ((unsigned long long)jy << MAP_CC_AXIS_BITS) | (unsigned long long)jz) + 1ull;
 }
 
+// lattice recovery of point i and its insert into the table (key -> point index), shared by the components and the map index.
+// Returns the point's hash key, 0 when it is off the lattice (*off); *dup: an earlier insert already holds its lattice index.
+__device__ __forceinline__ unsigned long long cc_insert_point(const float* __restrict__ xyz, int64_t i, int D,
+                                                              unsigned long long* __restrict__ table_key, uint32_t* __restrict__ table_val,
+                                                              uint32_t C, bool* off, bool* dup) {
+    int j[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) j[a] = cc_lattice_index(xyz[3 * i + a], D);
+    *off = j[0] < 0 || j[1] < 0 || j[2] < 0;
+    *dup = false;
+    if (*off) return 0ull;
+    const unsigned long long key = cc_key(j[0], j[1], j[2]);
+    bool inserted;
+    const uint32_t s = pag_hash_insert(table_key, C, key, &inserted);
+    if (inserted) table_val[s] = (uint32_t)i;
+    *dup = !inserted;
+    return key;
+}
+
 // keys and insert: lattice recovery, label checks, active test, every on-lattice point into the table (key -> point index).
 // info[1] += points off the lattice, info[2] += points whose lattice index an earlier insert already holds, info[3] += points with
 // a label out of range.
@@ -250,21 +269,10 @@ __global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_keys_kernel(const float* 
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     bool off = false, dup = false, bad = false;
     if (i < P) {
-        int j[3];
-#pragma unroll
-        for (int a = 0; a < 3; ++a) j[a] = cc_lattice_index(xyz[3 * i + a], D);
-        off = j[0] < 0 || j[1] < 0 || j[2] < 0;
+        const unsigned long long key = cc_insert_point(xyz, i, D, w.table_key, w.table_val, C, &off, &dup);
         const int64_t c = sem[i], q = inst[i];
         bad = c < 0 || c >= Cs || q < 0 || q >= Ci;
         const bool active = !off && !bad && ((thing_mask >> c) & 1u);
-        unsigned long long key = 0ull;
-        if (!off) {
-            key = cc_key(j[0], j[1], j[2]);
-            bool inserted;
-            const uint32_t s = pag_hash_insert(w.table_key, C, key, &inserted);
-            if (inserted) w.table_val[s] = (uint32_t)i;
-            dup = !inserted;
-        }
         w.key[i] = (long long)key;
         w.parent[i] = active ? (int)i : -1;
     }
@@ -406,6 +414,126 @@ __global__ void __launch_bounds__(MAP_CC_BLOCK) map_cc_label_kernel(int64_t P, i
     component[i] = (r >= 0 && w.count[r] >= min_points) ? w.key[r] : -1;
 }
 
+// ---- persistent lattice index of a map and lookups into it (pag_map_index, pag_map_lookup_points / _rays) ----
+// The index is the components' hash table alone: key u64[C] (packed lattice index + 1, 0 = empty) and point u32[C], C =
+// pag_hash_slots(P).  A lookup resolves a query position to the nearest map point of the (2r+1)^3 lattice window around it.
+#define MAP_LOOKUP_BLOCK 256
+#define MAP_LOOKUP_MAX_RADIUS 4
+
+// every point into the table; info[0] += points inserted, info[1] += points off the lattice, info[2] += repeated lattice indices
+__global__ void __launch_bounds__(MAP_CC_BLOCK) map_index_kernel(const float* __restrict__ xyz, int64_t P, int D, uint32_t C,
+                                                                 unsigned long long* __restrict__ table_key, uint32_t* __restrict__ table_val,
+                                                                 long long* __restrict__ info) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool off = false, dup = false;
+    if (i < P) cc_insert_point(xyz, i, D, table_key, table_val, C, &off, &dup);
+    const bool ins = i < P && !off && !dup;
+    const unsigned n_ins = __popc(__ballot_sync(0xffffffffu, ins)), n_off = __popc(__ballot_sync(0xffffffffu, off)),
+                   n_dup = __popc(__ballot_sync(0xffffffffu, dup));
+    if ((threadIdx.x & 31) == 0) {
+        if (n_ins) atomicAdd(reinterpret_cast<unsigned long long*>(info + 0), (unsigned long long)n_ins);
+        if (n_off) atomicAdd(reinterpret_cast<unsigned long long*>(info + 1), (unsigned long long)n_off);
+        if (n_dup) atomicAdd(reinterpret_cast<unsigned long long*>(info + 2), (unsigned long long)n_dup);
+    }
+}
+
+// lanes per query: the window offsets are spread over a group of G lanes, so a query's independent probes are in flight together
+// (one lane, one probe at radius 0; a warp of 32 from radius 1, 27 offsets, on)
+static int map_lookup_group(int radius) { return radius == 0 ? 1 : 32; }
+
+// One body for both query forms.  RAYS: the query is the surface point of a rendered ray, s = depth / alpha (IEEE fp32), x = o + d s
+// per axis (separately rounded mul and add, the marcher's sample-position convention); rays with alpha < min_alpha or a
+// non-finite s resolve to -1.  Otherwise the query is xyz.  Per axis in float64, every operation explicitly rounded:
+// t = ((x + 1) D) 0.5 - 0.5, window centre j0 = floor(t + 0.5); a non-finite x or t outside [-r - 0.5, D - 0.5 + r] resolves to -1.
+// Candidates: map points with lattice index j in [0, D)^3, |j - j0| <= r per axis; the chosen one has the smallest
+// ((tx-jx)^2 + (ty-jy)^2) + (tz-jz)^2, then the smallest point index: a total order, so the group's shuffle reduction is
+// deterministic.
+template <bool RAYS>
+__global__ void __launch_bounds__(MAP_LOOKUP_BLOCK) map_lookup_kernel(
+        const unsigned long long* __restrict__ table_key, const uint32_t* __restrict__ table_val, uint32_t C, int D,
+        const float* __restrict__ xyz, const float* __restrict__ dirs, const float* __restrict__ depth, const float* __restrict__ alpha,
+        float min_alpha, int64_t Q, int radius, int G, const int64_t* __restrict__ component, int64_t* __restrict__ point,
+        int64_t* __restrict__ object) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t q = tid / G;
+    const int sub = (int)(tid - q * G);
+    bool ok = q < Q;
+    float x[3] = {0.f, 0.f, 0.f};
+    if (ok) {
+        if (RAYS) {
+            const float a = alpha[q];
+            const float s = __fdiv_rn(depth[q], a);
+            ok = a >= min_alpha && isfinite(s);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) x[c] = __fadd_rn(xyz[3 * q + c], __fmul_rn(dirs[3 * q + c], s));
+        } else {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) x[c] = xyz[3 * q + c];
+        }
+    }
+    const double lo = -(double)radius - 0.5, hi = ((double)D - 0.5) + (double)radius;
+    double t[3];
+    int j0[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        t[c] = __dsub_rn(__dmul_rn(__dmul_rn(__dadd_rn((double)x[c], 1.0), (double)D), 0.5), 0.5);
+        ok = ok && t[c] >= lo && t[c] <= hi;      // false for NaN; an infinite x gives an infinite t
+        j0[c] = ok ? (int)floor(__dadd_rn(t[c], 0.5)) : 0;
+    }
+    double best_d = INFINITY;
+    uint32_t best_p = 0xffffffffu;
+    if (ok) {
+        const int w = 2 * radius + 1, W = w * w * w;
+        for (int o = sub; o < W; o += G) {
+            const int jx = j0[0] + o / (w * w) - radius, jy = j0[1] + (o / w) % w - radius, jz = j0[2] + o % w - radius;
+            if ((unsigned)jx >= (unsigned)D || (unsigned)jy >= (unsigned)D || (unsigned)jz >= (unsigned)D) continue;
+            const unsigned long long key = cc_key(jx, jy, jz);
+            uint32_t s = pag_hash64(key) & (C - 1);
+            unsigned long long cur;
+            while ((cur = __ldg(table_key + s)) != key && cur != 0ull) s = (s + 1) & (C - 1);
+            if (cur == 0ull) continue;
+            const uint32_t p = __ldg(table_val + s);
+            const double dx = __dsub_rn(t[0], (double)jx), dy = __dsub_rn(t[1], (double)jy), dz = __dsub_rn(t[2], (double)jz);
+            const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+            if (d2 < best_d || (d2 == best_d && p < best_p)) { best_d = d2; best_p = p; }
+        }
+    }
+    for (int m = G >> 1; m > 0; m >>= 1) {      // G = 32: the group is the warp, every lane takes part
+        const double od = __shfl_xor_sync(0xffffffffu, best_d, m);
+        const uint32_t op = __shfl_xor_sync(0xffffffffu, best_p, m);
+        if (od < best_d || (od == best_d && op < best_p)) { best_d = od; best_p = op; }
+    }
+    if (q < Q && sub == 0) {
+        const int64_t p = best_p == 0xffffffffu ? -1 : (int64_t)best_p;
+        point[q] = p;
+        if (object) object[q] = p >= 0 ? component[p] : -1;
+    }
+}
+
+static int map_lookup_launch(bool rays, const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* xyz,
+                             const float* dirs, const float* depth, const float* alpha, float min_alpha, int64_t Q, int radius,
+                             const int64_t* component, int64_t* point, int64_t* object, cudaStream_t s) {
+    if (C < 2 || C > (1ll << 31) || (C & (C - 1)) || Q < 0 || level < 0 || level > 15 || k < 1 || k > 8 || radius < 0 ||
+        radius > MAP_LOOKUP_MAX_RADIUS)
+        return PAG_ERR_ARG;
+    if (rays && !(min_alpha > 0.f && min_alpha <= 1.f)) return PAG_ERR_ARG;
+    if (Q == 0) return PAG_OK;
+    if (!keys || !points || !xyz || !point || (rays && (!dirs || !depth || !alpha))) return PAG_ERR_ARG;
+    const int G = map_lookup_group(radius);
+    const int64_t blocks = (Q * G + MAP_LOOKUP_BLOCK - 1) / MAP_LOOKUP_BLOCK;
+    if (blocks > 0x7fffffff) return PAG_ERR_ARG;
+    const unsigned long long* tk = reinterpret_cast<const unsigned long long*>(keys);
+    const uint32_t* tv = reinterpret_cast<const uint32_t*>(points);
+    if (rays)
+        map_lookup_kernel<true><<<(unsigned)blocks, MAP_LOOKUP_BLOCK, 0, s>>>(tk, tv, (uint32_t)C, k << level, xyz, dirs, depth, alpha,
+                                                                              min_alpha, Q, radius, G, component, point, object);
+    else
+        map_lookup_kernel<false><<<(unsigned)blocks, MAP_LOOKUP_BLOCK, 0, s>>>(tk, tv, (uint32_t)C, k << level, xyz, nullptr, nullptr,
+                                                                               nullptr, 1.f, Q, radius, G, component, point, object);
+    PAG_LAUNCH_CHECK();
+    return PAG_OK;
+}
+
 static int map_stats_launch(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* lab, int64_t P, int Cs, int Ci,
                             uint32_t thing_mask, int unlabelled_ok, const int64_t* inst_src, int64_t* inst_out, int64_t* count,
                             double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min, float* bbox_max, int64_t* errors,
@@ -510,6 +638,41 @@ int pag_map_component_stats(const float* xyz, const float* rgb, const int64_t* s
         return PAG_ERR_ARG;
     return map_stats_launch(xyz, rgb, semantic, component, P, Cs, K, 0xffffffffu, 1, instance, object_instance, count, sum_xyz, sum_rgb,
                             votes, bbox_min, bbox_max, nullptr, (cudaStream_t)stream);
+}
+
+int pag_map_index_bytes(int64_t P, int64_t* bytes) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || bytes == nullptr) return PAG_ERR_ARG;
+    *bytes = 12 * pag_hash_slots(P);
+    return PAG_OK;
+}
+
+int pag_map_index(const float* xyz, int64_t P, int level, int k, int64_t* keys, int32_t* points, int64_t C, int64_t* info,
+                  void* stream) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || level < 0 || level > 15 || k < 1 || k > 8 || !info || !keys || !points) return PAG_ERR_ARG;
+    if (C != pag_hash_slots(P) || (P > 0 && !xyz)) return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(info, 0, 4 * sizeof(int64_t), s);
+    if (e != cudaSuccess) return (int)e;
+    if ((e = cudaMemsetAsync(keys, 0, C * sizeof(int64_t), s)) != cudaSuccess) return (int)e;
+    if (P == 0) return PAG_OK;
+    map_index_kernel<<<pag_grid(P, MAP_CC_BLOCK), MAP_CC_BLOCK, 0, s>>>(xyz, P, k << level, (uint32_t)C,
+                                                                       reinterpret_cast<unsigned long long*>(keys),
+                                                                       reinterpret_cast<uint32_t*>(points), reinterpret_cast<long long*>(info));
+    PAG_LAUNCH_CHECK();
+    return PAG_OK;
+}
+
+int pag_map_lookup_points(const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* xyz, int64_t Q,
+                          int radius, const int64_t* component, int64_t* point, int64_t* object, void* stream) {
+    return map_lookup_launch(false, keys, points, C, level, k, xyz, nullptr, nullptr, nullptr, 1.f, Q, radius, component, point, object,
+                             (cudaStream_t)stream);
+}
+
+int pag_map_lookup_rays(const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* origins,
+                        const float* dirs, const float* depth, const float* alpha, float min_alpha, int64_t Q, int radius,
+                        const int64_t* component, int64_t* point, int64_t* object, void* stream) {
+    return map_lookup_launch(true, keys, points, C, level, k, origins, dirs, depth, alpha, min_alpha, Q, radius, component, point, object,
+                             (cudaStream_t)stream);
 }
 
 }  // extern "C"

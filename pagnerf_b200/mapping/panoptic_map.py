@@ -54,9 +54,37 @@ instance_components splits the map into objects:
   * Host reads: one per call (the error counts and K).  Device memory: at most 12 C + 24 P + 12 ceil(P / 1024) + 8 bytes for the
     labelling (C = the smallest power of two >= 2P: a hash table of 12-byte slots, 16 bytes of workspace per point and the i64
     component, so at most 72 bytes per point) plus (160 + 8 num_classes) bytes per object; 11.2 M points take 0.65 GB.
+
+map_index, lookup_points and lookup_rays answer which map point, and so which object, a 3-D point or a rendered pixel lies on:
+
+    index = map_index(pts, samples_per_axis=2, level=nef.grid.blas_level)               # MapIndex; one host read (error counts)
+    hit = lookup_points(index, xyz, radius=1, component=comps.component)                # MapLookup(point i64[Q], object i64[Q])
+    hit = lookup_rays(index, rays.origins, rays.dirs, rb.depth, rb.alpha, radius=1, min_alpha=0.5, component=comps.component)
+
+  * Index.  The lattice rules of instance_components (D = k << level; every point on the lattice bit for bit, no two points with one
+    lattice index, else ValueError with the same messages; xyz float32, P <= 2^30).  Labels are not read: every map point is
+    indexed, stuff and floater points included, so a leaf in front of a fruit resolves to the leaf, not to the fruit behind it.
+  * Query position.  Per axis, in float64 with explicitly rounded operations (no FMA contraction): t = ((x + 1) * D) * 0.5 - 0.5,
+    window centre j0 = floor(t + 0.5).
+  * Candidates.  Map points whose lattice index j lies in [0, D)^3 and differs from j0 by at most `radius` (an integer in [0, 4])
+    per axis.
+  * Choice.  The candidate with the smallest ((tx-jx)^2 + (ty-jy)^2) + (tz-jz)^2 (float64, in this order, no FMA), then the
+    smallest point index; point = -1 with no candidate, for a non-finite coordinate, and for t outside
+    [-radius - 0.5, D - 0.5 + radius] in any axis.
+  * Object.  object = component[point] where point >= 0, else -1 (so floaters and inactive points give -1 with a valid point);
+    component must have shape [P] of the indexed map.  Without component, MapLookup.object is None.
+  * Rays.  The surface point of a rendered ray, in fp32 with IEEE rounding: s = depth / alpha, then x = o + d * s per axis as a
+    separately rounded mul and add (the marcher's sample-position convention).  Rays with alpha < min_alpha (min_alpha in (0, 1],
+    compared in fp32) or a non-finite s give -1; a ray with alpha == min_alpha is looked up.  depth and alpha may be [N] or [N, 1],
+    as the tracer returns them.
+  * Host traffic.  Lookups make no host read and no host synchronisation; their launch geometry depends on Q and radius only, so
+    they can be captured in a CUDA graph.  The result depends only on the inputs: the same for any query order and on every run.
+  * Memory.  The index is the table alone: 12 C bytes (u64 key + u32 point per slot, C = the smallest power of two >= 2P), plus
+    the 4-entry info tensor; 2^25 slots, about 0.4 GB, for the 11.2 M points of a k = 4 map.  A lookup allocates only its outputs
+    (16 bytes per query with component, 8 without) when its inputs are contiguous.
 """
 import math
-from typing import NamedTuple
+from typing import NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -70,6 +98,7 @@ PRUNE_MIN_DENSITY = (0.01 * 512) / math.sqrt(3)      # PanopticNeF.prune()'s cel
 MAX_SUMMARY_CLASSES = 32                             # thing mask: one bit per class
 MAX_LEVEL = 15                                       # pag_map_cell_points' octree levels
 MAX_COMPONENT_POINTS = 1 << 30                       # i32 union-find parents, u32 table values
+MAX_LOOKUP_RADIUS = 4                                # a (2r+1)^3 window: 729 probes per query at most
 
 
 class PanopticPoints(NamedTuple):
@@ -92,6 +121,19 @@ class InstanceComponents(NamedTuple):
     bbox_min: torch.Tensor         # f32 [K, 3]
     bbox_max: torch.Tensor         # f32 [K, 3]
     votes: torch.Tensor            # i64 [K, Cs]
+
+
+class MapIndex(NamedTuple):
+    keys: torch.Tensor             # i64 [C]: packed lattice index + 1 per slot, 0 = empty (C = the smallest power of two >= 2P)
+    points: torch.Tensor           # i32 [C]: the map point of each filled slot
+    k: int                         # samples_per_axis of the map's lattice
+    level: int
+    P: int                         # points of the indexed map
+
+
+class MapLookup(NamedTuple):
+    point: torch.Tensor                    # i64 [Q]: the nearest map point in the window, -1 if none
+    object: Optional[torch.Tensor]         # i64 [Q]: component[point], -1 where there is no point or it is in no object
 
 
 class InstanceSummary(NamedTuple):
@@ -210,16 +252,29 @@ def _is_int(v):
     return not isinstance(v, bool) and isinstance(v, (int, np.integer))
 
 
+def _check_lattice(k, level):
+    if not _is_int(k) or not 1 <= k <= MAX_SAMPLES_PER_AXIS:
+        raise ValueError(f"samples_per_axis must be an integer in [1, {MAX_SAMPLES_PER_AXIS}], got {k!r}")
+    if not _is_int(level) or not 0 <= level <= MAX_LEVEL:
+        raise ValueError(f"level must be an integer in [0, {MAX_LEVEL}], got {level!r}")
+
+
+def _lattice_errors(off, dup, k, level):
+    errors = []
+    if off:
+        errors.append(f"{off} points are not on the lattice of samples_per_axis={k}, level={level}")
+    if dup:
+        errors.append(f"{dup} points repeat the lattice index of another point")
+    return errors
+
+
 def instance_components(pts, samples_per_axis, level, num_instances, num_classes, things=None, connectivity=26, min_points=1):
     """Objects of a labelled lattice map: connected components of equal instance labels (csrc/mapping.cu, one host read) ->
     InstanceComponents.  See the module docstring for the exact definitions and the memory bound.  Raises ValueError for points off
     the lattice of (samples_per_axis, level), for two points with the same lattice index and for out-of-range labels, with the
     number of points affected."""
     k = samples_per_axis
-    if not _is_int(k) or not 1 <= k <= MAX_SAMPLES_PER_AXIS:
-        raise ValueError(f"samples_per_axis must be an integer in [1, {MAX_SAMPLES_PER_AXIS}], got {k!r}")
-    if not _is_int(level) or not 0 <= level <= MAX_LEVEL:
-        raise ValueError(f"level must be an integer in [0, {MAX_LEVEL}], got {level!r}")
+    _check_lattice(k, level)
     Ci, Cs, mask = _thing_mask(num_instances, num_classes, things)
     if connectivity not in (6, 26) or isinstance(connectivity, bool):
         raise ValueError(f"connectivity must be 6 or 26, got {connectivity!r}")
@@ -233,11 +288,7 @@ def instance_components(pts, samples_per_axis, level, num_instances, num_classes
     component, info = ops.map_components(pts.xyz, pts.semantic, pts.instance, level, k, Cs, Ci, mask, int(connectivity),
                                          int(min_points))
     K, off, dup, bad = info.tolist()                # the call's one host read: the error counts and the output size
-    errors = []
-    if off:
-        errors.append(f"{off} points are not on the lattice of samples_per_axis={k}, level={level}")
-    if dup:
-        errors.append(f"{dup} points repeat the lattice index of another point")
+    errors = _lattice_errors(off, dup, k, level)
     if bad:
         errors.append(f"{bad} points carry a semantic label outside [0, {Cs}) or an instance label outside [0, {Ci})")
     if errors:
@@ -246,6 +297,97 @@ def instance_components(pts, samples_per_axis, level, num_instances, num_classes
                                                                               Cs, K)
     n = count.to(torch.float64)[:, None]
     return InstanceComponents(component, count, inst, votes.argmax(dim=1), sum_xyz / n, sum_rgb / n, bmin, bmax, votes)
+
+
+def _hash_slots(P):
+    """C of the index table: the smallest power of two >= 2P (at least 2), include/pagnerf_b200.h pag_map_index_bytes"""
+    return max(2, 1 << (2 * P - 1).bit_length()) if P > 0 else 2
+
+
+def _check_tensor(name, t, shapes, dtype):
+    """t must be a tensor of one of `shapes` (None = any size on that axis) and of `dtype`"""
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name} must be a tensor, got {type(t).__name__}")
+    ok = any(t.dim() == len(s) and all(w is None or t.shape[i] == w for i, w in enumerate(s)) for s in shapes)
+    if not ok:
+        want = " or ".join("[" + ", ".join("N" if w is None else str(w) for w in s) + "]" for s in shapes)
+        raise ValueError(f"{name} must have shape {want}, got {list(t.shape)}")
+    if t.dtype != dtype:
+        raise TypeError(f"{name} must be {dtype}, got {t.dtype}")
+
+
+def map_index(pts, samples_per_axis, level):
+    """Lattice index of a map (csrc/mapping.cu, one launch + one host read for the error counts) -> MapIndex.  pts: PanopticPoints or
+    its xyz f32 [P, 3].  Every point is indexed, whatever its labels.  Raises ValueError for points off the lattice of
+    (samples_per_axis, level) and for two points with the same lattice index, with their number.  See the module docstring for the
+    definitions and the memory bound (12 C bytes)."""
+    k = samples_per_axis
+    _check_lattice(k, level)
+    xyz = pts.xyz if isinstance(pts, PanopticPoints) else pts
+    _check_tensor("xyz", xyz, [(None, 3)], torch.float32)
+    P = int(xyz.shape[0])
+    if P > MAX_COMPONENT_POINTS:
+        raise ValueError(f"map_index serves up to {MAX_COMPONENT_POINTS} points, got {P}")
+    if not xyz.is_cuda:
+        raise RuntimeError("pagnerf_b200 map lookups run on CUDA tensors only (no CPU fallback)")
+    k, level = int(k), int(level)
+    keys, points, info = ops.map_index(xyz, level, k)
+    _, off, dup, _ = info.tolist()                  # the call's one host read: the error counts
+    errors = _lattice_errors(off, dup, k, level)
+    if errors:
+        raise ValueError("; ".join(errors))
+    return MapIndex(keys, points, k, level, P)
+
+
+def _check_lookup(index, radius, component):
+    if not isinstance(index, MapIndex):
+        raise TypeError(f"index must be a MapIndex (map_index), got {type(index).__name__}")
+    C = _hash_slots(index.P)
+    if index.keys.shape != (C,) or index.points.shape != (C,) or index.keys.dtype != torch.int64 or index.points.dtype != torch.int32:
+        raise ValueError(f"index is not the table of a {index.P}-point map: keys / points must be int64 / int32 [{C}]")
+    if not _is_int(radius) or not 0 <= radius <= MAX_LOOKUP_RADIUS:
+        raise ValueError(f"radius must be an integer in [0, {MAX_LOOKUP_RADIUS}], got {radius!r}")
+    if component is not None:
+        if not isinstance(component, torch.Tensor) or tuple(component.shape) != (index.P,):
+            shape = list(component.shape) if isinstance(component, torch.Tensor) else type(component).__name__
+            raise ValueError(f"component must have shape [{index.P}] (the indexed map's points), got {shape}")
+        if component.dtype != torch.int64:
+            raise TypeError(f"component must be torch.int64, got {component.dtype}")
+
+
+def _check_cuda(*tensors):
+    if not all(t.is_cuda for t in tensors if t is not None):
+        raise RuntimeError("pagnerf_b200 map lookups run on CUDA tensors only (no CPU fallback)")
+
+
+def lookup_points(index, xyz, radius=1, component=None):
+    """Nearest map point in the (2 radius + 1)^3 lattice window around each query xyz f32 [Q, 3], and its object when component
+    (i64 [P], e.g. InstanceComponents.component) is given -> MapLookup (csrc/mapping.cu, one launch, no host read).  See the module
+    docstring for the exact definitions."""
+    _check_lookup(index, radius, component)
+    _check_tensor("xyz", xyz, [(None, 3)], torch.float32)
+    _check_cuda(index.keys, index.points, xyz, component)
+    point, obj = ops.map_lookup_points(index.keys, index.points, index.level, index.k, xyz, int(radius), component)
+    return MapLookup(point, obj)
+
+
+def lookup_rays(index, origins, dirs, depth, alpha, radius=1, min_alpha=0.5, component=None):
+    """lookup_points for the surface point o + d * (depth / alpha) of each rendered ray (origins / dirs f32 [N, 3], depth / alpha
+    f32 [N] or [N, 1], e.g. a tracer's rb.depth / rb.alpha); rays with alpha < min_alpha resolve to -1 -> MapLookup (one launch,
+    no host read)."""
+    _check_lookup(index, radius, component)
+    if isinstance(min_alpha, bool) or not isinstance(min_alpha, (int, float, np.integer, np.floating)) or \
+            not (0.0 < float(np.float32(min_alpha)) and float(min_alpha) <= 1.0):
+        raise ValueError(f"min_alpha must be a number in (0, 1], got {min_alpha!r}")
+    _check_tensor("origins", origins, [(None, 3)], torch.float32)
+    N = int(origins.shape[0])
+    _check_tensor("dirs", dirs, [(N, 3)], torch.float32)
+    _check_tensor("depth", depth, [(N,), (N, 1)], torch.float32)
+    _check_tensor("alpha", alpha, [(N,), (N, 1)], torch.float32)
+    _check_cuda(index.keys, index.points, origins, dirs, depth, alpha, component)
+    point, obj = ops.map_lookup_rays(index.keys, index.points, index.level, index.k, origins, dirs, depth, alpha, float(min_alpha),
+                                     int(radius), component)
+    return MapLookup(point, obj)
 
 
 PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),

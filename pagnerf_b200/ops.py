@@ -674,6 +674,49 @@ def map_component_stats(xyz, rgb, semantic, instance, component, Cs, K):
     return count, sum_xyz, sum_rgb, votes, bmin, bmax, inst
 
 
+def map_index(xyz, level, k):
+    """Lattice index of a map (xyz f32[P,3]; csrc/mapping.cu pag_map_index) -> keys i64[C], points i32[C], info i64[4] = (points
+    inserted, points off the lattice, duplicate points), all on the device.  Allocates the 12 C-byte table and info only."""
+    _chk(xyz)
+    if xyz.dtype != torch.float32:
+        raise TypeError(f"map_index: xyz must be float32 (the lattice is defined bit for bit in fp32), got {xyz.dtype}")
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    P = x.shape[0]
+    C = query_i64("pag_map_index_bytes", P) // 12
+    keys = torch.empty(C, dtype=torch.int64, device=x.device)
+    points = torch.empty(C, dtype=torch.int32, device=x.device)
+    info = torch.empty(4, dtype=torch.int64, device=x.device)
+    call("pag_map_index", ptr(x), P, int(level), int(k), ptr(keys), ptr(points), C, ptr(info))
+    return keys, points, info
+
+
+def map_lookup_points(keys, points, level, k, xyz, radius, component=None):
+    """Nearest map point (and its component) of each query xyz f32[Q,3] in a map_index table (csrc/mapping.cu
+    pag_map_lookup_points) -> point i64[Q], object i64[Q] or None.  Allocates the outputs only (for contiguous inputs)."""
+    _chk(keys, points, xyz, component)
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    Q = x.shape[0]
+    point = torch.empty(Q, dtype=torch.int64, device=x.device)
+    obj = torch.empty(Q, dtype=torch.int64, device=x.device) if component is not None else None
+    call("pag_map_lookup_points", ptr(keys), ptr(points), keys.numel(), int(level), int(k), ptr(x), Q, int(radius),
+         ptr(component), ptr(point), ptr(obj))
+    return point, obj
+
+
+def map_lookup_rays(keys, points, level, k, origins, dirs, depth, alpha, min_alpha, radius, component=None):
+    """map_lookup_points for the surface point o + d (depth / alpha) of each rendered ray (origins / dirs f32[Q,3], depth / alpha
+    f32[Q]; csrc/mapping.cu pag_map_lookup_rays); rays with alpha < min_alpha resolve to -1."""
+    _chk(keys, points, origins, dirs, depth, alpha, component)
+    o, d = origins.detach().reshape(-1, 3).contiguous(), dirs.detach().reshape(-1, 3).contiguous()
+    t, a = depth.detach().reshape(-1).contiguous(), alpha.detach().reshape(-1).contiguous()
+    Q = o.shape[0]
+    point = torch.empty(Q, dtype=torch.int64, device=o.device)
+    obj = torch.empty(Q, dtype=torch.int64, device=o.device) if component is not None else None
+    call("pag_map_lookup_rays", ptr(keys), ptr(points), keys.numel(), int(level), int(k), ptr(o), ptr(d), ptr(t), ptr(a),
+         float(min_alpha), Q, int(radius), ptr(component), ptr(point), ptr(obj))
+    return point, obj
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""
