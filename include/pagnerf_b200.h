@@ -388,6 +388,23 @@ int pag_pq_update(const int64_t* preds, const int64_t* target, int64_t B, int64_
                   int K, int allow_unknown_preds, void* workspace, int64_t workspace_bytes, double* iou_sum, int64_t* counts,
                   int64_t* errors, void* stream);
 
+/* ---- scene-level panoptic quality on the device: one segment per id across all frames of a sequence ----
+ * Same rules as the per-image update above (evaluate_metrics, pc_nerf/trainer.py:651-941, scores each image on its own), applied to
+ * ONE image made of every pixel of every update: tables that persist across updates.  Three open-addressing tables (prediction
+ * segments, target segments, same-category pairs) of C = smallest power of two >= 2 * capacity slots, u64 areas; each admits at most
+ * `capacity` keys and counts the pixels of refused keys; capacity in [1, 2^26].  workspace: pag_scene_pq_workspace(capacity, &bytes)
+ * bytes = 64 * C + 128, zero-filled by the caller ONCE; it persists across updates (layout and counters in csrc/metrics.cu).
+ * update: preds / target i64[N, 2] (all pixels of the call), 16-byte aligned, categories as pag_pq_update; errors i64[2] as there.
+ *         One launch, no host synchronisation, geometry from N only.
+ * stats:  accumulates iou_sum f64[K] and counts i64[3][K] (tp | fp | fn) of the scene so far into caller-zeroed arrays; two launches;
+ *         the tables are left as found.
+ * merge:  inserts another workspace of the same capacity (another rank's tables) into `workspace`; two launches. */
+int pag_scene_pq_workspace(int64_t capacity, int64_t* bytes /* host */);
+int pag_scene_pq_update(const int64_t* preds, const int64_t* target, int64_t N, const int32_t* cat_ids, const int32_t* cat_code, int K,
+                        int allow_unknown_preds, void* workspace, int64_t capacity, int64_t workspace_bytes, int64_t* errors, void* stream);
+int pag_scene_pq_stats(void* workspace, int64_t capacity, int64_t workspace_bytes, int K, double* iou_sum, int64_t* counts, void* stream);
+int pag_scene_pq_merge(void* workspace, const void* other, int64_t capacity, int64_t workspace_bytes, void* stream);
+
 /* ---- panoptic point-map export (utils/render_map.py: the nef evaluated on the occupied octree cells, labelled, exported) ----
  * pag_map_cell_points: cells i16[C,3] (leaf cells of `level`, e.g. the octree's level points) -> xyz f32[C*k^3, 3], k in [1, 8]:
  * sub-point s = (ix*k + iy)*k + iz of cell c at row c*k^3 + s, coordinate (2*(p*k + i) + 1) / (k << level) - 1 in fp32 (IEEE division).
