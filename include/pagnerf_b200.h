@@ -461,6 +461,20 @@ int pag_map_lookup_points(const int64_t* keys, const int32_t* points, int64_t C,
 int pag_map_lookup_rays(const int64_t* keys, const int32_t* points, int64_t C, int level, int k, const float* origins,
                         const float* dirs, const float* depth, const float* alpha, float min_alpha, int64_t Q, int radius,
                         const int64_t* component, int64_t* point, int64_t* object, void* stream);
+/* ---- projection of a map into camera views: which map point, at what depth, and which object each pixel sees ----
+ * pag_map_project: xyz f32[P,3] (P <= 2^30), view f32[B,4,4] world-to-camera (rows 0..2 read), intrinsics f32[B,4] = (fx, fy, cx, cy)
+ * in pixels; the camera looks down -z, pixel (row r, column c) has the camera-space direction ((c + 0.5 - cx) / fx,
+ * (r + 0.5 - cy) / fy, -1).  In fp32, every operation separately rounded: p_q = ((V[q,0] x + V[q,1] y) + V[q,2] z) + V[q,3],
+ * z = -p_2, u = fx (p_0 / z) + cx, v = fy (p_1 / z) + cy, su = min((fx h) / z, max_radius), sv = min((fy h) / z, max_radius) (h =
+ * the lattice half-size 1 / D, passed by the caller).  A point is splatted iff z > near, u and v are finite and su, sv >= 0 (false
+ * for NaN); it covers columns floor(u - su) .. floor(u + su) and rows floor(v - sv) .. floor(v + sv), clipped to the image.  Each
+ * pixel keeps the covering point of smallest z, then of smallest index: point i64[B,H,W] (-1 if none), depth f32[B,H,W] (+inf if
+ * none), object i64[B,H,W] = component[point] (object nullable; component i64[P] required with object when P > 0; -1 where point is -1).  zbuf u64[B*H*W]:
+ * caller-owned depth buffer, filled by the call.  B <= 65535, H and W in [1, 16384], max_radius in [0, 32], near > 0.  A fill and
+ * two launches, geometry from (P, B, H, W) only, no host synchronisation (graph capturable), deterministic. */
+int pag_map_project(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h, float near,
+                    int max_radius, int64_t* zbuf, const int64_t* component, int64_t* point, float* depth, int64_t* object,
+                    void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

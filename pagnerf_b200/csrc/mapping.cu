@@ -534,6 +534,75 @@ static int map_lookup_launch(bool rays, const int64_t* keys, const int32_t* poin
     return PAG_OK;
 }
 
+// ---- projection of a map into camera views (pag_map_project): z-buffered splatting of the lattice cells' squares ----
+// The depth buffer holds one u64 key per pixel, (z bits << 32) | point, all ones where nothing is seen.  z > near > 0, so the float
+// bits order like the values and the smallest key is the nearest point, then the smallest point index.
+#define MAP_PROJECT_BLOCK 256
+#define MAP_PROJECT_MAX_RADIUS 32
+#define MAP_PROJECT_MAX_SIDE 16384
+#define MAP_PROJECT_MAX_CAMERAS 65535      // gridDim.y
+#define MAP_PROJECT_EMPTY 0xffffffffffffffffull
+
+// One thread per (point, camera): grid x over points, y over cameras.  Every operation is separately rounded (the oracle's numpy
+// order): p_q = ((V[q,0] x + V[q,1] y) + V[q,2] z) + V[q,3], depth z = -p_2, u = fx (p_0 / z) + cx, v = fy (p_1 / z) + cy,
+// su = min((fx h) / z, R), sv likewise.  A point is splatted iff z > near, u and v are finite and su, sv >= 0 (false for NaN, so
+// a NaN half-size never becomes R, and a negative focal length covers nothing).  Pixels: columns floor(u - su) .. floor(u + su),
+// rows floor(v - sv) .. floor(v + sv), clamped to the image in float before the conversion to int.  Each pixel is tested with a
+// plain load of its current key and takes an atomicMin only when the new key is smaller: the atomic decides, the load only skips
+// the atomics that cannot win (points arrive in leaf-cell order, so a warp's squares overlap and the skipped atomics would
+// serialise on one address).
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_splat_kernel(
+        const float* __restrict__ xyz, int64_t P, const float* __restrict__ view, const float* __restrict__ intrinsics, int H, int W,
+        float h, float near, int max_radius, unsigned long long* __restrict__ zbuf) {
+    __shared__ float s_cam[16];          // rows 0..2 of the view matrix, then fx, fy, cx, cy
+    const int b = blockIdx.y;
+    if (threadIdx.x < 12) s_cam[threadIdx.x] = view[16 * (int64_t)b + threadIdx.x];
+    else if (threadIdx.x < 16) s_cam[threadIdx.x] = intrinsics[4 * (int64_t)b + threadIdx.x - 12];
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    const float x = xyz[3 * i], y = xyz[3 * i + 1], zw = xyz[3 * i + 2];
+    float p[3];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) {
+        const float* V = s_cam + 4 * q;
+        p[q] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(V[0], x), __fmul_rn(V[1], y)), __fmul_rn(V[2], zw)), V[3]);
+    }
+    const float fx = s_cam[12], fy = s_cam[13], cx = s_cam[14], cy = s_cam[15];
+    const float z = -p[2];
+    if (!(z > near)) return;
+    const float u = __fadd_rn(__fmul_rn(fx, __fdiv_rn(p[0], z)), cx), v = __fadd_rn(__fmul_rn(fy, __fdiv_rn(p[1], z)), cy);
+    const float ru = __fdiv_rn(__fmul_rn(fx, h), z), rv = __fdiv_rn(__fmul_rn(fy, h), z);
+    if (!isfinite(u) || !isfinite(v) || !(ru >= 0.f) || !(rv >= 0.f)) return;
+    const float R = (float)max_radius;
+    const float su = fminf(ru, R), sv = fminf(rv, R);
+    const float c0f = fmaxf(floorf(__fsub_rn(u, su)), 0.f), c1f = fminf(floorf(__fadd_rn(u, su)), (float)(W - 1));
+    const float r0f = fmaxf(floorf(__fsub_rn(v, sv)), 0.f), r1f = fminf(floorf(__fadd_rn(v, sv)), (float)(H - 1));
+    if (c0f > c1f || r0f > r1f) return;
+    const int c0 = (int)c0f, c1 = (int)c1f, r0 = (int)r0f, r1 = (int)r1f;
+    const unsigned long long key = ((unsigned long long)__float_as_uint(z) << 32) | (unsigned long long)i;
+    unsigned long long* img = zbuf + (int64_t)b * H * W;
+    for (int r = r0; r <= r1; ++r) {
+        unsigned long long* row = img + (int64_t)r * W;
+        for (int c = c0; c <= c1; ++c)
+            if (key < __ldcg(row + c)) atomicMin(row + c, key);
+    }
+}
+
+// one thread per pixel: the key's point and depth, and component[point] (component nullable)
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_resolve_kernel(
+        const unsigned long long* __restrict__ zbuf, int64_t N, const int64_t* __restrict__ component, int64_t* __restrict__ point,
+        float* __restrict__ depth, int64_t* __restrict__ object) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= N) return;
+    const unsigned long long key = zbuf[t];
+    const bool hit = key != MAP_PROJECT_EMPTY;
+    const int64_t p = hit ? (int64_t)(key & 0xffffffffull) : -1;
+    point[t] = p;
+    depth[t] = hit ? __uint_as_float((uint32_t)(key >> 32)) : INFINITY;
+    if (object) object[t] = hit ? component[p] : -1;
+}
+
 static int map_stats_launch(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* lab, int64_t P, int Cs, int Ci,
                             uint32_t thing_mask, int unlabelled_ok, const int64_t* inst_src, int64_t* inst_out, int64_t* count,
                             double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min, float* bbox_max, int64_t* errors,
@@ -673,6 +742,33 @@ int pag_map_lookup_rays(const int64_t* keys, const int32_t* points, int64_t C, i
                         const int64_t* component, int64_t* point, int64_t* object, void* stream) {
     return map_lookup_launch(true, keys, points, C, level, k, origins, dirs, depth, alpha, min_alpha, Q, radius, component, point, object,
                              (cudaStream_t)stream);
+}
+
+int pag_map_project(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h, float near,
+                    int max_radius, int64_t* zbuf, const int64_t* component, int64_t* point, float* depth, int64_t* object,
+                    void* stream) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || B < 0 || B > MAP_PROJECT_MAX_CAMERAS || H < 1 || H > MAP_PROJECT_MAX_SIDE || W < 1 ||
+        W > MAP_PROJECT_MAX_SIDE || max_radius < 0 || max_radius > MAP_PROJECT_MAX_RADIUS || !(near > 0.f) || !isfinite(near) ||
+        !(h > 0.f) || !isfinite(h))
+        return PAG_ERR_ARG;
+    if (B == 0) return PAG_OK;
+    // an empty map's xyz and component may be null (torch gives an empty tensor no storage): no pixel is covered, nothing is read
+    if (!view || !intrinsics || !zbuf || !point || !depth || (P > 0 && (!xyz || (object && !component)))) return PAG_ERR_ARG;
+    const int64_t N = (int64_t)B * H * W;
+    if ((N + MAP_PROJECT_BLOCK - 1) / MAP_PROJECT_BLOCK > 0x7fffffff) return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(zbuf, 0xff, N * sizeof(int64_t), s);
+    if (e != cudaSuccess) return (int)e;
+    unsigned long long* zb = reinterpret_cast<unsigned long long*>(zbuf);
+    if (P > 0) {
+        map_project_splat_kernel<<<dim3((unsigned)pag_grid(P, MAP_PROJECT_BLOCK), (unsigned)B), MAP_PROJECT_BLOCK, 0, s>>>(
+            xyz, P, view, intrinsics, H, W, h, near, max_radius, zb);
+        PAG_LAUNCH_CHECK();
+    }
+    map_project_resolve_kernel<<<(unsigned)pag_grid(N, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(zb, N, component, point, depth,
+                                                                                                      object);
+    PAG_LAUNCH_CHECK();
+    return PAG_OK;
 }
 
 }  // extern "C"

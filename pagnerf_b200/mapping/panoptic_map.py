@@ -82,6 +82,35 @@ map_index, lookup_points and lookup_rays answer which map point, and so which ob
   * Memory.  The index is the table alone: 12 C bytes (u64 key + u32 point per slot, C = the smallest power of two >= 2P), plus
     the 4-entry info tensor; 2^25 slots, about 0.4 GB, for the 11.2 M points of a k = 4 map.  A lookup allocates only its outputs
     (16 bytes per query with component, 8 without) when its inputs are contiguous.
+
+project_map answers, from the map alone, which map point, at what depth and which object each pixel of a camera sees:
+
+    mv = project_map(pts, samples_per_axis=2, level=nef.grid.blas_level, view=V, intrinsics=K, height=H, width=W,
+                     component=comps.component)                                         # MapView(point, depth, object), [B, H, W]
+
+  * Cameras.  view f32 [B, 4, 4] world-to-camera matrices (BAPipeline's and bench.make_cameras' layout; rows 0..2 are read),
+    intrinsics f32 [B, 4] = (fx, fy, cx, cy) in pixels, both CUDA tensors.  The camera looks down its -z axis; the pixel in column c
+    and row r has the camera-space ray direction ((c + 0.5 - cx) / fx, (r + 0.5 - cy) / fy, -1), rows growing with +y (the
+    convention of bench.make_frame_rays).
+  * Arithmetic.  fp32, every operation separately rounded (no FMA contraction), in the order written.
+  * Transform.  Per row q of view: p_q = ((V[q,0] x + V[q,1] y) + V[q,2] z) + V[q,3]; the point's depth is z = -p_2.
+  * Pixel position.  u = fx (p_0 / z) + cx, v = fy (p_1 / z) + cy (the division, then the product, then the sum).
+  * Footprint.  A map point stands for its lattice cell, of half-size h = fl(1 / D), D = samples_per_axis << level (exact when
+    samples_per_axis is a power of two).  Half-sizes in pixels su = min((fx h) / z, max_radius), sv = min((fy h) / z, max_radius),
+    NaN propagating.  The point covers every pixel the closed square [u - su, u + su] x [v - sv, v + sv] touches: columns
+    floor(u - su) .. floor(u + su), rows floor(v - sv) .. floor(v + sv), clipped to the image.  With max_radius = 0 a point covers
+    exactly the pixel containing (u, v).  max_radius is an integer in [0, 32]; a point tests at most (2 max_radius + 2)^2 pixels
+    (2 max_radius + 1 per axis but for the rounding of u +- su).
+  * Dropped points.  A point is projected only if z > near, u and v are finite and su >= 0 and sv >= 0 (false for NaN; a negative
+    focal length gives an empty square).  Floors are clamped to the image in float before the conversion to an integer, so a point
+    far off-screen cannot overflow it.  Camera values are not validated (that would be a host read); they are used as defined here.
+  * Visibility.  Each pixel gets the covering point with the smallest z, then the smallest point index, whatever the thread schedule.
+  * Outputs.  point i64 [B, H, W] (-1 where no point covers the pixel), depth f32 [B, H, W] (its z, +inf where point == -1) and, with
+    component (i64 [P], e.g. InstanceComponents.component), object = component[point], -1 where point == -1.
+  * Lattice.  (samples_per_axis, level) only set the footprint; the points need not lie on the lattice and are not checked.
+  * Limits.  P <= 2^30, B <= 65535, height and width integers in [1, 16384], near a finite number > 0 (also in fp32).
+  * Host traffic.  None: the launch geometry depends on P, B, H, W and max_radius only, so the call can be captured in a CUDA graph.
+  * Memory.  The outputs and a u64 depth buffer of B H W entries: 28 bytes per pixel with component, 20 without.
 """
 import math
 from typing import NamedTuple, Optional
@@ -99,6 +128,9 @@ MAX_SUMMARY_CLASSES = 32                             # thing mask: one bit per c
 MAX_LEVEL = 15                                       # pag_map_cell_points' octree levels
 MAX_COMPONENT_POINTS = 1 << 30                       # i32 union-find parents, u32 table values
 MAX_LOOKUP_RADIUS = 4                                # a (2r+1)^3 window: 729 probes per query at most
+MAX_PROJECT_RADIUS = 32                              # a footprint of at most 66 x 66 pixels
+MAX_PROJECT_SIDE = 16384
+MAX_PROJECT_CAMERAS = 65535                          # one grid row per camera
 
 
 class PanopticPoints(NamedTuple):
@@ -134,6 +166,12 @@ class MapIndex(NamedTuple):
 class MapLookup(NamedTuple):
     point: torch.Tensor                    # i64 [Q]: the nearest map point in the window, -1 if none
     object: Optional[torch.Tensor]         # i64 [Q]: component[point], -1 where there is no point or it is in no object
+
+
+class MapView(NamedTuple):
+    point: torch.Tensor                    # i64 [B, H, W]: the visible map point of each pixel, -1 if none
+    depth: torch.Tensor                    # f32 [B, H, W]: its camera-space depth z (> near), +inf where point == -1
+    object: Optional[torch.Tensor]         # i64 [B, H, W]: component[point], -1 where point == -1 or the point is in no object
 
 
 class InstanceSummary(NamedTuple):
@@ -388,6 +426,45 @@ def lookup_rays(index, origins, dirs, depth, alpha, radius=1, min_alpha=0.5, com
     point, obj = ops.map_lookup_rays(index.keys, index.points, index.level, index.k, origins, dirs, depth, alpha, float(min_alpha),
                                      int(radius), component)
     return MapLookup(point, obj)
+
+
+def project_map(pts, samples_per_axis, level, view, intrinsics, height, width, max_radius=8, near=0.01, component=None):
+    """Z-buffered splatting of a map's points into B camera views (view f32 [B, 4, 4] world-to-camera, intrinsics f32 [B, 4] =
+    (fx, fy, cx, cy)): per pixel the nearest covering map point, its depth and, with component (i64 [P]), its object -> MapView of
+    [B, height, width] tensors (csrc/mapping.cu, a fill and two launches, no host read).  pts: PanopticPoints or its xyz f32 [P, 3].
+    See the module docstring for the exact definitions."""
+    k = samples_per_axis
+    _check_lattice(k, level)
+    xyz = pts.xyz if isinstance(pts, PanopticPoints) else pts
+    _check_tensor("xyz", xyz, [(None, 3)], torch.float32)
+    P = int(xyz.shape[0])
+    if P > MAX_COMPONENT_POINTS:
+        raise ValueError(f"project_map serves up to {MAX_COMPONENT_POINTS} points, got {P}")
+    _check_tensor("view", view, [(None, 4, 4)], torch.float32)
+    B = int(view.shape[0])
+    if B > MAX_PROJECT_CAMERAS:
+        raise ValueError(f"project_map serves up to {MAX_PROJECT_CAMERAS} cameras per call, got {B}")
+    _check_tensor("intrinsics", intrinsics, [(B, 4)], torch.float32)
+    for name, n in (("height", height), ("width", width)):
+        if not _is_int(n) or not 1 <= n <= MAX_PROJECT_SIDE:
+            raise ValueError(f"{name} must be an integer in [1, {MAX_PROJECT_SIDE}], got {n!r}")
+    if not _is_int(max_radius) or not 0 <= max_radius <= MAX_PROJECT_RADIUS:
+        raise ValueError(f"max_radius must be an integer in [0, {MAX_PROJECT_RADIUS}], got {max_radius!r}")
+    if isinstance(near, bool) or not isinstance(near, (int, float, np.integer, np.floating)) or \
+            not (np.isfinite(np.float32(near)) and np.float32(near) > 0):
+        raise ValueError(f"near must be a finite number > 0, got {near!r}")
+    if component is not None:
+        if not isinstance(component, torch.Tensor) or tuple(component.shape) != (P,):
+            shape = list(component.shape) if isinstance(component, torch.Tensor) else type(component).__name__
+            raise ValueError(f"component must have shape [{P}] (the projected map's points), got {shape}")
+        if component.dtype != torch.int64:
+            raise TypeError(f"component must be torch.int64, got {component.dtype}")
+    if not all(t.is_cuda for t in (xyz, view, intrinsics, component) if t is not None):
+        raise RuntimeError("pagnerf_b200 map projection runs on CUDA tensors only (no CPU fallback)")
+    h = float(np.float32(1.0) / np.float32(int(k) << int(level)))
+    point, depth, obj = ops.map_project(xyz, view, intrinsics, int(height), int(width), h, float(np.float32(near)), int(max_radius),
+                                        component)
+    return MapView(point, depth, obj)
 
 
 PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),

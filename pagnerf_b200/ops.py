@@ -717,6 +717,24 @@ def map_lookup_rays(keys, points, level, k, origins, dirs, depth, alpha, min_alp
     return point, obj
 
 
+def map_project(xyz, view, intrinsics, H, W, h, near, max_radius, component=None):
+    """Z-buffered splatting of the map points xyz f32[P,3] into B views (view f32[B,4,4], intrinsics f32[B,4]; csrc/mapping.cu
+    pag_map_project) -> point i64[B,H,W], depth f32[B,H,W], object i64[B,H,W] or None.  Allocates the u64 depth buffer and the
+    outputs only (for contiguous inputs)."""
+    _chk(xyz, view, intrinsics, component)
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    V, K = view.detach().contiguous(), intrinsics.detach().contiguous()
+    B = V.shape[0]
+    dev = x.device
+    zbuf = torch.empty(B * H * W, dtype=torch.int64, device=dev)
+    point = torch.empty(B, H, W, dtype=torch.int64, device=dev)
+    depth = torch.empty(B, H, W, dtype=torch.float32, device=dev)
+    obj = torch.empty(B, H, W, dtype=torch.int64, device=dev) if component is not None else None
+    call("pag_map_project", ptr(x), x.shape[0], ptr(V), ptr(K), B, int(H), int(W), float(h), float(near), int(max_radius), ptr(zbuf),
+         ptr(component), ptr(point), ptr(depth), ptr(obj))
+    return point, depth, obj
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""
