@@ -475,6 +475,27 @@ int pag_map_lookup_rays(const int64_t* keys, const int32_t* points, int64_t C, i
 int pag_map_project(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h, float near,
                     int max_radius, int64_t* zbuf, const int64_t* component, int64_t* point, float* depth, int64_t* object,
                     void* stream);
+/* ---- per-object visibility of a map in camera views: visible area, unoccluded silhouette and visible box per (view, object) ----
+ * Cameras, footprints and the front point of each pixel exactly as pag_map_project; component i64[P] (required when P > 0), K
+ * objects (K <= 2^30), N = B K pairs n = b K + o.  Points with component -1 occlude but own no pair; components outside [-1, K) are
+ * skipped and counted.  Two calls, with one host read between them:
+ * pag_map_visibility: fills the depth buffer zbuf u64[B*H*W] (not read, may be null, when P = 0) and splats the map (pag_map_project's kernel), then writes
+ * visible i64[N] (pixels whose front point has object o), bbox i32[N,4] = (col_min, row_min, col_max, row_max) of those pixels
+ * (-1s where visible is 0), box i32[N,4] (the union of the footprints of the pair's points, clipped to the image; (2^31-1,
+ * 2^31-1, -1, -1) when empty), words i32[N] (the size of the pair's silhouette bitmap: box rows times the 32-bit words of the
+ * image its columns touch) and offset i64[N+2]: exclusive scan of words (offset[N] = total words) and offset[N+1] = points with a
+ * component outside [-1, K).  Sets silhouette i64[N] to 0.  Five launches and a scan, no host synchronisation.
+ * pag_map_visibility_silhouette: silhouette[n] = pixels covered by a footprint of the pair's points, at any depth: the pairs'
+ * bitmaps are OR-splatted in rounds into bits i32[bits_words] and popcounted.  A round takes the pairs whose offset lies in
+ * [lo, lo + step), step = total_words when it fits bits_words, else bits_words - H ceil(W / 32) (the largest bitmap), which must be
+ * > 0.  Two launches and a fill per round. */
+int pag_map_visibility(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h, float near,
+                       int max_radius, const int64_t* component, int K, int64_t* zbuf, int32_t* box, int32_t* words, int64_t* offset,
+                       int64_t* visible, int64_t* silhouette, int32_t* bbox, void* stream);
+int pag_map_visibility_silhouette(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h,
+                                  float near, int max_radius, const int64_t* component, int K, const int32_t* box, const int32_t* words,
+                                  const int64_t* offset, int64_t total_words, int32_t* bits, int64_t bits_words, int64_t* silhouette,
+                                  void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

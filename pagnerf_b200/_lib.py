@@ -23,6 +23,9 @@ KERNELS_PER_CALL = {
     "pag_march_ray_count": 2, "pag_march_ray_bits_count": 2, "pag_compact_count": 2, "pag_raytrace_count": 2, "pag_voxel_filter_count": 2, "pag_voxel_filter_count_staged": 2, "pag_raytrace_stage": 4, "pag_octree_from_mask": 12, "pag_adam_step": 2, "pag_pan_composite_bwd_tc": 2, "pag_decode_dc_bwd_tc_dyn": 2,
     "pag_pq_update": 3, "pag_map_components": 7, "pag_scene_pq_stats": 2, "pag_scene_pq_merge": 2,
     "pag_map_project": 2,
+    # at most: pag_map_visibility skips the splat and the per-pixel kernel for an empty map and the pair kernels without pairs;
+    # pag_map_visibility_silhouette launches 2 kernels (and a fill) per round, the figure is for one round
+    "pag_map_visibility": 6, "pag_map_visibility_silhouette": 2,
 }
 launch_count = 0
 

@@ -543,24 +543,25 @@ static int map_lookup_launch(bool rays, const int64_t* keys, const int32_t* poin
 #define MAP_PROJECT_MAX_CAMERAS 65535      // gridDim.y
 #define MAP_PROJECT_EMPTY 0xffffffffffffffffull
 
-// One thread per (point, camera): grid x over points, y over cameras.  Every operation is separately rounded (the oracle's numpy
-// order): p_q = ((V[q,0] x + V[q,1] y) + V[q,2] z) + V[q,3], depth z = -p_2, u = fx (p_0 / z) + cx, v = fy (p_1 / z) + cy,
-// su = min((fx h) / z, R), sv likewise.  A point is splatted iff z > near, u and v are finite and su, sv >= 0 (false for NaN, so
-// a NaN half-size never becomes R, and a negative focal length covers nothing).  Pixels: columns floor(u - su) .. floor(u + su),
-// rows floor(v - sv) .. floor(v + sv), clamped to the image in float before the conversion to int.  Each pixel is tested with a
-// plain load of its current key and takes an atomicMin only when the new key is smaller: the atomic decides, the load only skips
-// the atomics that cannot win (points arrive in leaf-cell order, so a warp's squares overlap and the skipped atomics would
-// serialise on one address).
-__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_splat_kernel(
-        const float* __restrict__ xyz, int64_t P, const float* __restrict__ view, const float* __restrict__ intrinsics, int H, int W,
-        float h, float near, int max_radius, unsigned long long* __restrict__ zbuf) {
-    __shared__ float s_cam[16];          // rows 0..2 of the view matrix, then fx, fy, cx, cy
-    const int b = blockIdx.y;
+// camera b's rows 0..2 of the view matrix, then fx, fy, cx, cy, into s_cam[16]; the caller synchronises the block
+__device__ __forceinline__ void map_stage_camera(const float* __restrict__ view, const float* __restrict__ intrinsics, int b, float* s_cam) {
     if (threadIdx.x < 12) s_cam[threadIdx.x] = view[16 * (int64_t)b + threadIdx.x];
     else if (threadIdx.x < 16) s_cam[threadIdx.x] = intrinsics[4 * (int64_t)b + threadIdx.x - 12];
-    __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= P) return;
+}
+
+struct MapFootprint {
+    float z;
+    int c0, c1, r0, r1;      // covered columns / rows, clipped to the image
+};
+
+// The footprint of point i in the camera of s_cam, the one definition of coverage shared by the projection and the visibility
+// passes.  Every operation is separately rounded (the oracle's numpy order): p_q = ((V[q,0] x + V[q,1] y) + V[q,2] z) + V[q,3],
+// depth z = -p_2, u = fx (p_0 / z) + cx, v = fy (p_1 / z) + cy, su = min((fx h) / z, R), sv likewise.  A point is projected iff
+// z > near, u and v are finite and su, sv >= 0 (false for NaN, so a NaN half-size never becomes R, and a negative focal length
+// covers nothing).  Pixels: columns floor(u - su) .. floor(u + su), rows floor(v - sv) .. floor(v + sv), clamped to the image in
+// float before the conversion to int.  Returns false when the point is dropped or covers no pixel of the image.
+__device__ __forceinline__ bool map_footprint(const float* __restrict__ xyz, int64_t i, const float* s_cam, int H, int W, float h,
+                                              float near, int max_radius, MapFootprint& f) {
     const float x = xyz[3 * i], y = xyz[3 * i + 1], zw = xyz[3 * i + 2];
     float p[3];
 #pragma unroll
@@ -570,21 +571,40 @@ __global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_splat_kernel(
     }
     const float fx = s_cam[12], fy = s_cam[13], cx = s_cam[14], cy = s_cam[15];
     const float z = -p[2];
-    if (!(z > near)) return;
+    if (!(z > near)) return false;
     const float u = __fadd_rn(__fmul_rn(fx, __fdiv_rn(p[0], z)), cx), v = __fadd_rn(__fmul_rn(fy, __fdiv_rn(p[1], z)), cy);
     const float ru = __fdiv_rn(__fmul_rn(fx, h), z), rv = __fdiv_rn(__fmul_rn(fy, h), z);
-    if (!isfinite(u) || !isfinite(v) || !(ru >= 0.f) || !(rv >= 0.f)) return;
+    if (!isfinite(u) || !isfinite(v) || !(ru >= 0.f) || !(rv >= 0.f)) return false;
     const float R = (float)max_radius;
     const float su = fminf(ru, R), sv = fminf(rv, R);
     const float c0f = fmaxf(floorf(__fsub_rn(u, su)), 0.f), c1f = fminf(floorf(__fadd_rn(u, su)), (float)(W - 1));
     const float r0f = fmaxf(floorf(__fsub_rn(v, sv)), 0.f), r1f = fminf(floorf(__fadd_rn(v, sv)), (float)(H - 1));
-    if (c0f > c1f || r0f > r1f) return;
-    const int c0 = (int)c0f, c1 = (int)c1f, r0 = (int)r0f, r1 = (int)r1f;
-    const unsigned long long key = ((unsigned long long)__float_as_uint(z) << 32) | (unsigned long long)i;
+    if (c0f > c1f || r0f > r1f) return false;
+    f.z = z;
+    f.c0 = (int)c0f; f.c1 = (int)c1f; f.r0 = (int)r0f; f.r1 = (int)r1f;
+    return true;
+}
+
+// One thread per (point, camera): grid x over points, y over cameras.  Each pixel of the footprint is tested with a plain load of
+// its current key and takes an atomicMin only when the new key is smaller: the atomic decides, the load only skips the atomics
+// that cannot win (points arrive in leaf-cell order, so a warp's squares overlap and the skipped atomics would serialise on one
+// address).
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_splat_kernel(
+        const float* __restrict__ xyz, int64_t P, const float* __restrict__ view, const float* __restrict__ intrinsics, int H, int W,
+        float h, float near, int max_radius, unsigned long long* __restrict__ zbuf) {
+    __shared__ float s_cam[16];
+    const int b = blockIdx.y;
+    map_stage_camera(view, intrinsics, b, s_cam);
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    MapFootprint f;
+    if (!map_footprint(xyz, i, s_cam, H, W, h, near, max_radius, f)) return;
+    const unsigned long long key = ((unsigned long long)__float_as_uint(f.z) << 32) | (unsigned long long)i;
     unsigned long long* img = zbuf + (int64_t)b * H * W;
-    for (int r = r0; r <= r1; ++r) {
+    for (int r = f.r0; r <= f.r1; ++r) {
         unsigned long long* row = img + (int64_t)r * W;
-        for (int c = c0; c <= c1; ++c)
+        for (int c = f.c0; c <= f.c1; ++c)
             if (key < __ldcg(row + c)) atomicMin(row + c, key);
     }
 }
@@ -601,6 +621,148 @@ __global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_project_resolve_kernel(
     point[t] = p;
     depth[t] = hit ? __uint_as_float((uint32_t)(key >> 32)) : INFINITY;
     if (object) object[t] = hit ? component[p] : -1;
+}
+
+// ---- per-object visibility in camera views (pag_map_visibility, pag_map_visibility_silhouette) ----
+// Pair n = b K + o: object o in view b.  Boxes i32[N][4] = (col_min, row_min, col_max, row_max), empty as (BIG, BIG, -1, -1).  A
+// pair's silhouette bitmap covers its footprint-union box, one bit per pixel, each row padded to whole 32-bit words of the image
+// (word w holds columns 32 w .. 32 w + 31), so a pair takes rows * ((col_max >> 5) - (col_min >> 5) + 1) words.
+#define MAP_VIS_BIG 0x7fffffff
+
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_init_kernel(int64_t N, int* __restrict__ box, int* __restrict__ bbox,
+                                                                         long long* __restrict__ visible, long long* __restrict__ silhouette) {
+    const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    const int4 e = make_int4(MAP_VIS_BIG, MAP_VIS_BIG, -1, -1);
+    reinterpret_cast<int4*>(box)[n] = e;
+    reinterpret_cast<int4*>(bbox)[n] = e;
+    visible[n] = 0;
+    silhouette[n] = 0;
+}
+
+// Lanes with equal pair (all 32 lanes call; pair < 0: nothing to add) merge their rectangles with warp reductions, and the group's
+// first lane widens box[pair] with one atomic per side that the rectangle extends (a plain load skips the others: boxes stop
+// growing early, and the skipped atomics would serialise on one address) and adds the group's size to count[pair] (nullable).
+__device__ __forceinline__ void map_vis_widen(long long pair, int c0, int r0, int c1, int r1, int* __restrict__ box,
+                                              unsigned long long* __restrict__ count) {
+    const unsigned peers = __match_any_sync(0xffffffffu, pair);
+    c0 = __reduce_min_sync(peers, c0);
+    r0 = __reduce_min_sync(peers, r0);
+    c1 = __reduce_max_sync(peers, c1);
+    r1 = __reduce_max_sync(peers, r1);
+    if (pair < 0 || (int)(threadIdx.x & 31) != __ffs(peers) - 1) return;
+    if (count) atomicAdd(count + pair, (unsigned long long)__popc(peers));
+    int* bx = box + 4 * pair;
+    if (c0 < __ldcg(bx + 0)) atomicMin(bx + 0, c0);
+    if (r0 < __ldcg(bx + 1)) atomicMin(bx + 1, r0);
+    if (c1 > __ldcg(bx + 2)) atomicMax(bx + 2, c1);
+    if (r1 > __ldcg(bx + 3)) atomicMax(bx + 3, r1);
+}
+
+// one thread per pixel of the depth buffer: the front point's object o in [0, K) counts the pixel toward visible[b, o] and widens
+// bbox[b, o]; components outside [0, K) are skipped (out-of-range ones are counted by map_vis_box_kernel)
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_visible_kernel(
+        const unsigned long long* __restrict__ zbuf, int64_t N, int H, int W, const int64_t* __restrict__ component, int K,
+        long long* __restrict__ visible, int* __restrict__ bbox) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;      // every lane stays for the warp collectives
+    long long pair = -1;
+    int r = 0, c = 0;
+    if (t < N) {
+        const unsigned long long key = zbuf[t];
+        if (key != MAP_PROJECT_EMPTY) {
+            const int64_t o = component[key & 0xffffffffull];
+            if (o >= 0 && o < K) {
+                const int64_t hw = (int64_t)H * W, b = t / hw, pix = t - b * hw;
+                r = (int)(pix / W);
+                c = (int)(pix - (int64_t)r * W);
+                pair = b * K + o;
+            }
+        }
+    }
+    map_vis_widen(pair, c, r, c, r, bbox, reinterpret_cast<unsigned long long*>(visible));
+}
+
+// one thread per (point, camera), grid y = max(B, 1): the footprint of a point of object o in [0, K) widens box[b, o].  The cameras'
+// first row counts the points whose component lies outside [-1, K) into errors[0], once per point, also when B = 0.
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_box_kernel(
+        const float* __restrict__ xyz, int64_t P, const float* __restrict__ view, const float* __restrict__ intrinsics, int B, int H,
+        int W, float h, float near, int max_radius, const int64_t* __restrict__ component, int K, int* __restrict__ box,
+        long long* __restrict__ errors) {
+    __shared__ float s_cam[16];
+    const int b = blockIdx.y;
+    if (b < B) map_stage_camera(view, intrinsics, b, s_cam);
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t o = i < P ? component[i] : -1;
+    if (b == 0) {
+        const unsigned n_bad = __popc(__ballot_sync(0xffffffffu, o < -1 || o >= K));
+        if ((threadIdx.x & 31) == 0 && n_bad) atomicAdd(reinterpret_cast<unsigned long long*>(errors), (unsigned long long)n_bad);
+    }
+    MapFootprint f = {0.f, 0, 0, 0, 0};
+    const bool on = b < B && o >= 0 && o < K && map_footprint(xyz, i, s_cam, H, W, h, near, max_radius, f);
+    map_vis_widen(on ? (long long)b * K + o : -1, f.c0, f.r0, f.c1, f.r1, box, nullptr);
+}
+
+// one thread per pair: bbox = -1 where nothing is visible, words[n] = the size of the pair's bitmap (0 for an empty box)
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_pairs_kernel(int64_t N, const long long* __restrict__ visible,
+                                                                          const int* __restrict__ box, int* __restrict__ bbox,
+                                                                          int* __restrict__ words) {
+    const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    if (visible[n] == 0) reinterpret_cast<int4*>(bbox)[n] = make_int4(-1, -1, -1, -1);
+    const int4 e = reinterpret_cast<const int4*>(box)[n];
+    words[n] = e.z >= e.x ? (e.w - e.y + 1) * ((e.z >> 5) - (e.x >> 5) + 1) : 0;
+}
+
+// One round of silhouettes: thread per (point, camera); a point of object o whose pair's bitmap starts at offset[pair] in
+// [lo, hi) (in words) ORs its footprint into that bitmap at bits + offset - lo.  A footprint row spans at most 66 columns, so at
+// most 4 words; a plain load skips the atomicOr when the word already holds the bits.
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_or_kernel(
+        const float* __restrict__ xyz, int64_t P, const float* __restrict__ view, const float* __restrict__ intrinsics, int H, int W,
+        float h, float near, int max_radius, const int64_t* __restrict__ component, int K, const int* __restrict__ box,
+        const int64_t* __restrict__ offset, int64_t lo, int64_t hi, unsigned* __restrict__ bits) {
+    __shared__ float s_cam[16];
+    const int b = blockIdx.y;
+    map_stage_camera(view, intrinsics, b, s_cam);
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    const int64_t o = component[i];
+    if (o < 0 || o >= K) return;
+    const int64_t pair = (int64_t)b * K + o;
+    const int64_t off = offset[pair];
+    if (off < lo || off >= hi) return;
+    MapFootprint f;
+    if (!map_footprint(xyz, i, s_cam, H, W, h, near, max_radius, f)) return;
+    const int4 e = reinterpret_cast<const int4*>(box)[pair];
+    const int w0 = e.x >> 5, wpr = (e.z >> 5) - w0 + 1;
+    unsigned* img = bits + (off - lo) - w0;          // + row * wpr + word: word (c >> 5) of the pair's row
+    for (int r = f.r0; r <= f.r1; ++r) {
+        unsigned* row = img + (int64_t)(r - e.y) * wpr;
+        for (int w = f.c0 >> 5; w <= (f.c1 >> 5); ++w) {
+            const int a = max(f.c0 - 32 * w, 0), z = min(f.c1 - 32 * w, 31);
+            const unsigned m = (0xffffffffu >> (31 - z)) & (0xffffffffu << a);
+            if ((__ldcg(row + w) & m) != m) atomicOr(row + w, m);
+        }
+    }
+}
+
+// one warp per pair of the round: silhouette[n] = the popcount of its bitmap
+__global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_popc_kernel(int64_t N, const int* __restrict__ words,
+                                                                         const int64_t* __restrict__ offset, int64_t lo, int64_t hi,
+                                                                         const unsigned* __restrict__ bits,
+                                                                         long long* __restrict__ silhouette) {
+    const int64_t n = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (n >= N) return;                                                      // warp-uniform
+    const int64_t off = offset[n];
+    const int nw = words[n];
+    if (nw == 0 || off < lo || off >= hi) return;
+    const unsigned* w = bits + (off - lo);
+    long long s = 0;
+    for (int j = lane; j < nw; j += 32) s += __popc(__ldcg(w + j));
+    for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
+    if (lane == 0) silhouette[n] = s;
 }
 
 static int map_stats_launch(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* lab, int64_t P, int Cs, int Ci,
@@ -768,6 +930,85 @@ int pag_map_project(const float* xyz, int64_t P, const float* view, const float*
     map_project_resolve_kernel<<<(unsigned)pag_grid(N, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(zb, N, component, point, depth,
                                                                                                       object);
     PAG_LAUNCH_CHECK();
+    return PAG_OK;
+}
+
+static bool map_vis_args_ok(int64_t P, int B, int H, int W, float h, float near, int max_radius, int K) {
+    return P >= 0 && P <= MAP_CC_MAX_POINTS && B >= 0 && B <= MAP_PROJECT_MAX_CAMERAS && H >= 1 && H <= MAP_PROJECT_MAX_SIDE && W >= 1 &&
+           W <= MAP_PROJECT_MAX_SIDE && max_radius >= 0 && max_radius <= MAP_PROJECT_MAX_RADIUS && near > 0.f && isfinite(near) &&
+           h > 0.f && isfinite(h) && K >= 0 && K <= MAP_CC_MAX_POINTS;
+}
+
+int pag_map_visibility(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h, float near,
+                       int max_radius, const int64_t* component, int K, int64_t* zbuf, int32_t* box, int32_t* words, int64_t* offset,
+                       int64_t* visible, int64_t* silhouette, int32_t* bbox, void* stream) {
+    if (!map_vis_args_ok(P, B, H, W, h, near, max_radius, K) || !offset) return PAG_ERR_ARG;
+    const int64_t N = (int64_t)B * K, NP = (int64_t)B * H * W;
+    if ((NP + MAP_PROJECT_BLOCK - 1) / MAP_PROJECT_BLOCK > 0x7fffffff || (32 * N + MAP_PROJECT_BLOCK - 1) / MAP_PROJECT_BLOCK > 0x7fffffff)
+        return PAG_ERR_ARG;      // a thread per pixel, a warp per pair
+    if ((P > 0 && (!xyz || !component)) || (B > 0 && (!view || !intrinsics)) ||
+        (N > 0 && (!box || !words || !visible || !silhouette || !bbox)) || (N > 0 && P > 0 && !zbuf))
+        return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(offset + N + 1, 0, sizeof(int64_t), s);      // the error count
+    if (e != cudaSuccess) return (int)e;
+    long long* errors = reinterpret_cast<long long*>(offset + N + 1);
+    if (N > 0) {
+        map_vis_init_kernel<<<pag_grid(N, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(N, box, bbox, reinterpret_cast<long long*>(visible),
+                                                                                          reinterpret_cast<long long*>(silhouette));
+        PAG_LAUNCH_CHECK();
+    }
+    unsigned long long* zb = reinterpret_cast<unsigned long long*>(zbuf);
+    if (N > 0 && P > 0) {      // the front points (pag_map_project's fill and splat) and the visible counts; none in an empty map
+        if ((e = cudaMemsetAsync(zbuf, 0xff, NP * sizeof(int64_t), s)) != cudaSuccess) return (int)e;
+        map_project_splat_kernel<<<dim3((unsigned)pag_grid(P, MAP_PROJECT_BLOCK), (unsigned)B), MAP_PROJECT_BLOCK, 0, s>>>(
+            xyz, P, view, intrinsics, H, W, h, near, max_radius, zb);
+        PAG_LAUNCH_CHECK();
+        map_vis_visible_kernel<<<(unsigned)pag_grid(NP, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(
+            zb, NP, H, W, component, K, reinterpret_cast<long long*>(visible), bbox);
+        PAG_LAUNCH_CHECK();
+    }
+    if (P > 0) {      // footprint boxes; the out-of-range count also when there is no pair
+        map_vis_box_kernel<<<dim3((unsigned)pag_grid(P, MAP_PROJECT_BLOCK), (unsigned)(B > 0 ? B : 1)), MAP_PROJECT_BLOCK, 0, s>>>(
+            xyz, P, view, intrinsics, B, H, W, h, near, max_radius, component, K, box, errors);
+        PAG_LAUNCH_CHECK();
+    }
+    if (N > 0) {
+        map_vis_pairs_kernel<<<pag_grid(N, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(N, reinterpret_cast<const long long*>(visible),
+                                                                                           box, bbox, words);
+        PAG_LAUNCH_CHECK();
+        return pag_exclusive_scan_i32(words, N, offset, stream);
+    }
+    e = cudaMemsetAsync(offset, 0, sizeof(int64_t), s);      // no pair: total 0
+    return e == cudaSuccess ? PAG_OK : (int)e;
+}
+
+int pag_map_visibility_silhouette(const float* xyz, int64_t P, const float* view, const float* intrinsics, int B, int H, int W, float h,
+                                  float near, int max_radius, const int64_t* component, int K, const int32_t* box, const int32_t* words,
+                                  const int64_t* offset, int64_t total_words, int32_t* bits, int64_t bits_words, int64_t* silhouette,
+                                  void* stream) {
+    if (!map_vis_args_ok(P, B, H, W, h, near, max_radius, K) || total_words < 0 || bits_words < 0) return PAG_ERR_ARG;
+    const int64_t N = (int64_t)B * K;
+    if (N == 0 || P == 0 || total_words == 0) return PAG_OK;
+    if (!xyz || !view || !intrinsics || !component || !box || !words || !offset || !bits || !silhouette) return PAG_ERR_ARG;
+    // rounds are windows [lo, lo + step) of the bitmaps' offsets: a pair starting in the window ends before lo + step + (its size
+    // <= max_pair), so every round fits in bits_words = step + max_pair words
+    const int64_t max_pair = (int64_t)H * (((W - 1) >> 5) + 1);
+    const int64_t step = total_words <= bits_words ? total_words : bits_words - max_pair;
+    if (step <= 0) return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned* bw = reinterpret_cast<unsigned*>(bits);
+    for (int64_t lo = 0; lo < total_words; lo += step) {
+        const int64_t hi = lo + step, used = (total_words < hi + max_pair ? total_words : hi + max_pair) - lo;
+        cudaError_t e = cudaMemsetAsync(bits, 0, (used < bits_words ? used : bits_words) * sizeof(int32_t), s);
+        if (e != cudaSuccess) return (int)e;
+        map_vis_or_kernel<<<dim3((unsigned)pag_grid(P, MAP_PROJECT_BLOCK), (unsigned)B), MAP_PROJECT_BLOCK, 0, s>>>(
+            xyz, P, view, intrinsics, H, W, h, near, max_radius, component, K, box, offset, lo, hi, bw);
+        PAG_LAUNCH_CHECK();
+        map_vis_popc_kernel<<<pag_grid(32 * N, MAP_PROJECT_BLOCK), MAP_PROJECT_BLOCK, 0, s>>>(N, words, offset, lo, hi, bw,
+                                                                                            reinterpret_cast<long long*>(silhouette));
+        PAG_LAUNCH_CHECK();
+    }
     return PAG_OK;
 }
 

@@ -111,6 +111,31 @@ project_map answers, from the map alone, which map point, at what depth and whic
   * Limits.  P <= 2^30, B <= 65535, height and width integers in [1, 16384], near a finite number > 0 (also in fp32).
   * Host traffic.  None: the launch geometry depends on P, B, H, W and max_radius only, so the call can be captured in a CUDA graph.
   * Memory.  The outputs and a u64 depth buffer of B H W entries: 28 bytes per pixel with component, 20 without.
+
+object_visibility answers, per map object and camera view, how much of the object the view sees, how much of it is hidden and where:
+
+    vis = object_visibility(pts, samples_per_axis=2, level=nef.grid.blas_level, view=V, intrinsics=K, height=H, width=W,
+                            component=comps.component, num_objects=comps.count.numel())   # ObjectVisibility, [B, K] tensors
+    best = vis.visible.argmax(0)                          # the view that shows each object best; vis.bbox[best[o], o] crops it
+    occluded = 1 - vis.visible / vis.silhouette           # NaN where the view covers none of the object
+
+  * Arguments.  pts, samples_per_axis, level, view, intrinsics, height, width, max_radius and near mean exactly what they mean
+    for project_map, with its checks and limits.  component i64 [P]: each point's object in [0, num_objects) or -1; components
+    outside [-1, num_objects) raise ValueError with their number.  num_objects = K, an integer >= 0.
+  * Coverage.  Pixel (b, r, c) is covered by point i iff project_map's footprint rule covers it: the same fp32 arithmetic, the same
+    dropped points (near plane, non-finite, negative half-size, off-screen) and clamping before the integer conversion.
+  * visible[b, o]: the pixels of view b whose project_map point (smallest depth, then smallest index) has component o.
+  * silhouette[b, o]: the pixels of view b covered by at least one point with component o, at any depth; visible[b, o] of a
+    projection of object o's points alone.
+  * bbox[b, o] = (col_min, row_min, col_max, row_max) of the visible pixels, (-1, -1, -1, -1) where visible[b, o] == 0.
+  * Points with component -1 (stuff, floaters, inactive points) occlude but own no row.  So visible <= silhouette, and visible[b]
+    sums to the pixels of view b with MapView.object >= 0.  The occluded fraction and the best view are left to the caller.
+  * Host traffic.  One host read per call (the silhouette bitmaps' size and the error count); the call cannot be captured in a
+    CUDA graph.  The result depends only on the inputs: the same for any split of the cameras into calls and on every run.
+  * Memory.  The u64 depth buffer (8 B H W bytes, freed before the silhouettes), 32 bytes of outputs and 28 of workspace per
+    (view, object) pair plus 16 bytes, and the silhouette bitmaps: one bit per pixel of each pair's footprint box, rows padded to
+    32-bit words, at most VISIBILITY_BITMAP_BYTES (256 MiB).  When the bitmaps exceed it the silhouettes are built in rounds,
+    each a pass over the points and cameras.
 """
 import math
 from typing import NamedTuple, Optional
@@ -131,6 +156,7 @@ MAX_LOOKUP_RADIUS = 4                                # a (2r+1)^3 window: 729 pr
 MAX_PROJECT_RADIUS = 32                              # a footprint of at most 66 x 66 pixels
 MAX_PROJECT_SIDE = 16384
 MAX_PROJECT_CAMERAS = 65535                          # one grid row per camera
+VISIBILITY_BITMAP_BYTES = 256 << 20                  # silhouette bitmaps of one round; >= 32 MiB, one 16384 x 16384 view's
 
 
 class PanopticPoints(NamedTuple):
@@ -172,6 +198,12 @@ class MapView(NamedTuple):
     point: torch.Tensor                    # i64 [B, H, W]: the visible map point of each pixel, -1 if none
     depth: torch.Tensor                    # f32 [B, H, W]: its camera-space depth z (> near), +inf where point == -1
     object: Optional[torch.Tensor]         # i64 [B, H, W]: component[point], -1 where point == -1 or the point is in no object
+
+
+class ObjectVisibility(NamedTuple):
+    visible: torch.Tensor                  # i64 [B, K]: pixels of view b whose front map point belongs to object o
+    silhouette: torch.Tensor               # i64 [B, K]: pixels of view b covered by object o's points at any depth
+    bbox: torch.Tensor                     # i32 [B, K, 4]: (col_min, row_min, col_max, row_max) of the visible pixels, -1s if none
 
 
 class InstanceSummary(NamedTuple):
@@ -428,22 +460,18 @@ def lookup_rays(index, origins, dirs, depth, alpha, radius=1, min_alpha=0.5, com
     return MapLookup(point, obj)
 
 
-def project_map(pts, samples_per_axis, level, view, intrinsics, height, width, max_radius=8, near=0.01, component=None):
-    """Z-buffered splatting of a map's points into B camera views (view f32 [B, 4, 4] world-to-camera, intrinsics f32 [B, 4] =
-    (fx, fy, cx, cy)): per pixel the nearest covering map point, its depth and, with component (i64 [P]), its object -> MapView of
-    [B, height, width] tensors (csrc/mapping.cu, a fill and two launches, no host read).  pts: PanopticPoints or its xyz f32 [P, 3].
-    See the module docstring for the exact definitions."""
-    k = samples_per_axis
+def _check_projection(fn, pts, k, level, view, intrinsics, height, width, max_radius, near, component):
+    """The arguments project_map and object_visibility share -> (xyz, h, near) as the kernels take them"""
     _check_lattice(k, level)
     xyz = pts.xyz if isinstance(pts, PanopticPoints) else pts
     _check_tensor("xyz", xyz, [(None, 3)], torch.float32)
     P = int(xyz.shape[0])
     if P > MAX_COMPONENT_POINTS:
-        raise ValueError(f"project_map serves up to {MAX_COMPONENT_POINTS} points, got {P}")
+        raise ValueError(f"{fn} serves up to {MAX_COMPONENT_POINTS} points, got {P}")
     _check_tensor("view", view, [(None, 4, 4)], torch.float32)
     B = int(view.shape[0])
     if B > MAX_PROJECT_CAMERAS:
-        raise ValueError(f"project_map serves up to {MAX_PROJECT_CAMERAS} cameras per call, got {B}")
+        raise ValueError(f"{fn} serves up to {MAX_PROJECT_CAMERAS} cameras per call, got {B}")
     _check_tensor("intrinsics", intrinsics, [(B, 4)], torch.float32)
     for name, n in (("height", height), ("width", width)):
         if not _is_int(n) or not 1 <= n <= MAX_PROJECT_SIDE:
@@ -461,10 +489,38 @@ def project_map(pts, samples_per_axis, level, view, intrinsics, height, width, m
             raise TypeError(f"component must be torch.int64, got {component.dtype}")
     if not all(t.is_cuda for t in (xyz, view, intrinsics, component) if t is not None):
         raise RuntimeError("pagnerf_b200 map projection runs on CUDA tensors only (no CPU fallback)")
-    h = float(np.float32(1.0) / np.float32(int(k) << int(level)))
-    point, depth, obj = ops.map_project(xyz, view, intrinsics, int(height), int(width), h, float(np.float32(near)), int(max_radius),
-                                        component)
+    return xyz, float(np.float32(1.0) / np.float32(int(k) << int(level))), float(np.float32(near))
+
+
+def project_map(pts, samples_per_axis, level, view, intrinsics, height, width, max_radius=8, near=0.01, component=None):
+    """Z-buffered splatting of a map's points into B camera views (view f32 [B, 4, 4] world-to-camera, intrinsics f32 [B, 4] =
+    (fx, fy, cx, cy)): per pixel the nearest covering map point, its depth and, with component (i64 [P]), its object -> MapView of
+    [B, height, width] tensors (csrc/mapping.cu, a fill and two launches, no host read).  pts: PanopticPoints or its xyz f32 [P, 3].
+    See the module docstring for the exact definitions."""
+    xyz, h, near = _check_projection("project_map", pts, samples_per_axis, level, view, intrinsics, height, width, max_radius, near,
+                                     component)
+    point, depth, obj = ops.map_project(xyz, view, intrinsics, int(height), int(width), h, near, int(max_radius), component)
     return MapView(point, depth, obj)
+
+
+def object_visibility(pts, samples_per_axis, level, view, intrinsics, height, width, component, num_objects, max_radius=8, near=0.01):
+    """How much of each map object each of B camera views sees: per (view, object) the visible area, the unoccluded silhouette and
+    the visible pixels' box -> ObjectVisibility (csrc/mapping.cu, one host read).  The arguments shared with project_map mean and
+    are checked as there; component i64 [P] (e.g. InstanceComponents.component) gives each point's object in [0, num_objects) or
+    -1.  Raises ValueError with their number for components outside [-1, num_objects).  See the module docstring for the exact
+    definitions and the memory bound."""
+    if component is None:
+        raise TypeError("object_visibility needs component (i64 [P], each point's object or -1)")
+    if not _is_int(num_objects) or not 0 <= num_objects <= MAX_COMPONENT_POINTS:
+        raise ValueError(f"num_objects must be an integer in [0, {MAX_COMPONENT_POINTS}], got {num_objects!r}")
+    xyz, h, near = _check_projection("object_visibility", pts, samples_per_axis, level, view, intrinsics, height, width, max_radius,
+                                     near, component)
+    K = int(num_objects)
+    visible, silhouette, bbox, bad, _ = ops.map_visibility(xyz, view, intrinsics, int(height), int(width), h, near, int(max_radius),
+                                                           component, K, VISIBILITY_BITMAP_BYTES)
+    if bad:
+        raise ValueError(f"{bad} points carry a component outside [-1, {K})")
+    return ObjectVisibility(visible, silhouette, bbox)
 
 
 PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),

@@ -735,6 +735,48 @@ def map_project(xyz, view, intrinsics, H, W, h, near, max_radius, component=None
     return point, depth, obj
 
 
+def silhouette_bitmap_words(total_words, H, W, cap_bytes):
+    """-> (words of the bitmap buffer, rounds) pag_map_visibility_silhouette takes for `total_words` words of pair bitmaps under a
+    cap of cap_bytes (include/pagnerf_b200.h)"""
+    cap = int(cap_bytes) // 4
+    if total_words <= cap:
+        return total_words, int(total_words > 0)
+    step = cap - H * ((W + 31) // 32)
+    if step <= 0:
+        raise ValueError(f"a silhouette bitmap cap of {cap_bytes} bytes does not exceed the largest bitmap of a {H} x {W} view")
+    return cap, -(-total_words // step)
+
+
+def map_visibility(xyz, view, intrinsics, H, W, h, near, max_radius, component, K, cap_bytes):
+    """Per-(view, object) visibility of the map points xyz f32[P,3] in B views (csrc/mapping.cu pag_map_visibility and
+    pag_map_visibility_silhouette) -> visible i64[B,K], silhouette i64[B,K], bbox i32[B,K,4] on the device, and on the host the
+    number of points whose component lies outside [-1, K) and the total words of the silhouette bitmaps.  One host read between the
+    two entries (those two numbers); the silhouettes are skipped when the first is not 0.  Allocates the outputs, the u64 depth
+    buffer (freed before the bitmaps), 28 bytes of workspace per pair and at most cap_bytes of bitmaps."""
+    _chk(xyz, view, intrinsics, component)
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    V, Kc = view.detach().contiguous(), intrinsics.detach().contiguous()
+    comp = component.contiguous()
+    B, P, dev = V.shape[0], x.shape[0], x.device
+    N = B * K
+    visible = torch.empty(B, K, dtype=torch.int64, device=dev)
+    silhouette = torch.empty(B, K, dtype=torch.int64, device=dev)
+    bbox = torch.empty(B, K, 4, dtype=torch.int32, device=dev)
+    box = torch.empty(N, 4, dtype=torch.int32, device=dev)
+    words = torch.empty(N, dtype=torch.int32, device=dev)
+    offset = torch.empty(N + 2, dtype=torch.int64, device=dev)
+    args = (ptr(x), P, ptr(V), ptr(Kc), B, int(H), int(W), float(h), float(near), int(max_radius), ptr(comp), int(K))
+    zbuf = torch.empty(B * H * W if N > 0 and P > 0 else 0, dtype=torch.int64, device=dev)      # nothing to splat otherwise
+    call("pag_map_visibility", *args, ptr(zbuf), ptr(box), ptr(words), ptr(offset), ptr(visible), ptr(silhouette), ptr(bbox))
+    del zbuf
+    total, bad = offset[N:].tolist()                # the one host read
+    if bad == 0 and total > 0:
+        n_words, _ = silhouette_bitmap_words(total, H, W, cap_bytes)
+        bits = torch.empty(n_words, dtype=torch.int32, device=dev)
+        call("pag_map_visibility_silhouette", *args, ptr(box), ptr(words), ptr(offset), total, ptr(bits), n_words, ptr(silhouette))
+    return visible, silhouette, bbox, bad, total
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""
