@@ -1054,7 +1054,7 @@ int pag_decode_pan_bwd_tc(const float* feats, const float* dfeats, const float* 
                           const float* const* weights, float* const* grads, int hidden, int Cs, int Ci, int sem_softmax,
                           int inst_softmax, float inst_temperature, const float* sem, const float* inst,
                           const float* g_sem, const float* g_inst, const float* grad_scale, float* g_panop, void* stream) {
-    if (hidden != H || Cs < 0 || Ci < 0 || Cs > 32 || Ci > 256 || IN < 1 || IN > 64) return PAG_ERR_UNSUPPORTED;
+    if (hidden != H || Cs < 0 || Ci < 0 || Cs > 32 || Ci > 256 || IN < 1 || IN > 64 || (IN & 3)) return PAG_ERR_UNSUPPORTED;
     if (M == 0 || (Cs == 0 && Ci == 0)) return PAG_OK;
     PanParams p{};
     fill_pan(p, weights, grads);

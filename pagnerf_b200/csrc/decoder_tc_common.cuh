@@ -449,7 +449,7 @@ __host__ __device__ inline PanTcLayout pan_tc_layout(int IN, int Cs, int Ci, boo
     l.CiP = Ci > 0 ? ((Ci + 15) & ~15) : 16;
     l.nGi = l.CiP / 8;
     int o = 0;
-    l.oGs = o; o += bwd ? 2 * TCH : 0;
+    l.oGs = o; o += bwd ? (l.CsP / 8) * TCH : 0;   // semantic logit gradients: CsP <= 32 features
     l.oX = o; o += 8 * TCH;
     l.oHs = o; o += 8 * TCH;
     l.oH1 = o; o += 8 * TCH;

@@ -618,15 +618,17 @@ __global__ void __launch_bounds__(PCB_THREADS) pan_comp_bwd_kernel(
 #pragma unroll
                 for (int j = 0; j < 16; ++j) g[j] = (j < Cs) ? __ldg(g_sem + ray * Cs + j) : 0.f;
             }
-            float Z = 0.f, E = 0.f;
+            float Z = 0.f, E = 0.f, ZG = 0.f;
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 const float e = (j < Cs) ? (sem_softmax ? fast_exp2((zs[j] - mx) * LOG2E_F) : 1.f) : 0.f;
+                if (j < Cs) ZG = fmaf(zs[j], g[j], ZG);
                 zs[j] = e;
                 Z += e; E = fmaf(e, (j < Cs) ? g[j] : 0.f, E);
             }
             const float iz = 1.f / Z, dot = E * iz, css = cs * scale;
-            if (gw_sem && valid) gw_sem[m] = dot;      // <p_s, g_ray>: d out / d weight of this sample (DD tracer: weights carry gradient)
+            // <p_s, g_ray>: d out / d weight of this sample (DD tracer: weights carry gradient); p_s = the logits without softmax
+            if (gw_sem && valid) gw_sem[m] = sem_softmax ? dot : ZG;
 #pragma unroll
             for (int j = 0; j < 16; ++j) g[j] = (j < Cs) ? (sem_softmax ? css * zs[j] * iz * (g[j] - dot) : css * g[j]) : 0.f;
             grad16_store(g, Gs, row, lane, db_s2);
@@ -665,6 +667,22 @@ __global__ void __launch_bounds__(PCB_THREADS) pan_comp_bwd_kernel(
                 __syncthreads(); PAG_PHASE(8);
                 dot = (part_s[0][row] + part_s[1][row]) + (part_s[2][row] + part_s[3][row]);
                 if (gw_inst && cg == 0 && valid) gw_inst[m] = dot * inv_scale;      // the cached gradients carry the loss scale
+            } else if (gw_inst) {      // without softmax the sample's outputs are the scaled logits z / T: <z / T, g_ray>
+                float zg = 0.f;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const int c0 = 16 * (cg + PCB_NCG * k);
+                    if (c0 < l.CiP) {
+                        float v[16], g[16];
+                        load_g16(gc_row, grow, c0, Ci, vec4, scale, g);
+                        tmem_ld16(tl + c0, v);
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) zg = fmaf(fmaf(v[i], s2, bi3[c0 + i]), g[i], zg);   // padded columns: g = 0
+                    }
+                }
+                part_s[cg][row] = zg;
+                __syncthreads();
+                if (cg == 0 && valid) gw_inst[m] = ((part_s[0][row] + part_s[1][row]) + (part_s[2][row] + part_s[3][row])) * inv_scale;
             }
             const float c2 = cs * inst_inv_temp;
 #pragma unroll
