@@ -496,6 +496,20 @@ int pag_map_visibility_silhouette(const float* xyz, int64_t P, const float* view
                                   float near, int max_radius, const int64_t* component, int K, const int32_t* box, const int32_t* words,
                                   const int64_t* offset, int64_t total_words, int32_t* bits, int64_t bits_words, int64_t* silhouette,
                                   void* stream);
+/* ---- size and orientation of each map object: exact covariance, principal axes and oriented box ----
+ * pag_map_shape: xyz f32[P,3] on the lattice of (k, level), D = k << level, as for pag_map_components (P <= 2^30); component i64[P]
+ * (required when P > 0): each point's object in [0, K) or -1 (skipped), K <= 2^30.  Per object o, from the lattice indices j of its
+ * points: the moments n, S_a = sum j_a, S_ab = sum j_a j_b in exact integers (S_ab in 128 bits), covariance f64[K,3,3] =
+ * (((num / n) / n) 4 / D) / D with num = n S_ab - S_a S_b converted to f64 rounded to nearest even; its eigenvalues variance f64[K,3]
+ * (descending, ties in x, y, z order) and unit eigenvectors axes f64[K,3,3] (row a for variance[a]; cyclic Jacobi, the component of
+ * largest magnitude of rows 0 and 1 positive, row 2 = row 0 x row 1); the box of the projections p_a = ((jx e_ax + jy e_ay) +
+ * jz e_az) (f64, each operation rounded): extent f64[K,3] = ((hi_a - lo_a) + 1) 2 / D, center f64[K,3] = (2 c + 1) / D - 1 per axis with
+ * c = sum_a ((lo_a + hi_a) / 2) e_a.  Objects without points get NaN.  acc i64[K*22]: workspace, zeroed by the call (per object n,
+ * S_a, S_ab low and carry words, then the order-preserving images of lo and hi).  errors i64[2] (set by the call) = points off the
+ * lattice | points with a component outside [-1, K); the outputs are meaningful only when both are 0.  Two fills and four launches,
+ * no host synchronisation; the result does not depend on point order or thread schedule. */
+int pag_map_shape(const float* xyz, int64_t P, int level, int k, const int64_t* component, int K, int64_t* acc, double* covariance,
+                  double* variance, double* axes, double* center, double* extent, int64_t* errors, void* stream);
 
 /* ---- fused multi-tensor Adam (BASELINE config 4: "+ Adam"; SURVEY 8e "a single fused unscale + Adam kernel") ----
  * Replaces torch.optim.Adam.step() as the reference's trainer runs it (pc_nerf/trainer.py:229-300 parameter groups, :590 step;

@@ -26,6 +26,7 @@ KERNELS_PER_CALL = {
     # at most: pag_map_visibility skips the splat and the per-pixel kernel for an empty map and the pair kernels without pairs;
     # pag_map_visibility_silhouette launches 2 kernels (and a fill) per round, the figure is for one round
     "pag_map_visibility": 6, "pag_map_visibility_silhouette": 2,
+    "pag_map_shape": 4,      # at most: the per-point passes are skipped for an empty map, all but the moments without objects
 }
 launch_count = 0
 

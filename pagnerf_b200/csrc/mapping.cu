@@ -765,6 +765,381 @@ __global__ void __launch_bounds__(MAP_PROJECT_BLOCK) map_vis_popc_kernel(int64_t
     if (lane == 0) silhouette[n] = s;
 }
 
+// ---- size and orientation of each map object (pag_map_shape) ----
+// Per object, u64 accumulators acc[MAP_SHAPE_ACC * o + ...]: n | S_a (3) | S_ab low words (6) | S_ab high words (6) | lo (3) | hi (3).
+// S_ab = sum of j_a j_b over the object's points (a <= b in the order xx, xy, xz, yy, yz, zz), a 128-bit value held as a low word and
+// a carry word; lo / hi are the order-preserving integer images (shape_key) of the projections' minimum and maximum.
+#define MAP_SHAPE_BLOCK 256
+#define MAP_SHAPE_ACC 22
+#define MAP_SHAPE_SWEEPS 50
+#define MAP_SHAPE_WARPS_PER_SM 64
+
+__constant__ signed char c_shape_pair[6][2] = {{0, 0}, {0, 1}, {0, 2}, {1, 1}, {1, 2}, {2, 2}};
+
+// the IEEE total order of f64 (-0 < +0) as the unsigned order of a u64
+__device__ __forceinline__ unsigned long long shape_key(double v) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+    return (b >> 63) ? ~b : b | 0x8000000000000000ull;
+}
+__device__ __forceinline__ double shape_unkey(unsigned long long k) {
+    return __longlong_as_double((long long)((k >> 63) ? k & 0x7fffffffffffffffull : ~k));
+}
+
+// Sum of v over the lanes of `peers` (every lane of peers calls with the same mask), exact for any u64 v: three limbs of 27, 27 and
+// 10 bits, each limb's sum over at most 32 lanes fits 32 bits.
+__device__ __forceinline__ unsigned __int128 shape_warp_sum(unsigned peers, unsigned long long v) {
+    const unsigned m = (1u << 27) - 1u;
+    const unsigned a = __reduce_add_sync(peers, (unsigned)v & m), b = __reduce_add_sync(peers, (unsigned)(v >> 27) & m),
+                   c = __reduce_add_sync(peers, (unsigned)(v >> 54));
+    return (unsigned __int128)a + ((unsigned __int128)b << 27) + ((unsigned __int128)c << 54);
+}
+
+// minimum (MAX = false) or maximum of a u64 over the lanes of `peers`: the high words first, then the low words of the lanes that hold it
+template <bool MAX>
+__device__ __forceinline__ unsigned long long shape_warp_extreme(unsigned peers, unsigned long long v) {
+    const unsigned hi = (unsigned)(v >> 32), lo = (unsigned)v;
+    const unsigned h = MAX ? __reduce_max_sync(peers, hi) : __reduce_min_sync(peers, hi);
+    const unsigned l = MAX ? __reduce_max_sync(peers, hi == h ? lo : 0u) : __reduce_min_sync(peers, hi == h ? lo : 0xffffffffu);
+    return ((unsigned long long)h << 32) | l;
+}
+
+// 128-bit add into (low word, carry word): the value atomicAdd returns tells whether the low word wrapped
+__device__ __forceinline__ void shape_add_u128(unsigned long long* lo, unsigned long long* hi, unsigned __int128 v) {
+    const unsigned long long vl = (unsigned long long)v, vh = (unsigned long long)(v >> 64);
+    const unsigned long long old = vl ? atomicAdd(lo, vl) : 0ull;
+    const unsigned long long carry = vh + (old + vl < old ? 1ull : 0ull);
+    if (carry) atomicAdd(hi, carry);
+}
+
+// The points of warp w: the contiguous range [w * per, (w + 1) * per) of a grid of whole CTAs, per a multiple of 32, so a warp walks
+// through an object's run of Morton-ordered points and carries its sums from one 32-point step to the next.
+static void shape_grid(int64_t P, int* blocks, int64_t* per) {      // P >= 1
+    const int64_t warps_max = (int64_t)MAP_SHAPE_WARPS_PER_SM * map_num_sms();
+    int64_t warps = (P + 31) / 32;
+    if (warps > warps_max) warps = warps_max;
+    const int64_t wpb = MAP_SHAPE_BLOCK / 32;
+    *blocks = (int)((warps + wpb - 1) / wpb);
+    const int64_t all = (int64_t)*blocks * wpb;
+    *per = ((P + all - 1) / all + 31) / 32 * 32;
+}
+
+// lattice index j of point m and its object q in [0, K); q = -1 for points to skip.  off / bad: the point is off the lattice / its
+// component lies outside [-1, K).
+__device__ __forceinline__ int shape_point(const float* __restrict__ xyz, const int64_t* __restrict__ component, int64_t m, int64_t P,
+                                           int D, int K, int j[3], bool& off, bool& bad) {
+    off = bad = false;
+    j[0] = j[1] = j[2] = 0;
+    if (m >= P) return -1;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) j[a] = cc_lattice_index(xyz[3 * m + a], D);
+    const int64_t q = component[m];
+    off = j[0] < 0 || j[1] < 0 || j[2] < 0;
+    bad = q < -1 || q >= K;
+    return off || bad ? -1 : (int)q;
+}
+
+// Moments: every lane carries n, S_a and S_ab of its current object over the warp's steps (a lane's share of a warp range stays
+// below 2^23 points, so the u64 sums cannot wrap).  When some lane's object changes, the lanes that leave an object merge their sums
+// with the lanes leaving the same object (__match_any_sync) and the group's first lane adds them to the object's accumulators; the
+// rest keep carrying.  A map that is one giant component so costs one flush per lane group at the end of each warp's range.
+// errors[0] += points off the lattice, errors[1] += points with a component outside [-1, K).
+__device__ __forceinline__ void shape_flush_moments(int q, unsigned n, const unsigned long long s[3], const unsigned long long ss[6],
+                                                    unsigned long long* __restrict__ acc) {
+    const unsigned peers = __match_any_sync(0xffffffffu, q);
+    const unsigned n_all = __reduce_add_sync(peers, n);
+    unsigned __int128 tot_s[3], tot_ss[6];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) tot_s[a] = shape_warp_sum(peers, s[a]);
+#pragma unroll
+    for (int p = 0; p < 6; ++p) tot_ss[p] = shape_warp_sum(peers, ss[p]);
+    if (q < 0 || (int)(threadIdx.x & 31) != __ffs(peers) - 1) return;
+    unsigned long long* o = acc + (int64_t)MAP_SHAPE_ACC * q;
+    atomicAdd(o, (unsigned long long)n_all);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) atomicAdd(o + 1 + a, (unsigned long long)tot_s[a]);
+#pragma unroll
+    for (int p = 0; p < 6; ++p) shape_add_u128(o + 4 + p, o + 10 + p, tot_ss[p]);
+}
+
+__global__ void __launch_bounds__(MAP_SHAPE_BLOCK) map_shape_moments_kernel(const float* __restrict__ xyz,
+                                                                            const int64_t* __restrict__ component, int64_t P, int D,
+                                                                            int K, int64_t per, unsigned long long* __restrict__ acc,
+                                                                            long long* __restrict__ errors) {
+    const int lane = threadIdx.x & 31;
+    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t m0 = w * per, m1 = m0 + per < P ? m0 + per : P;
+    int cq = -1;
+    unsigned n = 0, n_off = 0, n_bad = 0;
+    unsigned long long s[3] = {0ull, 0ull, 0ull}, ss[6] = {0ull, 0ull, 0ull, 0ull, 0ull, 0ull};
+    for (int64_t base = m0; base < m1; base += 32) {      // warp-uniform
+        int j[3];
+        bool off, bad;
+        const int q = shape_point(xyz, component, base + lane, m1, D, K, j, off, bad);
+        n_off += off;
+        n_bad += bad;
+        const bool leave = cq >= 0 && q >= 0 && q != cq;      // skipped points keep the carry
+        if (__any_sync(0xffffffffu, leave)) {
+            shape_flush_moments(leave ? cq : -1, n, s, ss, acc);
+            if (leave) {
+                cq = -1;
+                n = 0;
+                s[0] = s[1] = s[2] = 0ull;
+#pragma unroll
+                for (int p = 0; p < 6; ++p) ss[p] = 0ull;
+            }
+        }
+        if (q >= 0) {
+            cq = q;
+            ++n;
+#pragma unroll
+            for (int a = 0; a < 3; ++a) s[a] += (unsigned long long)j[a];
+#pragma unroll
+            for (int p = 0; p < 6; ++p) ss[p] += (unsigned long long)j[c_shape_pair[p][0]] * (unsigned long long)j[c_shape_pair[p][1]];
+        }
+    }
+    shape_flush_moments(cq, n, s, ss, acc);
+    n_off = __reduce_add_sync(0xffffffffu, n_off);
+    n_bad = __reduce_add_sync(0xffffffffu, n_bad);
+    if (lane == 0) {
+        if (n_off) atomicAdd(reinterpret_cast<unsigned long long*>(errors), (unsigned long long)n_off);
+        if (n_bad) atomicAdd(reinterpret_cast<unsigned long long*>(errors + 1), (unsigned long long)n_bad);
+    }
+}
+
+// |m| of a signed 128-bit value to f64, rounded to nearest, ties to even (the conversion of (double)__int128 is not relied on)
+__device__ __forceinline__ double shape_u128_to_f64(unsigned __int128 m) {
+    const unsigned long long hi = (unsigned long long)(m >> 64), lo = (unsigned long long)m;
+    const int bits = hi ? 128 - __clzll((long long)hi) : 64 - __clzll((long long)lo);
+    if (bits <= 53) return (double)lo;                                       // exact
+    const int sh = bits - 53;
+    unsigned long long q = (unsigned long long)(m >> sh);                    // the top 53 bits
+    const unsigned __int128 rem = m & ((((unsigned __int128)1) << sh) - 1), half = ((unsigned __int128)1) << (sh - 1);
+    if (rem > half || (rem == half && (q & 1ull))) ++q;                      // q <= 2^53: exact in f64
+    return ldexp((double)q, sh);                                             // exact: a power-of-two scale, no overflow below 2^128
+}
+
+// Cyclic Jacobi on the symmetric 3x3 a (upper triangle used, every entry kept symmetric): the rotation of pair (p, q) zeroes a[p][q]
+// (Numerical Recipes' jacobi: t = sgn(theta) / (|theta| + sqrt(theta^2 + 1)), theta = (a_qq - a_pp) / (2 a_pq)); a pair whose entry is
+// exactly 0 is skipped, and after 4 sweeps an entry negligible against both diagonals is set to 0.  v accumulates the rotations:
+// column i of v is the eigenvector of a[i][i].
+__device__ void shape_jacobi(double a[3][3], double v[3][3]) {
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) v[r][c] = r == c ? 1.0 : 0.0;
+    for (int sweep = 0; sweep < MAP_SHAPE_SWEEPS; ++sweep) {
+        if (a[0][1] == 0.0 && a[0][2] == 0.0 && a[1][2] == 0.0) return;
+#pragma unroll
+        for (int pq = 0; pq < 3; ++pq) {
+            const int p = pq == 2 ? 1 : 0, q = pq == 0 ? 1 : 2;
+            const double apq = a[p][q];
+            if (apq == 0.0) continue;
+            const double app = a[p][p], aqq = a[q][q], g = 100.0 * fabs(apq), h = aqq - app;
+            if (sweep > 3 && fabs(app) + g == fabs(app) && fabs(aqq) + g == fabs(aqq)) {
+                a[p][q] = a[q][p] = 0.0;
+                continue;
+            }
+            double t;
+            if (fabs(h) + g == fabs(h)) {
+                t = apq / h;
+            } else {
+                const double theta = 0.5 * h / apq;
+                t = 1.0 / (fabs(theta) + sqrt(theta * theta + 1.0));
+                if (theta < 0.0) t = -t;
+            }
+            const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {      // a <- a J, v <- v J
+                const double arp = a[r][p], arq = a[r][q], vrp = v[r][p], vrq = v[r][q];
+                a[r][p] = c * arp - s * arq;
+                a[r][q] = s * arp + c * arq;
+                v[r][p] = c * vrp - s * vrq;
+                v[r][q] = s * vrp + c * vrq;
+            }
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {      // a <- J^T a
+                const double apr = a[p][r], aqr = a[q][r];
+                a[p][r] = c * apr - s * aqr;
+                a[q][r] = s * apr + c * aqr;
+            }
+            a[p][q] = a[q][p] = 0.0;
+        }
+    }
+}
+
+// the sign of e that makes its component of largest magnitude positive (the lowest index on ties), then unit length
+__device__ __forceinline__ void shape_orient(double e[3]) {
+    int m = 0;
+    if (fabs(e[1]) > fabs(e[m])) m = 1;
+    if (fabs(e[2]) > fabs(e[m])) m = 2;
+    const double inv = (e[m] < 0.0 ? -1.0 : 1.0) / sqrt(__dadd_rn(__dadd_rn(__dmul_rn(e[0], e[0]), __dmul_rn(e[1], e[1])), __dmul_rn(e[2], e[2])));
+#pragma unroll
+    for (int c = 0; c < 3; ++c) e[c] = __dmul_rn(e[c], inv);
+}
+
+// one thread per object: covariance from the exact moments, its eigen-decomposition, and the box accumulators' start values
+__global__ void __launch_bounds__(MAP_SHAPE_BLOCK) map_shape_axes_kernel(int K, int D, unsigned long long* __restrict__ acc,
+                                                                         double* __restrict__ covariance, double* __restrict__ variance,
+                                                                         double* __restrict__ axes) {
+    const int o = blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= K) return;
+    unsigned long long* A = acc + (int64_t)MAP_SHAPE_ACC * o;
+    const unsigned long long n = A[0];
+    double* cov = covariance + 9 * (int64_t)o;
+    double* var = variance + 3 * (int64_t)o;
+    double* ax = axes + 9 * (int64_t)o;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        A[16 + a] = shape_key(INFINITY);
+        A[19 + a] = shape_key(-INFINITY);
+    }
+    if (n == 0) {
+        for (int i = 0; i < 9; ++i) cov[i] = ax[i] = NAN;
+        var[0] = var[1] = var[2] = NAN;
+        return;
+    }
+    double a[3][3];
+    const double dn = (double)n, dD = (double)D;
+#pragma unroll
+    for (int p = 0; p < 6; ++p) {
+        const int r = c_shape_pair[p][0], c = c_shape_pair[p][1];
+        const unsigned __int128 sab = ((unsigned __int128)A[10 + p] << 64) | A[4 + p];
+        const unsigned __int128 x = (unsigned __int128)n * sab, y = (unsigned __int128)A[1 + r] * A[1 + c];      // both < 2^97
+        const double num = x >= y ? shape_u128_to_f64(x - y) : -shape_u128_to_f64(y - x);
+        const double v = __ddiv_rn(__ddiv_rn(__dmul_rn(__ddiv_rn(__ddiv_rn(num, dn), dn), 4.0), dD), dD);
+        a[r][c] = a[c][r] = v;
+    }
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) cov[3 * r + c] = a[r][c];
+    double v[3][3];
+    shape_jacobi(a, v);
+    // descending eigenvalues by a stable sort (ties keep the x, y, z order): column i goes to rank (number of columns before it with
+    // an eigenvalue >= its own) + (number after it with a larger one)
+    const double d[3] = {a[0][0], a[1][1], a[2][2]};
+    double e[3][3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        int rank = 0;
+#pragma unroll
+        for (int m = 0; m < 3; ++m) rank += m < i ? d[m] >= d[i] : m > i ? d[m] > d[i] : 0;
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            if (rank == r) {
+                var[r] = d[i];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) e[r][c] = v[c][i];
+            }
+        }
+    }
+    shape_orient(e[0]);
+    shape_orient(e[1]);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        ax[c] = e[0][c];
+        ax[3 + c] = e[1][c];
+        const int c1 = (c + 1) % 3, c2 = (c + 2) % 3;
+        ax[6 + c] = __dsub_rn(__dmul_rn(e[0][c1], e[1][c2]), __dmul_rn(e[0][c2], e[1][c1]));
+    }
+}
+
+// projection of lattice index j on axis row e: ((jx ex + jy ey) + jz ez), every operation rounded
+__device__ __forceinline__ double shape_project(const int j[3], const double* e) {
+    return __dadd_rn(__dadd_rn(__dmul_rn((double)j[0], e[0]), __dmul_rn((double)j[1], e[1])), __dmul_rn((double)j[2], e[2]));
+}
+
+// Extents: the same walk as the moments, each lane carrying the min / max of its current object's projections on the object's axes
+// (exact, so the result does not depend on the order); leaving lanes merge per object and one lane takes the atomicMin / atomicMax.
+__device__ __forceinline__ void shape_flush_box(int q, const unsigned long long lo[3], const unsigned long long hi[3],
+                                                unsigned long long* __restrict__ acc) {
+    const unsigned peers = __match_any_sync(0xffffffffu, q);
+    unsigned long long l[3], h[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        l[a] = shape_warp_extreme<false>(peers, lo[a]);
+        h[a] = shape_warp_extreme<true>(peers, hi[a]);
+    }
+    if (q < 0 || (int)(threadIdx.x & 31) != __ffs(peers) - 1) return;
+    unsigned long long* o = acc + (int64_t)MAP_SHAPE_ACC * q;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        if (l[a] < __ldcg(o + 16 + a)) atomicMin(o + 16 + a, l[a]);
+        if (h[a] > __ldcg(o + 19 + a)) atomicMax(o + 19 + a, h[a]);
+    }
+}
+
+__global__ void __launch_bounds__(MAP_SHAPE_BLOCK) map_shape_extent_kernel(const float* __restrict__ xyz,
+                                                                           const int64_t* __restrict__ component, int64_t P, int D,
+                                                                           int K, int64_t per, const double* __restrict__ axes,
+                                                                           unsigned long long* __restrict__ acc) {
+    const unsigned long long EMPTY_LO = 0xffffffffffffffffull, EMPTY_HI = 0ull;
+    const int lane = threadIdx.x & 31;
+    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t m0 = w * per, m1 = m0 + per < P ? m0 + per : P;
+    int cq = -1;
+    double e[9];
+    unsigned long long lo[3] = {EMPTY_LO, EMPTY_LO, EMPTY_LO}, hi[3] = {EMPTY_HI, EMPTY_HI, EMPTY_HI};
+    for (int64_t base = m0; base < m1; base += 32) {
+        int j[3];
+        bool off, bad;
+        const int q = shape_point(xyz, component, base + lane, m1, D, K, j, off, bad);
+        const bool leave = cq >= 0 && q >= 0 && q != cq;      // skipped points keep the carry
+        if (__any_sync(0xffffffffu, leave)) {
+            shape_flush_box(leave ? cq : -1, lo, hi, acc);
+            if (leave) {
+                cq = -1;
+#pragma unroll
+                for (int a = 0; a < 3; ++a) { lo[a] = EMPTY_LO; hi[a] = EMPTY_HI; }
+            }
+        }
+        if (q >= 0) {
+            if (q != cq) {
+#pragma unroll
+                for (int i = 0; i < 9; ++i) e[i] = __ldg(axes + 9 * (int64_t)q + i);
+                cq = q;
+            }
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const unsigned long long key = shape_key(shape_project(j, e + 3 * a));
+                lo[a] = key < lo[a] ? key : lo[a];
+                hi[a] = key > hi[a] ? key : hi[a];
+            }
+        }
+    }
+    shape_flush_box(cq, lo, hi, acc);
+}
+
+// one thread per object: extent_a = ((hi_a - lo_a) + 1) 2 / D; centre c = sum_a ((lo_a + hi_a) / 2) e_a in the lattice, (2 c + 1) / D - 1
+// in the world
+__global__ void __launch_bounds__(MAP_SHAPE_BLOCK) map_shape_box_kernel(int K, int D, const unsigned long long* __restrict__ acc,
+                                                                        const double* __restrict__ axes, double* __restrict__ center,
+                                                                        double* __restrict__ extent) {
+    const int o = blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= K) return;
+    const unsigned long long* A = acc + (int64_t)MAP_SHAPE_ACC * o;
+    double* ce = center + 3 * (int64_t)o;
+    double* ex = extent + 3 * (int64_t)o;
+    if (A[0] == 0) {
+        ce[0] = ce[1] = ce[2] = ex[0] = ex[1] = ex[2] = NAN;
+        return;
+    }
+    const double dD = (double)D;
+    const double* e = axes + 9 * (int64_t)o;
+    double mid[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const double l = shape_unkey(A[16 + a]), h = shape_unkey(A[19 + a]);
+        ex[a] = __ddiv_rn(__dmul_rn(__dadd_rn(__dsub_rn(h, l), 1.0), 2.0), dD);
+        mid[a] = __ddiv_rn(__dadd_rn(l, h), 2.0);
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const double lc = __dadd_rn(__dadd_rn(__dmul_rn(mid[0], e[c]), __dmul_rn(mid[1], e[3 + c])), __dmul_rn(mid[2], e[6 + c]));
+        ce[c] = __dsub_rn(__ddiv_rn(__dadd_rn(__dmul_rn(2.0, lc), 1.0), dD), 1.0);
+    }
+}
+
 static int map_stats_launch(const float* xyz, const float* rgb, const int64_t* semantic, const int64_t* lab, int64_t P, int Cs, int Ci,
                             uint32_t thing_mask, int unlabelled_ok, const int64_t* inst_src, int64_t* inst_out, int64_t* count,
                             double* sum_xyz, double* sum_rgb, int64_t* votes, float* bbox_min, float* bbox_max, int64_t* errors,
@@ -1009,6 +1384,37 @@ int pag_map_visibility_silhouette(const float* xyz, int64_t P, const float* view
                                                                                             reinterpret_cast<long long*>(silhouette));
         PAG_LAUNCH_CHECK();
     }
+    return PAG_OK;
+}
+
+int pag_map_shape(const float* xyz, int64_t P, int level, int k, const int64_t* component, int K, int64_t* acc, double* covariance,
+                  double* variance, double* axes, double* center, double* extent, int64_t* errors, void* stream) {
+    if (P < 0 || P > MAP_CC_MAX_POINTS || level < 0 || level > 15 || k < 1 || k > 8 || K < 0 || K > MAP_CC_MAX_POINTS || !errors)
+        return PAG_ERR_ARG;
+    if ((P > 0 && (!xyz || !component)) || (K > 0 && (!acc || !covariance || !variance || !axes || !center || !extent)))
+        return PAG_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(errors, 0, 2 * sizeof(int64_t), s);
+    if (e != cudaSuccess) return (int)e;
+    if (K > 0 && (e = cudaMemsetAsync(acc, 0, (size_t)K * MAP_SHAPE_ACC * sizeof(int64_t), s)) != cudaSuccess) return (int)e;
+    const int D = k << level;
+    unsigned long long* A = reinterpret_cast<unsigned long long*>(acc);
+    int blocks = 0;
+    int64_t per = 0;
+    if (P > 0) {      // the error counts also when there is no object
+        shape_grid(P, &blocks, &per);
+        map_shape_moments_kernel<<<blocks, MAP_SHAPE_BLOCK, 0, s>>>(xyz, component, P, D, K, per, A, reinterpret_cast<long long*>(errors));
+        PAG_LAUNCH_CHECK();
+    }
+    if (K == 0) return PAG_OK;
+    map_shape_axes_kernel<<<pag_grid(K, MAP_SHAPE_BLOCK), MAP_SHAPE_BLOCK, 0, s>>>(K, D, A, covariance, variance, axes);
+    PAG_LAUNCH_CHECK();
+    if (P > 0) {
+        map_shape_extent_kernel<<<blocks, MAP_SHAPE_BLOCK, 0, s>>>(xyz, component, P, D, K, per, axes, A);
+        PAG_LAUNCH_CHECK();
+    }
+    map_shape_box_kernel<<<pag_grid(K, MAP_SHAPE_BLOCK), MAP_SHAPE_BLOCK, 0, s>>>(K, D, A, axes, center, extent);
+    PAG_LAUNCH_CHECK();
     return PAG_OK;
 }
 

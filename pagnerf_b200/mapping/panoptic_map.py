@@ -136,6 +136,37 @@ object_visibility answers, per map object and camera view, how much of the objec
     (view, object) pair plus 16 bytes, and the silhouette bitmaps: one bit per pixel of each pair's footprint box, rows padded to
     32-bit words, at most VISIBILITY_BITMAP_BYTES (256 MiB).  When the bitmaps exceed it the silhouettes are built in rounds,
     each a pass over the points and cameras.
+
+object_shape measures each object's size and orientation from its points, in map units:
+
+    shape = object_shape(pts, samples_per_axis=2, level=nef.grid.blas_level, component=comps.component,
+                         num_objects=comps.count.numel())                               # ObjectShape of [K, ...] f64 tensors
+    length, width, height = shape.extent.unbind(-1)            # the oriented box's sides, longest principal axis first
+
+  * Lattice.  The rules of map_index: D = samples_per_axis << level, every point on the lattice bit for bit (xyz float32,
+    P <= 2^30); points off it raise ValueError with their number.  Duplicate lattice indices are not checked: such points count
+    once each.  component i64 [P] (e.g. InstanceComponents.component) gives each point's object in [0, num_objects) or -1;
+    components outside [-1, num_objects) raise ValueError with their number.  Points with component -1 are ignored.
+  * Exact moments.  From the integer lattice indices j in [0, D)^3 of an object's points: n, S_a = sum j_a and S_ab = sum j_a j_b,
+    exact (S_ab in 128 bits).  The numerator num_ab = n S_ab - S_a S_b is exact and converted to float64 rounded to nearest, ties
+    to even; covariance[a, b] = (((num_ab / n) / n) * 4 / D) / D in float64, each operation IEEE-rounded.  That is the population
+    covariance of the points' world positions (x = (2j + 1) / D - 1), bit for bit independent of point order and thread schedule.
+  * Axes.  A cyclic Jacobi eigensolver in float64, one thread per object, at most 50 sweeps; a rotation whose off-diagonal entry is
+    exactly 0 is skipped, so a diagonal covariance (lattice balls and axis-aligned boxes, by symmetry) yields the world axes.
+    variance = the eigenvalues in descending order, ties in x, y, z order; axes[a] = the unit eigenvector of variance[a], rows 0
+    and 1 signed so that their component of largest magnitude is positive (the lowest index on ties), axes[2] = axes[0] x axes[1].
+    Where eigenvalues are equal but the covariance is not diagonal, the rows spanning that eigenspace are an orthonormal basis of
+    it; which basis is deterministic but not specified.
+  * Box.  Projections p_a = ((jx e_ax + jy e_ay) + jz e_az) in float64, each operation rounded (no FMA), e_a = axes[a]; lo_a / hi_a
+    their minimum / maximum over the object's points in the IEEE total order (-0 < +0).  extent[a] = ((hi_a - lo_a) + 1) * 2 / D:
+    every point stands for its cell, as in project_map's footprint.  center = (2 c + 1) / D - 1 per axis, c = sum over a of
+    ((lo_a + hi_a) / 2) e_a in the lattice (((m_0 e_0 + m_1 e_1) + m_2 e_2) per coordinate, each operation rounded).
+  * Edge cases.  An object without points gets NaN in every output; one point gives covariance 0, the world axes and the extent of
+    one cell; K = 0 or P = 0 give empty (or NaN) outputs.
+  * Reading.  extent is the object's length, width and height along its principal axes.  For a solid ellipsoid the semi-axis along
+    axes[a] is sqrt(5 variance[a]); for a thin shell (points on the surface only) about sqrt(3 variance[a]), exact for a sphere.
+  * Host traffic.  One host read per call (the error counts); the call cannot be captured in a CUDA graph.
+  * Memory.  The outputs (216 bytes per object) and SHAPE_WORKSPACE_BYTES = 176 bytes of accumulators per object, plus 16 bytes.
 """
 import math
 from typing import NamedTuple, Optional
@@ -156,6 +187,7 @@ MAX_LOOKUP_RADIUS = 4                                # a (2r+1)^3 window: 729 pr
 MAX_PROJECT_RADIUS = 32                              # a footprint of at most 66 x 66 pixels
 MAX_PROJECT_SIDE = 16384
 MAX_PROJECT_CAMERAS = 65535                          # one grid row per camera
+SHAPE_WORKSPACE_BYTES = 8 * ops.SHAPE_ACC_WORDS          # object_shape's accumulators per object
 VISIBILITY_BITMAP_BYTES = 256 << 20                  # silhouette bitmaps of one round; >= 32 MiB, one 16384 x 16384 view's
 
 
@@ -204,6 +236,14 @@ class ObjectVisibility(NamedTuple):
     visible: torch.Tensor                  # i64 [B, K]: pixels of view b whose front map point belongs to object o
     silhouette: torch.Tensor               # i64 [B, K]: pixels of view b covered by object o's points at any depth
     bbox: torch.Tensor                     # i32 [B, K, 4]: (col_min, row_min, col_max, row_max) of the visible pixels, -1s if none
+
+
+class ObjectShape(NamedTuple):
+    covariance: torch.Tensor               # f64 [K, 3, 3]: population covariance of the object's point positions, world units^2
+    variance: torch.Tensor                 # f64 [K, 3]: its eigenvalues, descending
+    axes: torch.Tensor                     # f64 [K, 3, 3]: row a = the unit eigenvector of variance[:, a]
+    center: torch.Tensor                   # f64 [K, 3]: centre of the oriented box, world coordinates
+    extent: torch.Tensor                   # f64 [K, 3]: the box's side lengths along axes, world units
 
 
 class InstanceSummary(NamedTuple):
@@ -460,6 +500,20 @@ def lookup_rays(index, origins, dirs, depth, alpha, radius=1, min_alpha=0.5, com
     return MapLookup(point, obj)
 
 
+def _check_component(component, P, what):
+    """component must be an i64 [P] tensor, one entry per point of the `what` map"""
+    if not isinstance(component, torch.Tensor) or tuple(component.shape) != (P,):
+        shape = list(component.shape) if isinstance(component, torch.Tensor) else type(component).__name__
+        raise ValueError(f"component must have shape [{P}] (the {what} map's points), got {shape}")
+    if component.dtype != torch.int64:
+        raise TypeError(f"component must be torch.int64, got {component.dtype}")
+
+
+def _check_num_objects(num_objects):
+    if not _is_int(num_objects) or not 0 <= num_objects <= MAX_COMPONENT_POINTS:
+        raise ValueError(f"num_objects must be an integer in [0, {MAX_COMPONENT_POINTS}], got {num_objects!r}")
+
+
 def _check_projection(fn, pts, k, level, view, intrinsics, height, width, max_radius, near, component):
     """The arguments project_map and object_visibility share -> (xyz, h, near) as the kernels take them"""
     _check_lattice(k, level)
@@ -482,11 +536,7 @@ def _check_projection(fn, pts, k, level, view, intrinsics, height, width, max_ra
             not (np.isfinite(np.float32(near)) and np.float32(near) > 0):
         raise ValueError(f"near must be a finite number > 0, got {near!r}")
     if component is not None:
-        if not isinstance(component, torch.Tensor) or tuple(component.shape) != (P,):
-            shape = list(component.shape) if isinstance(component, torch.Tensor) else type(component).__name__
-            raise ValueError(f"component must have shape [{P}] (the projected map's points), got {shape}")
-        if component.dtype != torch.int64:
-            raise TypeError(f"component must be torch.int64, got {component.dtype}")
+        _check_component(component, P, "projected")
     if not all(t.is_cuda for t in (xyz, view, intrinsics, component) if t is not None):
         raise RuntimeError("pagnerf_b200 map projection runs on CUDA tensors only (no CPU fallback)")
     return xyz, float(np.float32(1.0) / np.float32(int(k) << int(level))), float(np.float32(near))
@@ -511,8 +561,7 @@ def object_visibility(pts, samples_per_axis, level, view, intrinsics, height, wi
     definitions and the memory bound."""
     if component is None:
         raise TypeError("object_visibility needs component (i64 [P], each point's object or -1)")
-    if not _is_int(num_objects) or not 0 <= num_objects <= MAX_COMPONENT_POINTS:
-        raise ValueError(f"num_objects must be an integer in [0, {MAX_COMPONENT_POINTS}], got {num_objects!r}")
+    _check_num_objects(num_objects)
     xyz, h, near = _check_projection("object_visibility", pts, samples_per_axis, level, view, intrinsics, height, width, max_radius,
                                      near, component)
     K = int(num_objects)
@@ -521,6 +570,36 @@ def object_visibility(pts, samples_per_axis, level, view, intrinsics, height, wi
     if bad:
         raise ValueError(f"{bad} points carry a component outside [-1, {K})")
     return ObjectVisibility(visible, silhouette, bbox)
+
+
+def object_shape(pts, samples_per_axis, level, component, num_objects):
+    """Size and orientation of each map object: the exact covariance of its points, its principal axes and the oriented box along
+    them -> ObjectShape of [num_objects, ...] float64 tensors (csrc/mapping.cu, one host read).  pts: PanopticPoints or its xyz
+    f32 [P, 3] on the lattice of (samples_per_axis, level); component i64 [P] (e.g. InstanceComponents.component) gives each
+    point's object in [0, num_objects) or -1.  Raises ValueError with their number for points off the lattice and components
+    outside [-1, num_objects).  See the module docstring for the exact definitions and the memory bound."""
+    if component is None:
+        raise TypeError("object_shape needs component (i64 [P], each point's object or -1)")
+    k = samples_per_axis
+    _check_lattice(k, level)
+    xyz = pts.xyz if isinstance(pts, PanopticPoints) else pts
+    _check_tensor("xyz", xyz, [(None, 3)], torch.float32)
+    P = int(xyz.shape[0])
+    if P > MAX_COMPONENT_POINTS:
+        raise ValueError(f"object_shape serves up to {MAX_COMPONENT_POINTS} points, got {P}")
+    _check_component(component, P, "measured")
+    _check_num_objects(num_objects)
+    if not (xyz.is_cuda and component.is_cuda):
+        raise RuntimeError("pagnerf_b200 object shape runs on CUDA tensors only (no CPU fallback)")
+    k, level, K = int(k), int(level), int(num_objects)
+    cov, var, axes, center, extent, _, errors = ops.map_shape(xyz, level, k, component, K)
+    off, bad = errors.tolist()                      # the call's one host read: the error counts
+    errs = _lattice_errors(off, 0, k, level)
+    if bad:
+        errs.append(f"{bad} points carry a component outside [-1, {K})")
+    if errs:
+        raise ValueError("; ".join(errs))
+    return ObjectShape(cov, var, axes, center, extent)
 
 
 PLY_PROPERTIES = [("x", "float", "<f4"), ("y", "float", "<f4"), ("z", "float", "<f4"),

@@ -777,6 +777,30 @@ def map_visibility(xyz, view, intrinsics, H, W, h, near, max_radius, component, 
     return visible, silhouette, bbox, bad, total
 
 
+SHAPE_ACC_WORDS = 22      # i64 accumulators per object of pag_map_shape (include/pagnerf_b200.h)
+
+
+def map_shape(xyz, level, k, component, K):
+    """Size and orientation of each of K map objects (xyz f32[P,3] on the lattice, component i64[P]; csrc/mapping.cu pag_map_shape)
+    -> covariance f64[K,3,3], variance f64[K,3], axes f64[K,3,3], center f64[K,3], extent f64[K,3], acc i64[K,22] (the workspace:
+    moments, then the order-preserving images of the projections' minima and maxima) and errors i64[2] = (points off the lattice,
+    points with a component outside [-1, K)), all on the device.  Allocates the outputs, 176 bytes of workspace per object and 16
+    bytes of error counts (for contiguous inputs)."""
+    _chk(xyz, component)
+    if xyz.dtype != torch.float32:
+        raise TypeError(f"map_shape: xyz must be float32 (the lattice is defined bit for bit in fp32), got {xyz.dtype}")
+    x = xyz.detach().reshape(-1, 3).contiguous()
+    comp = component.contiguous()
+    dev = x.device
+    f64 = lambda *s: torch.empty(*s, dtype=torch.float64, device=dev)
+    cov, var, axes, center, extent = f64(K, 3, 3), f64(K, 3), f64(K, 3, 3), f64(K, 3), f64(K, 3)
+    acc = torch.empty(K, SHAPE_ACC_WORDS, dtype=torch.int64, device=dev)
+    errors = torch.empty(2, dtype=torch.int64, device=dev)
+    call("pag_map_shape", ptr(x), x.shape[0], int(level), int(k), ptr(comp), int(K), ptr(acc), ptr(cov), ptr(var), ptr(axes),
+         ptr(center), ptr(extent), ptr(errors))
+    return cov, var, axes, center, extent, acc, errors
+
+
 class PanCompositeFn(Function):
     """Semantic + instance heads fused with their (detached-weight) compositing: per-ray outputs [N,Cs], [N,Ci].
     Tensor-core kernels only (training mode); csrc/decoder_tc_fused.cu."""

@@ -11,6 +11,15 @@ import inspect
 import torch.nn as nn
 
 
+class _FieldMethod:
+    """A forward function that is a method of the field, kept as its plain function and bound to the field again at each call.  The
+    bound method would make the field reference itself: a field its owner drops (and its parameters on the device) would then live
+    on until the cycle collector runs, which may be at any later allocation."""
+
+    def __init__(self, func):
+        self.func = func
+
+
 class BaseNeuralField(nn.Module):
     def __init__(self, grid_type='OctreeGrid', interpolation_type='linear', multiscale_type='none',
                  as_type='octree', raymarch_type='voxel', decoder_type='none', embedder_type='none',
@@ -70,6 +79,8 @@ class BaseNeuralField(nn.Module):
     def _register_forward_function(self, fn, channels):
         if isinstance(channels, str):
             channels = [channels]
+        if inspect.ismethod(fn) and fn.__self__ is self:
+            fn = _FieldMethod(fn.__func__)
         self._forward_functions[fn] = set(channels)
 
     def get_supported_channels(self):
@@ -98,6 +109,8 @@ class BaseNeuralField(nn.Module):
             supported = out_channels & requested
             if not supported:
                 continue
+            if isinstance(fn, _FieldMethod):
+                fn = fn.func.__get__(self, type(self))
             argspec = inspect.getfullargspec(fn)
             ndef = len(argspec.defaults) if argspec.defaults else 0
             required = argspec.args[:len(argspec.args) - ndef][1:]
